@@ -168,6 +168,16 @@ int smcp_kkt_assemble_cyclic(smcp_op *op, smcp_hess *h, int64_t block, int rank,
 int smcp_kkt_assemble_syrk(smcp_op *op, smcp_hess *h);
 int smcp_kkt_z_tmul(smcp_op *op, const double *X_dev, double *host_out);
 int smcp_kkt_z_mul(smcp_op *op, const double *host_y, double *X_dev);
+/* kktsolver='qr' in Householder form (the reference's geqrf / ormqr / trtrs): forms Zw as
+ * smcp_kkt_assemble_syrk does, factors Zw = Q1 R on the device, keeps Q1 (nblk x m) in place of Zw
+ * and L = R^T with diag(L) >= 0 as the lower triangle of H (L L^T = the SYRK-form H).  info_host = k > 0
+ * at the first k with R_kk <= 1e-14 max R_ii (Z rank deficient).  Needs Ns = 0.  Afterwards
+ * smcp_kkt_z_tmul / smcp_kkt_z_mul refuse until the next smcp_kkt_assemble_syrk.               */
+int smcp_kkt_factor_qr(smcp_op *op, smcp_hess *h, int32_t *info_host);
+/* Newton solve of the Householder form: with g = G_dev (= G(b_x), a chordal matrix) and r = host_r
+ * (= kk b_y), y = H^-1 (r + Z^T g) into host_y and X_dev = Z y - g (the argument of G^adj) through Q1 and
+ * L only; refuses without a successful smcp_kkt_factor_qr                                      */
+int smcp_kkt_qr_solve(smcp_op *op, const double *G_dev, const double *host_r, double *host_y, double *X_dev);
 /* lapack.potrf(H): info_host = 0 ok, k > 0 if the leading minor of order k is not PD        */
 int smcp_kkt_factor(smcp_op *op, int32_t *info_host);
 /* lapack.potrs(H, y) in place on a host m-vector */
@@ -224,13 +234,18 @@ int smcp_host_supernodes(int64_t n, const int64_t *colptr, const int64_t *rowind
  *   halves of cvxopt.lapack.potrs (solvers.py:526) and chompack.trsm on a dense supernode (491-492).
  * smcp_dense_gemm: C = [C +] alpha op(A) op(B)^T on the FP64 tensor cores; ta / tb = 1: the operand
  *   is stored K-major (A[k + i*lda]); tri = 1: lower triangle only (the contraction of
- *   solvers.py:486 and every frontal update). */
+ *   solvers.py:486 and every frontal update).
+ * smcp_dense_geqrf / smcp_dense_orgqr: lapack.geqrf / lapack.orgqr of an M x N matrix, M >= N
+ *   (Householder vectors below the diagonal with a unit diagonal, LAPACK's beta and tau; orgqr
+ *   overwrites them with the M x N Q1), by the blocked Householder QR of kktsolver='qr'. */
 int smcp_dense_potrf(smcp_ctx *ctx, double *A_host, int64_t lda, int64_t m, int64_t ncols, int32_t *info_host, double *ms_out);
 int smcp_dense_trsm(smcp_ctx *ctx, int trans, const double *L_host, int64_t ldl, int64_t n, double *B_host, int64_t ldb,
                     int64_t nrhs, double *ms_out);
 int smcp_dense_gemm(smcp_ctx *ctx, int ta, int tb, const double *A_host, int64_t lda, const double *B_host, int64_t ldb,
                     double *C_host, int64_t ldc, int64_t M, int64_t N, int64_t K, double alpha, int accumulate, int tri,
                     double *ms_out);
+int smcp_dense_geqrf(smcp_ctx *ctx, double *A_host, int64_t lda, int64_t M, int64_t N, double *tau_host, double *ms_out);
+int smcp_dense_orgqr(smcp_ctx *ctx, double *A_host, int64_t lda, int64_t M, int64_t N, const double *tau_host, double *ms_out);
 
 #ifdef __cplusplus
 }

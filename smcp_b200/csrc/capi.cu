@@ -215,6 +215,7 @@ extern "C" int smcp_ctx_destroy(smcp_ctx *ctx) {
     if (ctx->wave_buf) cudaFree(ctx->wave_buf);
     if (ctx->potrf_pt) cudaFree(ctx->potrf_pt);
     if (ctx->trs_dinv) cudaFree(ctx->trs_dinv);
+    if (ctx->qr_ws) cudaFree(ctx->qr_ws);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
     cudaEventDestroy(ctx->ev0);
     cudaEventDestroy(ctx->ev1);
@@ -589,6 +590,8 @@ struct smcp_op {
     size_t Ub_cap = 0;
     double *Zinv = nullptr;       // n x n dense inverse for the sparse-constraint technique
     double *Zq = nullptr;         // kktsolver='qr': Z = [G(A_1) ... G(A_m)] weighted by sqrt(wdot), nblk x m
+    int zq_state = 0;             // what Zq holds: 0 nothing, 1 Zw (SYRK form), 2 Q1 of Zw = Q1 R (Householder form)
+    double *qr_tau = nullptr;     // Householder form: tau (m), signs of diag(R) (m), right-hand side r (m)
     double *sqrtw = nullptr;      // sqrt of the trace inner-product weights (nblk)
     double *Dinv = nullptr;       // inverses of the 64 x 64 diagonal blocks of chol(H) (potrs)
     std::vector<long long> h_colptr;
@@ -788,6 +791,7 @@ extern "C" int smcp_op_destroy(smcp_op *op) {
     if (op->Kpos) cudaFree(op->Kpos);
     if (op->ell_val) { cudaFree(op->ell_val); cudaFree(op->ell_pid); }
     if (op->Zq) cudaFree(op->Zq);
+    if (op->qr_tau) cudaFree(op->qr_tau);
     if (op->sqrtw) cudaFree(op->sqrtw);
     if (op->Dinv) cudaFree(op->Dinv);
     cudaFree(op->H); cudaFree(op->info_dev); cudaFree(op->yv);
@@ -1256,15 +1260,16 @@ __global__ void __launch_bounds__(256) zmul_kernel(const double *__restrict__ Z,
     if (r < nblk) x[r] = (s0 + s1) + (s2 + s3);
 }
 
-extern "C" int smcp_kkt_assemble_syrk(smcp_op *op, smcp_hess *h) {
+// Zw = diag(sqrt(wdot)) [G(A_1) ... G(A_m)] in op->Zq (G = identity when h is NULL)
+static int form_zw(smcp_op *op, smcp_hess *h, const char *who) {
     smcp_sym *s = op->sym;
     smcp_ctx *ctx = s->ctx;
-    RegionScope rs(ctx, "kkt_assemble");
     const int64_t m = op->m;
     const long long nblk = s->d.nblk;
-    if (op->Ns) { smcp_set_error("smcp_kkt_assemble_syrk: the sparse-constraint technique does not apply (Ns must be 0)"); return -2; }
+    if (op->Ns) { smcp_set_error("%s: the sparse-constraint technique does not apply (Ns must be 0)", who); return -2; }
     const size_t bytes = (size_t)nblk * (size_t)m * sizeof(double);
     if (bytes > ((size_t)96 << 30)) { smcp_set_error("kktsolver='qr' needs m*|blkval| doubles (%.1f GB)", bytes / 1073741824.0); return -2; }
+    op->zq_state = 0;
     if (!op->Zq) CUDA_TRY(cudaMalloc(&op->Zq, bytes ? bytes : 8));
     if (!op->sqrtw) {
         CUDA_TRY(cudaMalloc(&op->sqrtw, (size_t)nblk * sizeof(double)));
@@ -1286,6 +1291,17 @@ extern "C" int smcp_kkt_assemble_syrk(smcp_op *op, smcp_hess *h) {
         LaunchScope ls(ctx, "level1");
         rowscale_kernel<<<ctx->num_sms * 8, 256, 0, ctx->stream>>>(op->Zq, op->sqrtw, nblk, m, 0);
     }
+    op->zq_state = 1;
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int smcp_kkt_assemble_syrk(smcp_op *op, smcp_hess *h) {
+    smcp_ctx *ctx = op->sym->ctx;
+    RegionScope rs(ctx, "kkt_assemble");
+    const int64_t m = op->m;
+    const long long nblk = op->sym->d.nblk;
+    if (int rc = form_zw(op, h, "smcp_kkt_assemble_syrk")) return rc;
     if (launch_gemm(ctx, true, true, op->Zq, nblk, op->Zq, nblk, op->H, m, m, m, nblk, 1.0, 0, 1, 0, "schur_syrk_dmma")) return -1;
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -1295,7 +1311,7 @@ extern "C" int smcp_kkt_assemble_syrk(smcp_op *op, smcp_hess *h) {
 extern "C" int smcp_kkt_z_tmul(smcp_op *op, const double *X, double *host_out) {
     smcp_sym *s = op->sym;
     smcp_ctx *ctx = s->ctx;
-    if (!op->Zq) { smcp_set_error("smcp_kkt_z_tmul: no SYRK-form assembly yet"); return -2; }
+    if (op->zq_state != 1) { smcp_set_error("smcp_kkt_z_tmul: no SYRK-form assembly (Zq holds %s)", op->zq_state ? "Q1 of the Householder form" : "nothing"); return -2; }
     const long long nblk = s->d.nblk;
     if (grow((void **)&s->tmp, &s->tmp_cap, (size_t)nblk * sizeof(double))) return -1;
     CUDA_TRY(cudaMemcpyAsync(s->tmp, X, (size_t)nblk * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
@@ -1317,7 +1333,7 @@ extern "C" int smcp_kkt_z_tmul(smcp_op *op, const double *X, double *host_out) {
 extern "C" int smcp_kkt_z_mul(smcp_op *op, const double *host_y, double *X) {
     smcp_sym *s = op->sym;
     smcp_ctx *ctx = s->ctx;
-    if (!op->Zq) { smcp_set_error("smcp_kkt_z_mul: no SYRK-form assembly yet"); return -2; }
+    if (op->zq_state != 1) { smcp_set_error("smcp_kkt_z_mul: no SYRK-form assembly (Zq holds %s)", op->zq_state ? "Q1 of the Householder form" : "nothing"); return -2; }
     const long long nblk = s->d.nblk;
     CUDA_TRY(cudaMemcpyAsync(op->yv, host_y, (size_t)op->m * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     {
@@ -1330,6 +1346,94 @@ extern "C" int smcp_kkt_z_mul(smcp_op *op, const double *host_y, double *X) {
     }
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));       // host_y may be reused by the caller
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------
+// kktsolver='qr' in Householder form, the reference's kkt_qr (solvers.py:413-475: geqrf / ormqr / trtrs):
+// Zw = Q1 R with Q1 (nblk x m) formed explicitly in Zq and L = R^T (diag >= 0) in H, so that L L^T is the
+// SYRK-form H and the solves never multiply by R and undo it:
+//   gw = sqrt(w) g,  c = Q1^T gw,  a = L^-1 r,  v = a + c,  y = L^-T v,  x = (Q1 v - gw) / sqrt(w)
+// ---------------------------------------------------------------------------------------
+// x[r] = (q[r] - gw[r]) / sw[r], and -g[r] where the weight is 0 (entries outside the vector space: the
+// SYRK form's z_mul(y) - g there)
+__global__ void qr_xout_kernel(const double *__restrict__ q, const double *__restrict__ gw, const double *g,
+                               const double *__restrict__ sw, double *x, long long n) {
+    for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += (long long)gridDim.x * blockDim.x) {
+        const double s = sw[r];
+        x[r] = s > 0.0 ? (q[r] - gw[r]) / s : -g[r];
+    }
+}
+__global__ void qr_vadd_kernel(double *__restrict__ v, const double *__restrict__ a, long long n) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) v[i] = a[i] + v[i];
+}
+
+extern "C" int smcp_kkt_factor_qr(smcp_op *op, smcp_hess *h, int32_t *info_host) {
+    smcp_sym *s = op->sym;
+    smcp_ctx *ctx = s->ctx;
+    const int64_t m = op->m;
+    const long long nblk = s->d.nblk;
+    if (m > nblk) { smcp_set_error("smcp_kkt_factor_qr: more constraints (%lld) than rows of Z (%lld)", (long long)m, nblk); return -2; }
+    {
+        RegionScope rs(ctx, "kkt_assemble");
+        if (int rc = form_zw(op, h, "smcp_kkt_factor_qr")) return rc;
+        op->zq_state = 0;           // Zq is overwritten with Q1 below
+    }
+    if (!op->qr_tau) CUDA_TRY(cudaMalloc(&op->qr_tau, (size_t)3 * std::max<int64_t>(m, 1) * sizeof(double)));
+    {
+        RegionScope rs(ctx, "kkt_factor");
+        if (d_geqrf(ctx, op->Zq, nblk, nblk, m, op->qr_tau)) return -1;
+        if (qr_extract_lower(ctx, op->Zq, nblk, m, op->H, m, op->qr_tau + m, op->info_dev)) return -1;
+        if (d_orgqr(ctx, op->Zq, nblk, nblk, m, op->qr_tau)) return -1;
+        if (qr_apply_colsign(ctx, op->Zq, nblk, nblk, m, op->qr_tau + m)) return -1;
+        if (d_potrs_prepare(ctx, op->H, m, m, op->Dinv)) return -1;
+    }
+    CUDA_TRY(cudaMemcpyAsync(info_host, op->info_dev, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    op->zq_state = *info_host ? 0 : 2;
+    return 0;
+}
+
+extern "C" int smcp_kkt_qr_solve(smcp_op *op, const double *G_dev, const double *host_r, double *host_y, double *X_dev) {
+    smcp_sym *s = op->sym;
+    smcp_ctx *ctx = s->ctx;
+    if (op->zq_state != 2) { smcp_set_error("smcp_kkt_qr_solve: no Householder-form factorisation (smcp_kkt_factor_qr)"); return -2; }
+    const int64_t m = op->m;
+    const long long nblk = s->d.nblk;
+    double *rv = op->qr_tau + 2 * m;
+    if (grow((void **)&s->tmp, &s->tmp_cap, (size_t)2 * nblk * sizeof(double))) return -1;
+    double *gw = s->tmp, *q = s->tmp + nblk;
+    CUDA_TRY(cudaMemcpyAsync(rv, host_r, (size_t)m * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    {
+        RegionScope rs(ctx, "kkt_solve");
+        CUDA_TRY(cudaMemcpyAsync(gw, G_dev, (size_t)nblk * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        {
+            LaunchScope ls(ctx, "level1");
+            rowscale_kernel<<<ctx->num_sms * 2, 256, 0, ctx->stream>>>(gw, op->sqrtw, nblk, 1, 2);
+        }
+        if (d_trs_cluster(ctx, op->H, m, m, op->Dinv, rv, m, 1, 1, 0, "potrs")) return -1;        // a = L^-1 r
+        {
+            LaunchScope ls(ctx, "qr_qmul", 1, 8.0 * (double)nblk * (double)m);
+            amap_dense_kernel<<<(unsigned)m, 256, 0, ctx->stream>>>(op->Zq, nblk, gw, op->yv, 0);      // c = Q1^T gw
+        }
+        {
+            LaunchScope ls(ctx, "level1");
+            qr_vadd_kernel<<<(unsigned)((m + 255) / 256), 256, 0, ctx->stream>>>(op->yv, rv, m);          // v = a + c
+        }
+        {
+            LaunchScope ls(ctx, "qr_qmul", 1, 8.0 * (double)nblk * (double)m);
+            zmul_kernel<<<(unsigned)((nblk + 255) / 256), 256, 0, ctx->stream>>>(op->Zq, nblk, m, op->yv, q);   // Q1 v
+        }
+        {
+            LaunchScope ls(ctx, "level1");
+            qr_xout_kernel<<<ctx->num_sms * 2, 256, 0, ctx->stream>>>(q, gw, G_dev, op->sqrtw, X_dev, nblk);
+        }
+        if (d_trs_cluster(ctx, op->H, m, m, op->Dinv, op->yv, m, 1, 0, 1, "potrs")) return -1;    // y = L^-T v
+    }
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpyAsync(host_y, op->yv, (size_t)m * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return 0;
 }
 
@@ -1451,6 +1555,48 @@ extern "C" int smcp_dense_gemm(smcp_ctx *ctx, int ta, int tb, const double *A_ho
     if (launch_gemm(ctx, ta != 0, tb != 0, A.p, lda, B.p, ldb, Cd.p, ldc, M, N, K, alpha, accumulate, tri, 0, "dense_gemm_dmma")) return -1;
     CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
     CUDA_TRY(cudaMemcpyAsync(C_host, Cd.p, nc * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    if (ms_out) {
+        float ms = 0.f;
+        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+        *ms_out = ms;
+    }
+    return 0;
+}
+
+extern "C" int smcp_dense_geqrf(smcp_ctx *ctx, double *A_host, int64_t lda, int64_t M, int64_t N, double *tau_host, double *ms_out) {
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    if (N < 1 || M < N || lda < M) { smcp_set_error("smcp_dense_geqrf: bad arguments (needs 1 <= N <= M <= lda)"); return -2; }
+    DevBuf A, T;
+    CUDA_TRY(cudaMalloc(&A.p, (size_t)lda * N * sizeof(double)));
+    CUDA_TRY(cudaMalloc(&T.p, (size_t)N * sizeof(double)));
+    CUDA_TRY(cudaMemcpyAsync(A.p, A_host, (size_t)lda * N * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
+    if (d_geqrf(ctx, A.p, lda, M, N, T.p)) return -1;
+    CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(A_host, A.p, (size_t)lda * N * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(tau_host, T.p, (size_t)N * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    if (ms_out) {
+        float ms = 0.f;
+        CUDA_TRY(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+        *ms_out = ms;
+    }
+    return 0;
+}
+
+extern "C" int smcp_dense_orgqr(smcp_ctx *ctx, double *A_host, int64_t lda, int64_t M, int64_t N, const double *tau_host, double *ms_out) {
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    if (N < 1 || M < N || lda < M) { smcp_set_error("smcp_dense_orgqr: bad arguments (needs 1 <= N <= M <= lda)"); return -2; }
+    DevBuf A, T;
+    CUDA_TRY(cudaMalloc(&A.p, (size_t)lda * N * sizeof(double)));
+    CUDA_TRY(cudaMalloc(&T.p, (size_t)N * sizeof(double)));
+    CUDA_TRY(cudaMemcpyAsync(A.p, A_host, (size_t)lda * N * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(T.p, tau_host, (size_t)N * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
+    if (d_orgqr(ctx, A.p, lda, M, N, T.p)) return -1;
+    CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(A_host, A.p, (size_t)lda * N * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (ms_out) {
         float ms = 0.f;

@@ -84,6 +84,8 @@ struct smcp_ctx {
     int lane_cur = 0;                   // lane whose members are currently swapped in
     int lanes_active = 0;               // > 1 between lanes_fork and lanes_join
     cudaEvent_t lane_fork_ev = nullptr;
+    double *qr_ws = nullptr;            // blocked Householder QR (qr.cu): V | Y | W | partial sums
+    size_t qr_ws_cap = 0;
     // pinned staging for small host<->device transfers
     void *pinned = nullptr;
     size_t pinned_bytes = 0;
@@ -329,6 +331,14 @@ bool potrf_tile_fits(const smcp_ctx *ctx, int64_t mm, int64_t npiv, bool panel_o
 int potrf_tile(smcp_ctx *ctx, double *H, int64_t ld, int64_t mm, int64_t npiv, bool panel_only, int32_t *info_dev, int col_off);
 bool trsm_slab_fits(int64_t n);
 int trsm_slab(smcp_ctx *ctx, bool trans, const double *L, int64_t ldl, int64_t n, double *B, int64_t ldb, int64_t nrhs);
+// blocked Householder QR of an M x N matrix, M >= N (qr.cu): lapack.geqrf / lapack.orgqr semantics in place
+int d_geqrf(smcp_ctx *ctx, double *A, int64_t lda, int64_t M, int64_t N, double *tau_dev);
+int d_orgqr(smcp_ctx *ctx, double *A, int64_t lda, int64_t M, int64_t N, const double *tau_dev);
+// L = R^T (lower, leading dimension ldl) with diag(L) >= 0 from the R of d_geqrf; sgn[i] = sign of R(i, i);
+// info_dev = first k (1-based) with |R_kk| <= 1e-14 max |R_ii|, 0 if none
+int qr_extract_lower(smcp_ctx *ctx, const double *A, int64_t lda, int64_t m, double *L, int64_t ldl, double *sgn, int *info_dev);
+// column c of A (M x N) times sgn[c]
+int qr_apply_colsign(smcp_ctx *ctx, double *A, int64_t lda, int64_t M, int64_t N, const double *sgn);
 // TMA-fed DMMA GEMM for K-major operands (gemm_tma.cu)
 bool gemm_tma_eligible(const double *A, int64_t lda, const double *B, int64_t ldb, int64_t M, int64_t N, int64_t K);
 int launch_gemm_tma_tn(smcp_ctx *ctx, const double *A, int64_t lda, const double *B, int64_t ldb, double *C, int64_t ldc,

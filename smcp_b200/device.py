@@ -82,6 +82,8 @@ API = {
     "smcp_kkt_assemble_syrk": (_int, [_vp, _vp]),
     "smcp_kkt_z_tmul": (_int, [_vp, _dp, _f64p]),
     "smcp_kkt_z_mul": (_int, [_vp, _f64p, _dp]),
+    "smcp_kkt_factor_qr": (_int, [_vp, _vp, _i32p]),
+    "smcp_kkt_qr_solve": (_int, [_vp, _dp, _f64p, _f64p, _dp]),
     "smcp_kkt_factor": (_int, [_vp, _i32p]),
     "smcp_kkt_factor_dist": (_int, [_vp, _int, _int, _i32p]),
     "smcp_kkt_factor_block": (_int, [_vp, _i64, _int, _int, _i32p]),
@@ -89,6 +91,8 @@ API = {
     "smcp_dense_trsm": (_int, [_vp, _int, _f64p, _i64, _i64, _f64p, _i64, _i64, C.POINTER(_dbl)]),
     "smcp_dense_gemm": (_int, [_vp, _int, _int, _f64p, _i64, _f64p, _i64, _f64p, _i64, _i64, _i64, _i64, _dbl, _int, _int,
                                C.POINTER(_dbl)]),
+    "smcp_dense_geqrf": (_int, [_vp, _f64p, _i64, _i64, _i64, _f64p, C.POINTER(_dbl)]),
+    "smcp_dense_orgqr": (_int, [_vp, _f64p, _i64, _i64, _i64, _f64p, C.POINTER(_dbl)]),
     "smcp_kkt_solve": (_int, [_vp, _f64p]),
     "smcp_kkt_get_H": (_int, [_vp, _f64p]),
     "smcp_kkt_set_H": (_int, [_vp, _f64p]),
@@ -564,6 +568,27 @@ class DeviceBackend:
         _ck(self.lib, self.lib.smcp_kkt_factor(self._op, info))
         if info[0]:
             raise ArithmeticError("Z = G(A) is rank deficient (info=%d)" % info[0])
+
+    # -- kktsolver='qr' in Householder form (options['qr_method'] = 'householder') -------------------
+    def schur_factor_householder(self, tok):
+        """Zw = Q1 R on the device: Q1 replaces Zw, L = R^T (diag >= 0) becomes the factor of H."""
+        info = np.zeros(1, dtype=np.int32)
+        _ck(self.lib, self.lib.smcp_kkt_factor_qr(self._op, tok, info))
+        if info[0]:
+            raise ArithmeticError("Z = G(A) is rank deficient (info=%d)" % info[0])
+
+    def qr_solve(self, g_buf, r):
+        """y = H^-1 (r + Z^T g) and X = Z y - g through Q1 and L (``smcp_kkt_qr_solve``)."""
+        TRAFFIC["h2d"] += 8 * self.m
+        TRAFFIC["d2h"] += 8 * self.m
+        y = np.empty(self.m)
+        p = self._alloc(False)
+        try:
+            _ck(self.lib, self.lib.smcp_kkt_qr_solve(self._op, g_buf, np.ascontiguousarray(r, dtype=np.float64).ravel(), y, p))
+        except DeviceError:
+            self.release(p)
+            raise
+        return y, p
 
     def gram_factor(self):
         """Cholesky factor of the Gram matrix <A_i, A_j> (trace inner product) of the constraints: the

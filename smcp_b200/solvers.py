@@ -7,7 +7,8 @@ Public surface (drop-in for ``smcp.solvers``, reference ``src/python/solvers.py`
 * ``chordalsolver_esd(A, b, ...)``  – extended self-dual embedding (``solvers.py:1330-2467``)
 * ``conelp(c, G, h, dims)``         – CVXOPT-style cone-LP front end (``solvers.py:2470-2599``)
 
-``kktsolver='chol'`` is the north-star path; ``'qr'`` is provided in its SYRK form (``_KKTqr``).
+``kktsolver='chol'`` is the north-star path; ``'qr'`` is provided in its SYRK form (``_KKTqr``, the default)
+and, with ``options['qr_method'] = 'householder'``, in the reference's Householder form (``_KKTqrh``).
 
 The numerical work of every iteration — chordal Cholesky / completion / projected inverse,
 the barrier Hessian, the dense Schur complement and its Cholesky, step-length probes and
@@ -42,6 +43,9 @@ options = {
     "prediction": True, "step": 0.98,
     # extension (not in the reference): relaxed supernodes, see smcp_b200.symbolic.amalgamate; 0 = the reference's pattern
     "amalgamation": 0.0,
+    # extension: how kktsolver='qr' factors Z = [G(A_1) ... G(A_m)]: 'syrk' (H = Z^T Z and its Cholesky factor)
+    # or 'householder' (Z = Q R on the device, Newton solves through Q and R like the reference's kkt_qr)
+    "qr_method": "syrk",
 }
 
 _backend_factory = None
@@ -110,6 +114,9 @@ def _read_options(n, feas):
     o.amalgamation = g.get("amalgamation", 0.0)
     _check(type(o.amalgamation) in (float, int) and 0.0 <= o.amalgamation < 1.0, ValueError,
            "options['amalgamation'] must be a number in [0, 1)")
+    o.qr_method = g.get("qr_method", "syrk")
+    _check(o.qr_method in ("syrk", "householder"), ValueError,
+           "options['qr_method'] must be 'syrk' or 'householder'")
     if feas:
         o.alpha = g["alpha"]
         _check(type(o.alpha) is float and 0.0 < o.alpha < 0.5, TypeError,
@@ -149,6 +156,7 @@ class _Problem:
         if kktsolver not in ("chol", "qr"):
             raise ValueError("Unknown 'kktsolver'.")
         self.kktsolver = kktsolver
+        self.qr_method = opt.qr_method
         A = misc.as_csc(A)
         self.m = m = A.shape[1] - 1
         self.n = n = int(math.sqrt(A.shape[0]))
@@ -318,8 +326,34 @@ class _KKTqr:
         return x, y
 
 
+class _KKTqrh:
+    """``kkt_qr`` as the reference computes it (``lapack.geqrf / ormqr / trtrs``), ``options['qr_method'] =
+    'householder'``: with the weights w of the trace inner product, Zw = diag(sqrt(w)) Z = Q1 R by a blocked
+    Householder QR on the device, and the solve goes through Q1 and R:
+        gw = sqrt(w) G(bx),  v = R^-T (kk*by) + Q1^T gw,  y = R^-1 v,  x = (1/kk) G^adj((Q1 v - gw) / sqrt(w)).
+    This equals ``_KKTqr.solve`` in exact arithmetic (Z y = Q1 R y = Q1 v); it never forms Z^T Z, whose
+    condition number is that of Z squared."""
+
+    def __init__(self, prob, L, Y, scaling):
+        self.prob, self.L, self.Y, self.scaling = prob, L, Y, scaling
+        prob.ops.schur_factor_householder(schur_token(L, Y))      # raises ArithmeticError if Z is rank deficient
+
+    def solve(self, bx, by, t):
+        kk = 1.0 / t if self.scaling == "primal" else t
+        ops = self.prob.ops
+        r1 = bx.copy()
+        hessian(self.L, self.Y, [r1], inv=False, adj=False)
+        y, xbuf = ops.qr_solve(r1.buf, kk * np.asarray(by, dtype=np.float64))
+        x = cspmatrix(ops, xbuf)
+        hessian(self.L, self.Y, [x], inv=False, adj=True)
+        x.scale(1.0 / kk)
+        return x, y
+
+
 def _make_kkt(prob, L, Y, scaling):
-    return (_KKTqr if prob.kktsolver == "qr" else _KKT)(prob, L, Y, scaling)
+    if prob.kktsolver == "qr":
+        return (_KKTqrh if prob.qr_method == "householder" else _KKTqr)(prob, L, Y, scaling)
+    return _KKT(prob, L, Y, scaling)
 
 
 def _nrm2(v):
