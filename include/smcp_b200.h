@@ -151,6 +151,11 @@ int smcp_op_destroy(smcp_op *op);
  * needed by the sparse-constraint technique (the Ip/Jp/Kl arguments of misc.SCMcolumn2,
  * src/C/misc.c:620-663) */
 int smcp_op_set_entry_coords(smcp_op *op, const int64_t *rows_int, const int64_t *cols_int);
+/* rows of the dense weighted constraint copy built at smcp_op_create for the "dense" constraints:
+ * 0 without one (no dense constraint), |blkval| for the full copy, the number of distinct rows of blkval
+ * any constraint touches for the support copy (chosen when they are at most a quarter of |blkval|;
+ * SMCP_B200_AVW_SUPPORT=0 / =1 forces the full / the support copy) */
+int smcp_op_dense_rows(smcp_op *op, int64_t *rows_out);
 /* Amap: v = 2*Av^T*vec_half(X) (solvers.py:369-378); col >= 0 evaluates one entry only    */
 int smcp_op_amap(smcp_op *op, const double *X, int64_t col, double *host_out);
 /* Aadj: X = mat(Av*y) (solvers.py:380-384) */

@@ -232,7 +232,10 @@ class SDP(object):
         opt = solvers._read_options(n, True)
         prob = solvers._Problem(A, self.b, opt, "qr", None)          # 'qr': no constraint reordering (Ns = 0)
         ops, symb, pm = prob.ops, prob.symb, prob.p
-        dense_bytes = 8.0 * symb.nblk * m
+        # the product runs over the rows of the backend's dense constraint copy: all of blkval, or on filled
+        # patterns only the rows the constraints touch (a backend without dense_rows() contracts over all)
+        rows = ops.dense_rows() if hasattr(ops, "dense_rows") else symb.nblk
+        dense_bytes = 8.0 * rows * m
         if dense_bytes <= (16 << 30):
             ops.gram_factor()
             u = ops.schur_solve(prob.b)

@@ -583,6 +583,14 @@ struct smcp_op {
     double *r_val = nullptr;
     // dense weighted copy w.Av (nblk x m) for the DMMA assembly (only if md > 0)
     double *AvW = nullptr;
+    // ... or, when few rows of blkval are touched by any constraint (filled patterns), the same copy on
+    // those rows only: AvWs (lds x m, lds = nsup rounded up to even) on the sorted support rows sup[0..nsup),
+    // srow[p] = position of rowblk[p] in sup.  Exactly one of AvW / AvWs is set when md > 0.
+    double *AvWs = nullptr;
+    int *sup = nullptr, *srow = nullptr;
+    long long nsup = 0, lds = 0;
+    double *Ubs = nullptr;        // Hessian batch gathered onto the support rows (lds x ncols)
+    size_t Ubs_cap = 0;
     double *H = nullptr;
     int *info_dev = nullptr;
     double *yv = nullptr;
@@ -613,19 +621,23 @@ __global__ void amap_kernel(const long long *__restrict__ colptr, const int *__r
 
 // dense variant for (nearly) dense Av: column c of the weighted dense copy AvW is contiguous, one CTA
 // per column streams it once (coalesced 8-byte loads, 4 independent accumulators per thread) against
-// X, which stays in L2; fixed reduction tree -> deterministic.
-__global__ void __launch_bounds__(256) amap_dense_kernel(const double *__restrict__ AvW, long long nblk,
-                                                         const double *__restrict__ X, double *out, long long col0) {
-    const double *a = AvW + (col0 + blockIdx.x) * nblk;
+// X, which stays in L2; fixed reduction tree -> deterministic.  SUP: the copy holds the support rows
+// only (AvWs, column stride lda), row r of it multiplies X[sup[r]].
+template <bool SUP>
+__global__ void __launch_bounds__(256) amap_dense_kernel(const double *__restrict__ AvW, long long lda, long long nblk,
+                                                         const int *__restrict__ sup, const double *__restrict__ X,
+                                                         double *out, long long col0) {
+    const double *a = AvW + (col0 + blockIdx.x) * lda;
+    auto x = [&](long long r) { return SUP ? X[sup[r]] : X[r]; };
     double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
     long long r = threadIdx.x;
     for (; r + 768 < nblk; r += 1024) {
-        s0 = fma(a[r], X[r], s0);
-        s1 = fma(a[r + 256], X[r + 256], s1);
-        s2 = fma(a[r + 512], X[r + 512], s2);
-        s3 = fma(a[r + 768], X[r + 768], s3);
+        s0 = fma(a[r], x(r), s0);
+        s1 = fma(a[r + 256], x(r + 256), s1);
+        s2 = fma(a[r + 512], x(r + 512), s2);
+        s3 = fma(a[r + 768], x(r + 768), s3);
     }
-    for (; r < nblk; r += 256) s0 = fma(a[r], X[r], s0);
+    for (; r < nblk; r += 256) s0 = fma(a[r], x(r), s0);
     double s = (s0 + s1) + (s2 + s3);
     __shared__ double sh[8];
     for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
@@ -656,6 +668,27 @@ __global__ void scatter_cols_kernel(const long long *__restrict__ colptr, const 
     if (c >= ncols) return;
     double *u = U + (long long)c * ldu;
     for (long long p = colptr[c0 + c] + threadIdx.x; p < colptr[c0 + c + 1]; p += blockDim.x) u[rowblk[p]] = vals[p];
+}
+
+// as scatter_cols_kernel onto the support rows (compact row srow[p]), each value times scale[rowblk[p]] if scale is set
+__global__ void scatter_support_kernel(const long long *__restrict__ colptr, const int *__restrict__ srow,
+                                       const int *__restrict__ rowblk, const double *__restrict__ vals,
+                                       const double *__restrict__ scale, double *U, long long ldu, long long c0, int ncols) {
+    int c = blockIdx.x;
+    if (c >= ncols) return;
+    double *u = U + (long long)c * ldu;
+    for (long long p = colptr[c0 + c] + threadIdx.x; p < colptr[c0 + c + 1]; p += blockDim.x)
+        u[srow[p]] = scale ? vals[p] * scale[rowblk[p]] : vals[p];
+}
+
+// Ubs[k + j lds] = Ub[sup[k] + j nblk] for k < nsup, 0 on the padding rows k in [nsup, lds)
+__global__ void support_gather_kernel(const double *__restrict__ Ub, long long nblk, const int *__restrict__ sup, long long nsup,
+                                      long long lds, double *__restrict__ Ubs, long long ncols) {
+    const long long total = lds * ncols;
+    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
+        const long long k = idx % lds, j = idx / lds;
+        Ubs[idx] = k < nsup ? Ub[sup[k] + j * nblk] : 0.0;
+    }
 }
 
 template <class T>
@@ -714,7 +747,35 @@ extern "C" int smcp_op_create(smcp_sym *s, int64_t m, int64_t Ns, const int64_t 
     CUDA_TRY(cudaMalloc(&op->info_dev, 64));
     CUDA_TRY(cudaMalloc(&op->yv, (size_t)(m + 1) * sizeof(double)));
     CUDA_TRY(cudaMalloc(&op->Dinv, (size_t)((m + 63) / 64 + 1) * 64 * 64 * sizeof(double)));
+    // rows of blkval that some constraint touches (all m columns: the rows of H below the dense block come from
+    // the same product); the dense copy keeps only those when they are at most a quarter of blkval.
+    // SMCP_B200_AVW_SUPPORT=0 / =1 forces the full / the support copy.
+    bool support = false;
+    std::vector<int> sup, srow;
     if (op->md > 0) {
+        std::vector<int> cidx(nblk, -1);
+        for (int64_t p = 0; p < nnz; ++p) cidx[rb[p]] = 0;
+        for (int r = 0; r < nblk; ++r)
+            if (cidx[r] == 0) { cidx[r] = (int)sup.size(); sup.push_back(r); }
+        const char *env = getenv("SMCP_B200_AVW_SUPPORT");
+        const int mode = env && !strcmp(env, "0") ? 0 : env && !strcmp(env, "1") ? 1 : -1;
+        support = !sup.empty() && (mode == 1 || (mode == -1 && (double)sup.size() <= 0.25 * (double)nblk));
+        if (support) {
+            srow.resize(nnz);
+            for (int64_t p = 0; p < nnz; ++p) srow[p] = cidx[rb[p]];
+        }
+    }
+    if (support) {
+        op->nsup = (long long)sup.size();
+        op->lds = (op->nsup + 1) & ~1LL;          // even: 16-byte aligned columns for the TMA operand path
+        if (dev_upload(sup, &op->sup) || dev_upload(srow, &op->srow)) return -1;
+        size_t bytes = (size_t)op->lds * (size_t)m * sizeof(double);
+        CUDA_TRY(cudaMalloc(&op->AvWs, bytes));
+        CUDA_TRY(cudaMemsetAsync(op->AvWs, 0, bytes, ctx->stream));
+        LaunchScope ls(ctx, "setup");
+        scatter_support_kernel<<<(unsigned)m, 128, 0, ctx->stream>>>(op->colptr, op->srow, op->rowblk, op->valsw, nullptr, op->AvWs,
+                                                                     op->lds, 0, (int)m);
+    } else if (op->md > 0) {
         // dense weighted copy of all m columns (rows of H below the dense block included)
         size_t bytes = (size_t)nblk * (size_t)m * sizeof(double);
         CUDA_TRY(cudaMalloc(&op->AvW, bytes));
@@ -786,6 +847,8 @@ extern "C" int smcp_op_destroy(smcp_op *op) {
     if (op->sp_pid) { cudaFree(op->sp_pid); cudaFree(op->pos_r); cudaFree(op->pos_c); }
     if (op->ent_c) cudaFree(op->ent_c);
     if (op->AvW) cudaFree(op->AvW);
+    if (op->AvWs) { cudaFree(op->AvWs); cudaFree(op->sup); cudaFree(op->srow); }
+    if (op->Ubs) cudaFree(op->Ubs);
     if (op->Ub) cudaFree(op->Ub);
     if (op->Zinv) cudaFree(op->Zinv);
     if (op->Kpos) cudaFree(op->Kpos);
@@ -806,7 +869,10 @@ extern "C" int smcp_op_amap(smcp_op *op, const double *X, int64_t col, double *h
     if (ncols == 0) return 0;
     if (op->AvW && op->nnz * 4 >= (int64_t)op->sym->d.nblk * op->m) {
         LaunchScope ls(ctx, "amap_dense", 1, 8.0 * (double)op->sym->d.nblk * ncols);
-        amap_dense_kernel<<<ncols, 256, 0, ctx->stream>>>(op->AvW, op->sym->d.nblk, X, op->yv, c0);
+        amap_dense_kernel<false><<<ncols, 256, 0, ctx->stream>>>(op->AvW, op->sym->d.nblk, op->sym->d.nblk, nullptr, X, op->yv, c0);
+    } else if (op->AvWs && op->nnz * 4 >= op->nsup * op->m) {
+        LaunchScope ls(ctx, "amap_dense", 1, 12.0 * (double)op->nsup * ncols);
+        amap_dense_kernel<true><<<ncols, 256, 0, ctx->stream>>>(op->AvWs, op->lds, op->nsup, op->sup, X, op->yv, c0);
     } else {
         LaunchScope ls(ctx, "amap", 1, 12.0 * (double)(op->h_colptr[c0 + ncols] - op->h_colptr[c0]));
         amap_kernel<<<(ncols * 32 + 255) / 256, 256, 0, ctx->stream>>>(op->colptr, op->rowblk, op->valsw, X, op->yv, c0, ncols);
@@ -814,6 +880,11 @@ extern "C" int smcp_op_amap(smcp_op *op, const double *X, int64_t col, double *h
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(host_out, op->yv, (size_t)ncols * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+extern "C" int smcp_op_dense_rows(smcp_op *op, int64_t *rows_out) {
+    *rows_out = op->AvWs ? op->nsup : op->AvW ? op->sym->d.nblk : 0;
     return 0;
 }
 
@@ -1040,7 +1111,9 @@ static int assemble_dense_ranges(smcp_op *op, smcp_hess *h, const std::vector<st
     const int64_t m = op->m;
     const long long nblk = s->d.nblk;
     if (ranges.empty()) return 0;
-    size_t per_col = ((size_t)nblk + (size_t)s->d.nupd) * sizeof(double);
+    // support copy: the Hessian batch is gathered onto the support rows and contracted over K = nsup of them
+    const bool support = op->AvWs != nullptr;
+    size_t per_col = ((size_t)nblk + (size_t)s->d.nupd + (support ? (size_t)op->lds : 0)) * sizeof(double);
     int64_t cap = (int64_t)std::max<size_t>(1, ((size_t)6 << 30) / per_col);
     cap = std::min<int64_t>(cap, 2048);
     // split ranges that exceed the capacity, then group consecutive pieces up to `cap` columns
@@ -1065,11 +1138,21 @@ static int assemble_dense_ranges(smcp_op *op, smcp_hess *h, const std::vector<st
             off += nc;
         }
         if (k_hess_apply(h, op->Ub, ncols, 0)) return -1;
+        if (support) {
+            if (grow((void **)&op->Ubs, &op->Ubs_cap, (size_t)ncols * op->lds * sizeof(double))) return -1;
+            const long long total = (long long)ncols * op->lds;
+            LaunchScope ls(ctx, "support_gather", 1, 20.0 * (double)op->nsup * (double)ncols);
+            support_gather_kernel<<<(unsigned)std::min<long long>((total + 255) / 256, (long long)ctx->num_sms * 16), 256, 0, ctx->stream>>>(
+                op->Ub, nblk, op->sup, op->nsup, op->lds, op->Ubs, ncols);
+        }
         off = 0;
         for (size_t q = gi; q < ge; ++q) {
             const int64_t c0 = pieces[q].first, nc = pieces[q].second - c0;
             // H[c0:m, c0:c0+nc] = (w.Av[:, c0:m])^T W
-            if (d_gemm_tn(ctx, op->AvW + (size_t)c0 * nblk, nblk, op->Ub + (size_t)off * nblk, nblk, op->H + c0 + c0 * m, m, m - c0, nc, nblk, 0)) return -1;
+            if (support) {
+                if (d_gemm_tn(ctx, op->AvWs + (size_t)c0 * op->lds, op->lds, op->Ubs + (size_t)off * op->lds, op->lds, op->H + c0 + c0 * m, m,
+                              m - c0, nc, op->nsup, 0)) return -1;
+            } else if (d_gemm_tn(ctx, op->AvW + (size_t)c0 * nblk, nblk, op->Ub + (size_t)off * nblk, nblk, op->H + c0 + c0 * m, m, m - c0, nc, nblk, 0)) return -1;
             off += nc;
         }
         gi = ge;
@@ -1260,6 +1343,16 @@ __global__ void __launch_bounds__(256) zmul_kernel(const double *__restrict__ Z,
     if (r < nblk) x[r] = (s0 + s1) + (s2 + s3);
 }
 
+static int ensure_sqrtw(smcp_op *op) {
+    smcp_sym *s = op->sym;
+    if (!op->sqrtw) {
+        const long long nblk = s->d.nblk;
+        CUDA_TRY(cudaMalloc(&op->sqrtw, (size_t)nblk * sizeof(double)));
+        sqrtw_kernel<<<(unsigned)((nblk + 255) / 256), 256, 0, s->ctx->stream>>>(s->d.wdot, op->sqrtw, nblk);
+    }
+    return 0;
+}
+
 // Zw = diag(sqrt(wdot)) [G(A_1) ... G(A_m)] in op->Zq (G = identity when h is NULL)
 static int form_zw(smcp_op *op, smcp_hess *h, const char *who) {
     smcp_sym *s = op->sym;
@@ -1271,10 +1364,7 @@ static int form_zw(smcp_op *op, smcp_hess *h, const char *who) {
     if (bytes > ((size_t)96 << 30)) { smcp_set_error("kktsolver='qr' needs m*|blkval| doubles (%.1f GB)", bytes / 1073741824.0); return -2; }
     op->zq_state = 0;
     if (!op->Zq) CUDA_TRY(cudaMalloc(&op->Zq, bytes ? bytes : 8));
-    if (!op->sqrtw) {
-        CUDA_TRY(cudaMalloc(&op->sqrtw, (size_t)nblk * sizeof(double)));
-        sqrtw_kernel<<<(unsigned)((nblk + 255) / 256), 256, 0, ctx->stream>>>(s->d.wdot, op->sqrtw, nblk);
-    }
+    if (ensure_sqrtw(op)) return -1;
     CUDA_TRY(cudaMemsetAsync(op->Zq, 0, bytes, ctx->stream));
     {
         LaunchScope ls(ctx, "scatter_cols");
@@ -1301,6 +1391,25 @@ extern "C" int smcp_kkt_assemble_syrk(smcp_op *op, smcp_hess *h) {
     RegionScope rs(ctx, "kkt_assemble");
     const int64_t m = op->m;
     const long long nblk = op->sym->d.nblk;
+    if (!h && op->AvWs) {
+        // Gram matrix sum_p w_p A_pi A_pj of the constraints over the support rows: one triangular product with
+        // K = nsup of the sqrt(w)-weighted support copy (in the Ubs workspace; Zq is not formed and stays refused
+        // by smcp_kkt_z_tmul / z_mul)
+        if (op->Ns) { smcp_set_error("smcp_kkt_assemble_syrk: the sparse-constraint technique does not apply (Ns must be 0)"); return -2; }
+        op->zq_state = 0;
+        if (ensure_sqrtw(op)) return -1;
+        const size_t bytes = (size_t)op->lds * (size_t)m * sizeof(double);
+        if (grow((void **)&op->Ubs, &op->Ubs_cap, bytes)) return -1;
+        CUDA_TRY(cudaMemsetAsync(op->Ubs, 0, bytes, ctx->stream));
+        {
+            LaunchScope ls(ctx, "scatter_cols");
+            scatter_support_kernel<<<(unsigned)m, 128, 0, ctx->stream>>>(op->colptr, op->srow, op->rowblk, op->vals, op->sqrtw, op->Ubs,
+                                                                         op->lds, 0, (int)m);
+        }
+        if (launch_gemm(ctx, true, true, op->Ubs, op->lds, op->Ubs, op->lds, op->H, m, m, m, op->nsup, 1.0, 0, 1, 0, "schur_syrk_dmma")) return -1;
+        CUDA_TRY(cudaGetLastError());
+        return 0;
+    }
     if (int rc = form_zw(op, h, "smcp_kkt_assemble_syrk")) return rc;
     if (launch_gemm(ctx, true, true, op->Zq, nblk, op->Zq, nblk, op->H, m, m, m, nblk, 1.0, 0, 1, 0, "schur_syrk_dmma")) return -1;
     CUDA_TRY(cudaGetLastError());
@@ -1321,7 +1430,7 @@ extern "C" int smcp_kkt_z_tmul(smcp_op *op, const double *X, double *host_out) {
     }
     {
         LaunchScope ls(ctx, "amap_dense", 1, 8.0 * (double)nblk * (double)op->m);
-        amap_dense_kernel<<<(unsigned)op->m, 256, 0, ctx->stream>>>(op->Zq, nblk, s->tmp, op->yv, 0);
+        amap_dense_kernel<false><<<(unsigned)op->m, 256, 0, ctx->stream>>>(op->Zq, nblk, nblk, nullptr, s->tmp, op->yv, 0);
     }
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(host_out, op->yv, (size_t)op->m * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1415,7 +1524,7 @@ extern "C" int smcp_kkt_qr_solve(smcp_op *op, const double *G_dev, const double 
         if (d_trs_cluster(ctx, op->H, m, m, op->Dinv, rv, m, 1, 1, 0, "potrs")) return -1;        // a = L^-1 r
         {
             LaunchScope ls(ctx, "qr_qmul", 1, 8.0 * (double)nblk * (double)m);
-            amap_dense_kernel<<<(unsigned)m, 256, 0, ctx->stream>>>(op->Zq, nblk, gw, op->yv, 0);      // c = Q1^T gw
+            amap_dense_kernel<false><<<(unsigned)m, 256, 0, ctx->stream>>>(op->Zq, nblk, nblk, nullptr, gw, op->yv, 0);      // c = Q1^T gw
         }
         {
             LaunchScope ls(ctx, "level1");

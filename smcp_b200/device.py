@@ -75,6 +75,7 @@ API = {
     "smcp_op_create": (_int, [_vp, _i64, _i64, _i64p, _i64p, _f64p, C.POINTER(_vp)]),
     "smcp_op_destroy": (_int, [_vp]),
     "smcp_op_set_entry_coords": (_int, [_vp, _i64p, _i64p]),
+    "smcp_op_dense_rows": (_int, [_vp, C.POINTER(_i64)]),
     "smcp_op_amap": (_int, [_vp, _dp, _i64, _f64p]),
     "smcp_op_aadj": (_int, [_vp, _f64p, _dp]),
     "smcp_kkt_assemble": (_int, [_vp, _vp, _i64, _i64]),
@@ -521,6 +522,13 @@ class DeviceBackend:
             ri = symb.iperm[symb.Ip[rowind]]
             ci = symb.iperm[symb.Jp[rowind]]
             _ck(self.lib, self.lib.smcp_op_set_entry_coords(h, _i64(ri), _i64(ci)))
+
+    def dense_rows(self):
+        """Rows of the dense constraint copy on the device: 0 (no dense constraint), ``symb.nblk`` (full
+        copy) or the number of rows any constraint touches (support copy)."""
+        out = C.c_int64()
+        _ck(self.lib, self.lib.smcp_op_dense_rows(self._op, C.byref(out)))
+        return out.value
 
     def Amap(self, buf):
         TRAFFIC["d2h"] += 8 * self.m
