@@ -132,6 +132,23 @@ int smcp_csp_probe(smcp_sym *sym, int kind, const double *x, const double *dx,
 /* chompack.trsm(L, B[, trans='T']): B (n x nrhs, column-major, rows in Vp order, DEVICE) */
 int smcp_csp_trsm(smcp_sym *sym, const double *L, double *B_dev, int64_t ldb, int64_t nrhs, int trans);
 
+/* ---- randomized rounding (an extension: the reference has none) ------------------------------
+ * Gaussian samples of the max-det completion: with L from smcp_csp_completion (P_V((L L^T)^-1) = X),
+ * B[:, c] = L^-T g_{col0+c}, c = 0..k-1, g_j the standard normal vector of sample j under `seed`
+ * (Philox4x64-10, Box-Muller; entry i of sample j depends only on (seed, j, i)).
+ * B: n x k column-major on the device, rows in the internal order of sym. */
+int smcp_csp_sample(smcp_sym *sym, const double *L, uint64_t seed, int64_t col0,
+                    double *B_dev, int64_t ldb, int64_t k);
+/* ±1 rounding: trials t = 0..trials-1 of s_t = sign(L^-T g_t); values_host[t] = sum over the nc
+ * lower-triangular objective entries (internal coordinates, host arrays) of c s_r s_c (x2 off the diagonal);
+ * x_host = s of the smallest value (lowest t on ties), *best_out = that t.  `chunk` trials per pass
+ * (0: as many as fit in 1 GiB of n x chunk doubles), rounded up to whole solve blocks: the trials are solved in
+ * blocks of equal width, at most 256 columns, so every output is independent of chunk.  The workspace is
+ * allocated once per call; nothing of size n x trials leaves the device. */
+int smcp_round_pm1(smcp_sym *sym, const double *L, uint64_t seed, int64_t trials, int64_t chunk,
+                   int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
+                   double *values_host, int8_t *x_host, int64_t *best_out);
+
 /* ---- barrier Hessian: chompack.hessian(L, Y, U, adj=None, inv=...) ---------------------- */
 int smcp_hess_create(smcp_sym *sym, const double *L, const double *Y, smcp_hess **out);
 int smcp_hess_destroy(smcp_hess *h);

@@ -22,7 +22,7 @@ import scipy.sparse.linalg as spla
 from . import misc, solvers
 from .symbolic import Symbolic, embed, maxcardsearch, min_degree, lower_pattern
 
-__all__ = ["SDP", "band_SDP", "mtxnorm_SDP", "rand_SDP", "maxcut_SDP", "mk_rand", "completion"]
+__all__ = ["SDP", "band_SDP", "mtxnorm_SDP", "rand_SDP", "maxcut_SDP", "mk_rand", "completion", "completion_sample"]
 
 
 class SDP(object):
@@ -294,6 +294,35 @@ class SDP(object):
         X0 = (Xz[:n, :n] - s * sp.identity(n, format="csc")).tocsc()
         return X0, sol
 
+    # -- rounding (an extension: the reference has none) ---------------------------------
+    def round_pm1(self, sol, trials=256, seed=0, chunk=0):
+        """Goemans-Williamson rounding of a solution with diag(X) = 1: ``trials`` sign vectors
+        s_t = sign(v_t), v_t drawn with covariance the max-det completion of ``sol['x']``
+        (``completion_sample``), evaluated against the objective C on the device; ``chunk`` trials per pass
+        (0: as many as fit in 1 GiB), with no effect on the result.  Returns a dict: ``x`` (int8 +-1, original
+        order) of the smallest C . x x^T (lowest trial on ties), ``value`` = C . x x^T, ``values`` of every
+        trial and ``trial``, the index of the best one.  Raises ``ArithmeticError`` if X has no positive
+        definite completion."""
+        trials = _check_count(trials, "trials", 1)
+        seed = _check_seed(seed)
+        chunk = _check_count(chunk, "chunk", 0)
+        if not isinstance(sol, dict) or "x" not in sol:
+            raise ValueError("sol must be a solution dict holding 'x'")
+        L, order = _completion_factor(sol["x"])
+        n = self.n
+        if len(order) != n:
+            raise ValueError("sol['x'] is %d x %d, the problem has n = %d" % (len(order), len(order), n))
+        A = self._need()
+        r = A.indices[A.indptr[0]:A.indptr[1]]
+        I, J = misc.ind2sub(n, r)
+        pos = np.empty(n, dtype=np.int64)
+        pos[order] = np.arange(n, dtype=np.int64)
+        values, xi, best = L.ops.round_pm1(L.buf, pos[np.asarray(I)], pos[np.asarray(J)],
+                                           A.data[A.indptr[0]:A.indptr[1]], trials, seed, chunk)
+        x = np.empty(n, dtype=np.int8)
+        x[order] = xi
+        return {"x": x, "value": float(values[best]), "values": values, "trial": int(best)}
+
 
 # --------------------------------------------------------------------------------------
 # generators
@@ -513,12 +542,20 @@ class maxcut_SDP(SDP):
         self._b = np.ones(n)
         self._pname = "maxcut_n%i" % n
 
+    def cut(self, sol, trials=256, seed=0):
+        """A cut from a solution of the relaxation by Goemans-Williamson rounding (``SDP.round_pm1``):
+        returns ``(x, weight, bound)`` with the +-1 vector x of the heaviest of ``trials`` random hyperplane
+        cuts, its weight (= -C . x x^T) and the certified upper bound -``sol['dual objective']`` on every
+        cut's weight."""
+        r = self.round_pm1(sol, trials=trials, seed=seed)
+        return r["x"], -r["value"], -float(sol["dual objective"])
 
-def completion(X):
-    """Maximum-determinant positive definite completion of the sparse symmetric matrix ``X``
-    (lower triangle used) as a dense n x n array; raises ``ArithmeticError`` if none exists
-    (``base.py:952-973``: ``symbolic`` under a fill-reducing ordering, ``chompack.completion``,
-    then two ``chompack.trsm`` on the identity: X_hat = L^{-T} L^{-1})."""
+
+def _completion_factor(X):
+    """``symbolic`` of the pattern of ``X`` (lower triangle used) under a fill-reducing ordering and
+    ``chompack.completion`` on the backend: returns the factor L (a cspmatrix, P_V((L L^T)^-1) = X) and
+    ``order``, the original vertex at each internal position.  Raises ``ArithmeticError`` if X has no
+    positive definite completion."""
     from .chordal import cspmatrix
     from . import chordal
     X = sp.tril(sp.csc_matrix(X), format="coo")
@@ -535,9 +572,47 @@ def completion(X):
     full = (lo + sp.tril(lo, -1).T).tocsr()
     L = cspmatrix.from_vec(ops, np.asarray(full[p[symb.Ip], p[symb.Jp]]).ravel())
     chordal.completion(L)                       # ArithmeticError if X has no PD completion
-    Z = ops.trsm(L.buf, np.eye(n), "N")
-    Z = ops.trsm(L.buf, Z, "T")                 # internal order: vertex p[perm[i]] at position i
-    order = p[symb.perm]
+    return L, p[symb.perm]                      # internal order: vertex p[perm[i]] at position i
+
+
+def completion(X):
+    """Maximum-determinant positive definite completion of the sparse symmetric matrix ``X``
+    (lower triangle used) as a dense n x n array; raises ``ArithmeticError`` if none exists
+    (``base.py:952-973``: ``symbolic`` under a fill-reducing ordering, ``chompack.completion``,
+    then two ``chompack.trsm`` on the identity: X_hat = L^{-T} L^{-1})."""
+    L, order = _completion_factor(X)
+    n = len(order)
+    Z = L.ops.trsm(L.buf, np.eye(n), "N")
+    Z = L.ops.trsm(L.buf, Z, "T")
     out = np.empty((n, n))
     out[np.ix_(order, order)] = Z
+    return out
+
+
+def _check_seed(seed):
+    if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)):
+        raise TypeError("seed must be an integer")
+    if not 0 <= int(seed) < 1 << 64:
+        raise ValueError("seed must be in [0, 2**64)")
+    return int(seed)
+
+
+def _check_count(k, name, lo):
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or int(k) < lo:
+        raise ValueError("%s must be an integer >= %d" % (name, lo))
+    return int(k)
+
+
+def completion_sample(X, k, seed=0):
+    """``k`` Gaussian samples whose covariance is the maximum-determinant positive definite completion X_hat
+    of the sparse symmetric matrix ``X`` (lower triangle used), as an n x k array in the original order
+    (an extension: the reference has no sampling).  With L from ``chompack.completion``, X_hat = L^-T L^-1,
+    so column j is L^-T g_j: one chordal triangular solve, nothing dense of size n x n.  g_j is the standard
+    normal vector of sample j under ``seed`` (Philox4x64-10 and Box-Muller; entry i depends on (seed, j, i)
+    only).  Raises ``ArithmeticError`` where ``completion`` does."""
+    k = _check_count(k, "k", 0)
+    seed = _check_seed(seed)
+    L, order = _completion_factor(X)
+    out = np.empty((len(order), k))
+    out[order] = L.ops.completion_sample(L.buf, k, seed)
     return out

@@ -514,6 +514,14 @@ extern "C" int smcp_csp_probe(smcp_sym *s, int kind, const double *x, const doub
 extern "C" int smcp_csp_trsm(smcp_sym *s, const double *L, double *B_dev, int64_t ldb, int64_t nrhs, int trans) {
     return k_trsm(s, L, B_dev, ldb, nrhs, trans);
 }
+extern "C" int smcp_csp_sample(smcp_sym *s, const double *L, uint64_t seed, int64_t col0, double *B_dev, int64_t ldb, int64_t k) {
+    return k_sample(s, L, seed, col0, B_dev, ldb, k);
+}
+extern "C" int smcp_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc,
+                              const int64_t *crow, const int64_t *ccol, const double *cval, double *values_host, int8_t *x_host,
+                              int64_t *best_out) {
+    return k_round_pm1(s, L, seed, trials, chunk, nc, crow, ccol, cval, values_host, x_host, best_out);
+}
 
 // ---------------------------------------------------------------------------------------
 // Hessian factor

@@ -283,6 +283,11 @@ int k_scatter_vec(smcp_sym *s, double *dst, const double *dev_vec);
 int k_gather_vec(smcp_sym *s, const double *src, double *dev_vec);
 int k_axpy_batch(smcp_sym *s, const double *x, const double *dx, const double *gam_dev, double *out, int64_t count);
 
+// randomized rounding (rounding.cu): Gaussian samples L^-T g of the max-det completion, +-1 trials against the objective
+int k_sample(smcp_sym *s, const double *L, uint64_t seed, int64_t col0, double *B, int64_t ldb, int64_t k);
+int k_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc, const int64_t *crow,
+                const int64_t *ccol, const double *cval, double *values_host, int8_t *x_host, int64_t *best_out);
+
 // dense path for the top set of large supernodes (bigfront.cu)
 int big_setup(smcp_sym *s, const smcp_sym_desc *D);
 int big_cholesky(smcp_sym *s, const BigNode &q, double *X, int64_t b);

@@ -68,6 +68,9 @@ API = {
     "smcp_csp_llt": (_int, [_vp, _dp, _i64]),
     "smcp_csp_probe": (_int, [_vp, _int, _dp, _dp, _f64p, _i64, _i32p, _f64p]),
     "smcp_csp_trsm": (_int, [_vp, _dp, _dp, _i64, _i64, _int]),
+    "smcp_csp_sample": (_int, [_vp, _dp, C.c_uint64, _i64, _dp, _i64, _i64]),
+    "smcp_round_pm1": (_int, [_vp, _dp, C.c_uint64, _i64, _i64, _i64, _i64p, _i64p, _f64p, _f64p,
+                              np.ctypeslib.ndpointer(dtype=np.int8, flags="C_CONTIGUOUS"), C.POINTER(_i64)]),
     "smcp_hess_create": (_int, [_vp, _dp, _dp, C.POINTER(_vp)]),
     "smcp_hess_destroy": (_int, [_vp]),
     "smcp_hess_apply": (_int, [_vp, _dp, _i64, _int]),
@@ -469,6 +472,40 @@ class DeviceBackend:
         finally:
             self.free_batch(buf)
         return out
+
+    # -- randomized rounding ----------------------------------------------------------------
+    def completion_sample(self, Lbuf, k, seed, col0=0):
+        """``L^-T g_j`` for the samples j = col0 .. col0+k-1 under ``seed`` (``smcp_csp_sample``), with L from
+        ``completion``: an n x k host array, rows in the internal order, columns with covariance the max-det
+        completion."""
+        n, k, nblk = self.symb.n, int(k), self.symb.nblk
+        count = max(1, -(-(n * k) // nblk))
+        buf = self.alloc_batch(count)
+        try:
+            _ck(self.lib, self.lib.smcp_csp_sample(self.sym, Lbuf, int(seed), int(col0), buf, n, k))
+            out = self.get_batch(buf, count).reshape(-1)[:n * k].reshape(n, k, order="F")
+        finally:
+            self.free_batch(buf)
+        TRAFFIC["d2h"] += 8 * n * k
+        return out
+
+    def round_pm1(self, Lbuf, crow, ccol, cval, trials, seed, chunk=0):
+        """``trials`` +-1 roundings sign(L^-T g_t) against the objective given by its lower-triangular entries
+        (``crow``, ``ccol`` in internal coordinates, ``cval``) on the device (``smcp_round_pm1``).  Returns
+        ``(values, x, best)``: the value of every trial, the int8 sign vector of the best one (internal order)
+        and its index."""
+        crow, ccol = _i64(crow), _i64(ccol)
+        cval = np.ascontiguousarray(cval, dtype=np.float64)
+        if not len(crow) == len(ccol) == len(cval):
+            raise ValueError("crow, ccol and cval must have the same length")
+        values = np.empty(max(0, int(trials)))
+        x = np.empty(self.symb.n, dtype=np.int8)
+        best = C.c_int64()
+        _ck(self.lib, self.lib.smcp_round_pm1(self.sym, Lbuf, int(seed), int(trials), int(chunk), len(cval), crow, ccol,
+                                              cval, values, x, C.byref(best)))
+        TRAFFIC["h2d"] += 24 * len(cval)
+        TRAFFIC["d2h"] += 8 * len(values) + len(x)
+        return values, x, best.value
 
     def cholesky_batch(self, buf, count):
         info = np.zeros(count, dtype=np.int32)
