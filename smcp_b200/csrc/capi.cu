@@ -1223,8 +1223,9 @@ static int assemble_sparse_range(smcp_op *op, smcp_hess *h, int64_t s0, int64_t 
         const double kmat_gb = getenv("SMCP_B200_SCM_KMAT_GB") ? atof(getenv("SMCP_B200_SCM_KMAT_GB")) : 4.0;
         const long long ldk = (op->npos + 1) & ~1LL;
         const double kbytes = (double)ldk * (double)op->npos * 8.0;
-        const double nnz_sp = op->sp_avg_nnz * (double)(m - op->md);
-        if (kbytes <= kmat_gb * 1073741824.0 && 2 * n <= cap && nnz_sp >= 2.0 * (double)op->npos) {
+        // counted, not avg * (m - md): that product can round below an exact 2 npos
+        const int64_t nnz_sp = op->h_colptr[m] - op->h_colptr[op->md];
+        if (kbytes <= kmat_gb * 1073741824.0 && 2 * n <= cap && nnz_sp >= 2 * (int64_t)op->npos) {
             if (!op->Kpos_valid) {
                 if (grow((void **)&op->Kpos, &op->Kpos_cap, (size_t)kbytes)) return -1;
                 LaunchScope ls(ctx, "scm_kmat");
