@@ -148,6 +148,25 @@ int smcp_csp_sample(smcp_sym *sym, const double *L, uint64_t seed, int64_t col0,
 int smcp_round_pm1(smcp_sym *sym, const double *L, uint64_t seed, int64_t trials, int64_t chunk,
                    int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
                    double *values_host, int8_t *x_host, int64_t *best_out);
+/* One-flip local search of ±1 vectors against f(x) = sum_ij C_ij x_i x_j, C the symmetric matrix of the nc
+ * objective entries (host arrays; entries off the diagonal count for both triangles, duplicates are summed in input
+ * order).  With s_i = sum_{j != i} C_ij x_j, a_i = sum_{j != i} |C_ij| (both in increasing j) and the gain
+ * g_i = x_i s_i, each step flips the vertex of largest g_i among those with g_i > tol a_i (lowest index on ties),
+ * which lowers f by 4 g_i; the search stops when none qualifies or after max_flips flips.  Values are evaluated as
+ * smcp_round_pm1 evaluates its trials.  Needs n <= 2^20 (-2 beyond), max_flips >= 0 and a finite tol >= 0.
+ * smcp_round_pm1_ls: smcp_round_pm1 with the search run on every trial; values0_host[t] is the value of trial t
+ * before the search, flips_host[t] its number of flips, and values_host, x_host and *best_out refer to the searched
+ * trials.  The search reuses the pass's sample buffer for s.
+ * smcp_pm1_local_search: the search on k caller-given vectors x_host (k x n int8, row t = vector t, every entry ±1),
+ * replaced by the searched ones; values_host[t] and flips_host[t] as above.  Its workspace follows the pass rule of
+ * smcp_round_pm1 (n x pass doubles within 1 GiB). */
+int smcp_round_pm1_ls(smcp_sym *sym, const double *L, uint64_t seed, int64_t trials, int64_t chunk,
+                      int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
+                      int64_t max_flips, double tol, double *values0_host,
+                      double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host);
+int smcp_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host,
+                          int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
+                          int64_t max_flips, double tol, double *values_host, int64_t *flips_host);
 
 /* ---- barrier Hessian: chompack.hessian(L, Y, U, adj=None, inv=...) ---------------------- */
 int smcp_hess_create(smcp_sym *sym, const double *L, const double *Y, smcp_hess **out);

@@ -295,33 +295,70 @@ class SDP(object):
         return X0, sol
 
     # -- rounding (an extension: the reference has none) ---------------------------------
-    def round_pm1(self, sol, trials=256, seed=0, chunk=0):
+    def round_pm1(self, sol, trials=256, seed=0, chunk=0, local_search=False, max_flips=None, tol=1e-12):
         """Goemans-Williamson rounding of a solution with diag(X) = 1: ``trials`` sign vectors
         s_t = sign(v_t), v_t drawn with covariance the max-det completion of ``sol['x']``
         (``completion_sample``), evaluated against the objective C on the device; ``chunk`` trials per pass
         (0: as many as fit in 1 GiB), with no effect on the result.  Returns a dict: ``x`` (int8 +-1, original
         order) of the smallest C . x x^T (lowest trial on ties), ``value`` = C . x x^T, ``values`` of every
         trial and ``trial``, the index of the best one.  Raises ``ArithmeticError`` if X has no positive
-        definite completion."""
+        definite completion.
+
+        ``local_search=True`` runs the one-flip local search of ``local_search_pm1`` (``max_flips``, ``tol``) on
+        every trial on the device, in the internal order of the completion (which decides ties); ``x``, ``value``,
+        ``values`` and ``trial`` then refer to the searched trials, ``values_rounded`` holds the values before the
+        search and ``flips`` the number of flips of every trial."""
         trials = _check_count(trials, "trials", 1)
         seed = _check_seed(seed)
         chunk = _check_count(chunk, "chunk", 0)
+        if not isinstance(local_search, (bool, np.bool_)):
+            raise TypeError("local_search must be a bool")
+        if max_flips is not None:
+            max_flips = _check_count(max_flips, "max_flips", 0)
+        tol = _check_tol(tol)
         if not isinstance(sol, dict) or "x" not in sol:
             raise ValueError("sol must be a solution dict holding 'x'")
         L, order = _completion_factor(sol["x"])
         n = self.n
         if len(order) != n:
             raise ValueError("sol['x'] is %d x %d, the problem has n = %d" % (len(order), len(order), n))
-        A = self._need()
-        r = A.indices[A.indptr[0]:A.indptr[1]]
-        I, J = misc.ind2sub(n, r)
+        I, J, v = self._objective_entries()
         pos = np.empty(n, dtype=np.int64)
         pos[order] = np.arange(n, dtype=np.int64)
-        values, xi, best = L.ops.round_pm1(L.buf, pos[np.asarray(I)], pos[np.asarray(J)],
-                                           A.data[A.indptr[0]:A.indptr[1]], trials, seed, chunk)
+        out = {}
+        if local_search:
+            values0, values, flips, xi, best = L.ops.round_pm1_ls(L.buf, pos[I], pos[J], v, trials, seed, chunk,
+                                                                  max_flips, tol)
+            out = {"values_rounded": values0, "flips": flips}
+        else:
+            values, xi, best = L.ops.round_pm1(L.buf, pos[I], pos[J], v, trials, seed, chunk)
         x = np.empty(n, dtype=np.int8)
         x[order] = xi
-        return {"x": x, "value": float(values[best]), "values": values, "trial": int(best)}
+        out.update({"x": x, "value": float(values[best]), "values": values, "trial": int(best)})
+        return out
+
+    def local_search_pm1(self, x, max_flips=None, tol=1e-12):
+        """One-flip local search of +-1 vectors against f(x) = C . x x^T (minimized), on the device (an
+        extension).  ``x``: integers +-1 of shape (n,) or (k, n), original order.  With s_i = sum_{j != i} C_ij x_j
+        and a_i = sum_{j != i} |C_ij|, each step flips the vertex with the largest gain g_i = x_i s_i among those
+        with g_i > ``tol`` a_i (lowest index on ties), which lowers f by 4 g_i; a vector's search stops when no
+        vertex qualifies or after ``max_flips`` flips (None: n).  Returns a dict: ``x`` (int8, the shape of the
+        input), ``values`` = f of the searched vectors and ``flips``, their numbers of flips (shape x.shape[:-1])."""
+        n = self.n
+        xa = _check_pm1(x, n)
+        max_flips = n if max_flips is None else _check_count(max_flips, "max_flips", 0)
+        tol = _check_tol(tol)
+        I, J, v = self._objective_entries()
+        ops = solvers._make_backend(Symbolic(n, np.arange(n + 1), np.arange(n)))
+        xs, values, flips = ops.pm1_local_search(xa.reshape(-1, n), I, J, v, max_flips, tol)
+        shape = np.shape(x)
+        return {"x": xs.reshape(shape), "values": values.reshape(shape[:-1]), "flips": flips.reshape(shape[:-1])}
+
+    def _objective_entries(self):
+        """Lower-triangular entries (row, col, value) of C in the original order."""
+        A = self._need()
+        I, J = misc.ind2sub(self.n, A.indices[A.indptr[0]:A.indptr[1]])
+        return np.asarray(I, dtype=np.int64), np.asarray(J, dtype=np.int64), A.data[A.indptr[0]:A.indptr[1]]
 
 
 # --------------------------------------------------------------------------------------
@@ -542,12 +579,13 @@ class maxcut_SDP(SDP):
         self._b = np.ones(n)
         self._pname = "maxcut_n%i" % n
 
-    def cut(self, sol, trials=256, seed=0):
+    def cut(self, sol, trials=256, seed=0, local_search=False):
         """A cut from a solution of the relaxation by Goemans-Williamson rounding (``SDP.round_pm1``):
         returns ``(x, weight, bound)`` with the +-1 vector x of the heaviest of ``trials`` random hyperplane
         cuts, its weight (= -C . x x^T) and the certified upper bound -``sol['dual objective']`` on every
-        cut's weight."""
-        r = self.round_pm1(sol, trials=trials, seed=seed)
+        cut's weight.  ``local_search=True`` improves every cut by single-vertex moves first (one-flip local
+        search, see ``SDP.local_search_pm1``) and returns the heaviest improved cut."""
+        r = self.round_pm1(sol, trials=trials, seed=seed, local_search=local_search)
         return r["x"], -r["value"], -float(sol["dual objective"])
 
 
@@ -601,6 +639,26 @@ def _check_count(k, name, lo):
     if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or int(k) < lo:
         raise ValueError("%s must be an integer >= %d" % (name, lo))
     return int(k)
+
+
+def _check_tol(tol):
+    if isinstance(tol, bool) or not isinstance(tol, (int, float, np.integer, np.floating)):
+        raise TypeError("tol must be a real number")
+    if not (np.isfinite(tol) and tol >= 0):
+        raise ValueError("tol must be finite and >= 0")
+    return float(tol)
+
+
+def _check_pm1(x, n):
+    """x as a (k, n) int8 array, k >= 1, for x of shape (n,) or (k, n) holding integers +-1 only."""
+    a = np.asarray(x)
+    if a.dtype == bool or a.dtype.kind not in "iu":
+        raise TypeError("x must be an integer array")
+    if a.ndim not in (1, 2) or a.shape[-1] != n or a.size == 0:
+        raise ValueError("x must have shape (%d,) or (k, %d) with k >= 1, got %s" % (n, n, a.shape))
+    if not np.all((a == 1) | (a == -1)):
+        raise ValueError("x must hold +-1 only")
+    return np.ascontiguousarray(a.reshape(-1, n), dtype=np.int8)
 
 
 def completion_sample(X, k, seed=0):

@@ -522,6 +522,17 @@ extern "C" int smcp_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64
                               int64_t *best_out) {
     return k_round_pm1(s, L, seed, trials, chunk, nc, crow, ccol, cval, values_host, x_host, best_out);
 }
+extern "C" int smcp_round_pm1_ls(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc,
+                                 const int64_t *crow, const int64_t *ccol, const double *cval, int64_t max_flips, double tol,
+                                 double *values0_host, double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host) {
+    return k_round_pm1_ls(s, L, seed, trials, chunk, nc, crow, ccol, cval, max_flips, tol, values0_host, values_host, x_host,
+                          best_out, flips_host);
+}
+extern "C" int smcp_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow,
+                                     const int64_t *ccol, const double *cval, int64_t max_flips, double tol, double *values_host,
+                                     int64_t *flips_host) {
+    return k_pm1_local_search(ctx, n, k, x_host, nc, crow, ccol, cval, max_flips, tol, values_host, flips_host);
+}
 
 // ---------------------------------------------------------------------------------------
 // Hessian factor

@@ -14,6 +14,8 @@
 //    the per-slice partial sums are added in a fixed order: the values are bitwise reproducible and do not
 //    depend on how many trials a pass holds.  The best trial (smallest value, lowest t on ties) is tracked on
 //    the device and only its sign vector returns to the host.
+//  * round_ls: one-flip local search of the +-1 trials (see the section before ROUND_MAX_PASS), between the packing
+//    of the samples and their evaluation; the searched signs are evaluated by the same round_pack / eval / sum.
 #include "internal.cuh"
 #include <algorithm>
 #include <cmath>
@@ -194,30 +196,201 @@ int k_sample(smcp_sym *s, const double *L, uint64_t seed, int64_t col0, double *
     return k_trsm(s, L, B, ldb, k, 1);
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// One-flip local search of +-1 trials (an extension, like the rounding), f(x) = sum_ij C_ij x_i x_j minimized.
+// Row i of the search's CSR holds the off-diagonal entries (i, j) of C from both triangles in increasing j, duplicates
+// summed in input order (ls_rows).  Per trial, s_i = sum_{j != i} C_ij x_j in row order and g_i = x_i s_i: flipping i
+// changes f by -4 g_i.  A step flips the vertex of largest g_i among those with g_i > thr_i = tol sum_{j != i} |C_ij|
+// (lowest i on ties), adds 2 x_i C_ij to s_j over row i (the factor is exact, so a contraction to an FMA changes no
+// bit) and negates g_i; the search stops when no vertex qualifies or after max_flips flips.
+// round_ls_kernel: one CTA per trial, persistent over the T trials of a pass.  The signs are a bit array in shared
+// memory, s is the trial's column of the pass buffer V (dead once the samples are packed), and the largest qualifying
+// gain of every LS_CHUNK-vertex chunk is kept in shared memory.  A flip recomputes the chunks of the flipped vertex and
+// of its neighbours (all chunks once the row reaches as many), one warp per chunk.  The columns of a row are distinct,
+// so no two threads update the same s_j: no atomics, and every result depends on the trial's signs alone.
+#define LS_THREADS 256
+#define LS_WARPS (LS_THREADS / 32)
+#define LS_CHUNK 256
+// largest n of the shared layout: n / 8 bytes of signs + 12 bytes per chunk = 176 KiB at 2^20
+#define LS_MAX_N (1 << 20)
+
+static size_t ls_smem_bytes(int n) {
+    const size_t nch = (size_t)(n + LS_CHUNK - 1) / LS_CHUNK, nxw = (size_t)(n + 31) / 32;
+    return nch * (sizeof(double) + sizeof(int)) + nxw * sizeof(unsigned);
+}
+
+// (v, i) comes before (bv, bi) in the order of the search: a qualifying vertex (i >= 0), larger gain, lower index
+__device__ __forceinline__ bool ls_before(double v, int i, double bv, int bi) {
+    return i >= 0 && (bi < 0 || v > bv || (v == bv && i < bi));
+}
+
+// the first (v, i) of the warp lands in lane 0
+__device__ __forceinline__ void ls_warp_first(double &v, int &i) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ov = __shfl_down_sync(0xffffffffu, v, o);
+        const int oi = __shfl_down_sync(0xffffffffu, i, o);
+        if (ls_before(ov, oi, v, i)) { v = ov; i = oi; }
+    }
+}
+
+// largest qualifying gain of chunk c (one warp); INIT: s of the chunk's vertices is summed from their rows first
+template <bool INIT>
+__device__ __forceinline__ void ls_chunk(int c, int n, int lane, const long long *__restrict__ rp, const int *__restrict__ col,
+                                         const double *__restrict__ val, const double *__restrict__ thr, const unsigned *xw,
+                                         double *s, double *cv, int *ci) {
+    double bv = 0.0;
+    int bi = -1;
+    const int i1 = min(n, (c + 1) * LS_CHUNK);
+    for (int i = c * LS_CHUNK + lane; i < i1; i += 32) {     // ascending i per lane: the first of equal gains stays
+        double si;
+        if (INIT) {
+            si = 0.0;
+            for (long long p = rp[i]; p < rp[i + 1]; ++p) {
+                const int j = col[p];
+                si += ((xw[j >> 5] >> (j & 31)) & 1u) ? -val[p] : val[p];
+            }
+            s[i] = si;
+        } else {
+            si = s[i];
+        }
+        const double g = ((xw[i >> 5] >> (i & 31)) & 1u) ? -si : si;
+        if (g > thr[i] && (bi < 0 || g > bv)) { bv = g; bi = i; }
+    }
+    ls_warp_first(bv, bi);
+    if (lane == 0) {
+        cv[c] = bv;
+        ci[c] = bi;
+    }
+}
+
+// trial t of the pass: signs from bit t & 63 of the word group t >> 6 of bits, s in V[t n ..], final signs back into
+// V[t n + i] as +-1.0 (for round_pack_kernel), the number of flips in flips[t]
+// (6 CTAs per SM: 40 registers without spills; at 8, the cap of 32 registers spills)
+__global__ void __launch_bounds__(LS_THREADS, 6) round_ls_kernel(int n, int T, const unsigned long long *__restrict__ bits,
+                                                              const long long *__restrict__ rp, const int *__restrict__ col,
+                                                              const double *__restrict__ val, const double *__restrict__ thr,
+                                                              long long max_flips, double *V, long long *__restrict__ flips) {
+    extern __shared__ __align__(16) unsigned char ls_smem[];
+    const int nch = (n + LS_CHUNK - 1) / LS_CHUNK, nxw = (n + 31) / 32;
+    double *cv = (double *)ls_smem;                 // largest qualifying gain of each chunk
+    int *ci = (int *)(cv + nch);                    // its vertex, -1: none
+    unsigned *xw = (unsigned *)(ci + nch);          // bit i: x_i = -1
+    __shared__ double wv[LS_WARPS];
+    __shared__ int wi[LS_WARPS];
+    __shared__ int pick, pneg;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int t = blockIdx.x; t < T; t += gridDim.x) {
+        const unsigned long long *wg = bits + (long long)(t >> 6) * n;
+        const int b = t & 63;
+        double *s = V + (long long)t * n;
+        for (int w = warp; w < nxw; w += LS_WARPS) {
+            const int i = 32 * w + lane;
+            const unsigned m = __ballot_sync(0xffffffffu, i < n && ((wg[i] >> b) & 1ULL));
+            if (lane == 0) xw[w] = m;
+        }
+        __syncthreads();
+        for (int c = warp; c < nch; c += LS_WARPS) ls_chunk<true>(c, n, lane, rp, col, val, thr, xw, s, cv, ci);
+        __syncthreads();
+        long long nf = 0;
+        while (nf < max_flips) {
+            double bv = 0.0;
+            int bi = -1;
+            for (int c = threadIdx.x; c < nch; c += LS_THREADS)
+                if (ls_before(cv[c], ci[c], bv, bi)) { bv = cv[c]; bi = ci[c]; }
+            ls_warp_first(bv, bi);
+            if (lane == 0) {
+                wv[warp] = bv;
+                wi[warp] = bi;
+            }
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                for (int w = 1; w < LS_WARPS; ++w)
+                    if (ls_before(wv[w], wi[w], bv, bi)) { bv = wv[w]; bi = wi[w]; }
+                if (bi >= 0) {
+                    const unsigned m = 1u << (bi & 31);
+                    pneg = (xw[bi >> 5] & m) == 0u;      // the new sign of x_bi
+                    xw[bi >> 5] ^= m;
+                }
+                pick = bi;
+            }
+            __syncthreads();
+            const int i = pick;
+            if (i < 0) break;
+            ++nf;
+            const long long p0 = rp[i], p1 = rp[i + 1];
+            const double two = pneg ? -2.0 : 2.0;
+            for (long long p = p0 + threadIdx.x; p < p1; p += LS_THREADS) {
+                const int j = col[p];
+                s[j] = s[j] + two * val[p];
+            }
+            __syncthreads();
+            const int d = (int)(p1 - p0), c0 = i / LS_CHUNK;
+            if (d + 1 >= nch) {
+                for (int c = warp; c < nch; c += LS_WARPS) ls_chunk<false>(c, n, lane, rp, col, val, thr, xw, s, cv, ci);
+            } else {
+                // entry d: the chunk of i; entry e < d: the chunk of the e-th neighbour unless an earlier entry has it
+                // (columns ascend, so equal chunks of neighbours are adjacent)
+                for (int e = warp; e <= d; e += LS_WARPS) {
+                    int c = c0;
+                    if (e < d) {
+                        c = col[p0 + e] / LS_CHUNK;
+                        if (c == c0 || (e > 0 && col[p0 + e - 1] / LS_CHUNK == c)) continue;
+                    }
+                    ls_chunk<false>(c, n, lane, rp, col, val, thr, xw, s, cv, ci);
+                }
+            }
+            __syncthreads();
+        }
+        for (int i = threadIdx.x; i < n; i += LS_THREADS) s[i] = ((xw[i >> 5] >> (i & 31)) & 1u) ? -1.0 : 1.0;
+        if (threadIdx.x == 0) flips[t] = nf;
+        __syncthreads();
+    }
+}
+
 // largest number of trials a pass holds: bounds the word groups (grid.y) and the slice partial sums
 #define ROUND_MAX_PASS 65536
 // columns of one trsm call; every call of a smcp_round_pm1 has the same width, so the samples of a trial are the
 // same bits whatever the pass size (k_trsm picks its kernels from the number of right-hand sides)
 #define ROUND_BLOCK 256
 
-int k_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc, const int64_t *crow,
-                const int64_t *ccol, const double *cval, double *values_host, int8_t *x_host, int64_t *best_out) {
-    smcp_ctx *ctx = s->ctx;
-    const int n = s->d.n;
-    if (trials < 1 || chunk < 0 || nc < 0) {
-        smcp_set_error("smcp_round_pm1: need trials >= 1, chunk >= 0, nc >= 0 (got %lld, %lld, %lld)", (long long)trials,
-                       (long long)chunk, (long long)nc);
-        return -2;
+// device workspace of one call, freed (after the stream drains) when it goes out of scope
+struct RoundWs {
+    smcp_ctx *ctx;
+    const char *fn;
+    std::vector<void *> p;
+    ~RoundWs() {
+        cudaStreamSynchronize(ctx->stream);
+        for (void *q : p) cudaFree(q);
     }
-    if (!L || !values_host || !x_host || !best_out || (nc > 0 && (!crow || !ccol || !cval))) {
-        smcp_set_error("smcp_round_pm1: null argument");
-        return -2;
+    void *alloc(size_t bytes) {
+        void *q = nullptr;
+        if (cudaMalloc(&q, std::max<size_t>(bytes, 16)) != cudaSuccess) {
+            cudaGetLastError();
+            smcp_set_error("%s: cudaMalloc(%zu bytes) failed", fn, bytes);
+            return nullptr;
+        }
+        p.push_back(q);
+        return q;
     }
+};
+
+// the objective on the device, as round_eval_kernel reads it: nc entries (r, c, coef), the factor 2 off the diagonal
+// folded into coef, cut into S fixed slices of `per` entries (independent of the trials)
+struct RoundObj {
+    int *er = nullptr, *ec = nullptr;
+    double *ev = nullptr;
+    long long nc = 0, per = 1;
+    int S = 1;
+};
+
+static int round_obj_upload(RoundWs &ws, const char *fn, int n, int64_t nc, const int64_t *crow, const int64_t *ccol,
+                            const double *cval, RoundObj &o) {
     std::vector<int> hr((size_t)nc), hc((size_t)nc);
     std::vector<double> hv((size_t)nc);
     for (int64_t q = 0; q < nc; ++q) {
         if (crow[q] < 0 || crow[q] >= n || ccol[q] < 0 || ccol[q] >= n) {
-            smcp_set_error("smcp_round_pm1: objective entry %lld at (%lld, %lld) is outside 0..%d", (long long)q, (long long)crow[q],
+            smcp_set_error("%s: objective entry %lld at (%lld, %lld) is outside 0..%d", fn, (long long)q, (long long)crow[q],
                            (long long)ccol[q], n - 1);
             return -2;
         }
@@ -225,6 +398,159 @@ int k_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int
         hc[q] = (int)ccol[q];
         hv[q] = crow[q] == ccol[q] ? cval[q] : 2.0 * cval[q];
     }
+    o.nc = nc;
+    o.S = (int)std::min<int64_t>(256, std::max<int64_t>(1, (nc + 511) / 512));
+    o.per = std::max<long long>(1, (nc + o.S - 1) / o.S);
+    o.er = (int *)ws.alloc((size_t)nc * sizeof(int));
+    o.ec = (int *)ws.alloc((size_t)nc * sizeof(int));
+    o.ev = (double *)ws.alloc((size_t)nc * sizeof(double));
+    if (!o.er || !o.ec || !o.ev) return -1;
+    if (nc) {
+        CUDA_TRY(cudaMemcpyAsync(o.er, hr.data(), (size_t)nc * sizeof(int), cudaMemcpyHostToDevice, ws.ctx->stream));
+        CUDA_TRY(cudaMemcpyAsync(o.ec, hc.data(), (size_t)nc * sizeof(int), cudaMemcpyHostToDevice, ws.ctx->stream));
+        CUDA_TRY(cudaMemcpyAsync(o.ev, hv.data(), (size_t)nc * sizeof(double), cudaMemcpyHostToDevice, ws.ctx->stream));
+    }
+    return 0;
+}
+
+// the search's rows on the device (see round_ls_kernel): CSR of the off-diagonal entries and thr_i = tol a_i
+struct LsRows {
+    long long *rp = nullptr;
+    int *col = nullptr;
+    double *val = nullptr, *thr = nullptr;
+};
+
+// entries already checked by round_obj_upload
+static int ls_rows_upload(RoundWs &ws, int n, int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
+                          double tol, LsRows &d) {
+    std::vector<int64_t> q;
+    for (int64_t e = 0; e < nc; ++e)
+        if (crow[e] != ccol[e]) q.push_back(e);
+    auto lo = [&](int64_t e) { return std::min(crow[e], ccol[e]); };
+    auto hi = [&](int64_t e) { return std::max(crow[e], ccol[e]); };
+    std::stable_sort(q.begin(), q.end(), [&](int64_t a, int64_t b) { return lo(a) < lo(b) || (lo(a) == lo(b) && hi(a) < hi(b)); });
+    // merged pairs (l < h) ascending; row l gets (h, v) and row h gets (l, v).  In this order every row receives its
+    // columns ascending: first the l < row (pairs of smaller l come first), then the h > row.
+    std::vector<int> pl, ph;
+    std::vector<double> pv;
+    for (size_t a = 0; a < q.size();) {
+        const int64_t l = lo(q[a]), h = hi(q[a]);
+        double v = cval[q[a]];
+        size_t b = a + 1;
+        for (; b < q.size() && lo(q[b]) == l && hi(q[b]) == h; ++b) v += cval[q[b]];
+        pl.push_back((int)l);
+        ph.push_back((int)h);
+        pv.push_back(v);
+        a = b;
+    }
+    std::vector<long long> rp((size_t)n + 1, 0);
+    for (size_t e = 0; e < pv.size(); ++e) {
+        ++rp[pl[e] + 1];
+        ++rp[ph[e] + 1];
+    }
+    for (int i = 0; i < n; ++i) rp[i + 1] += rp[i];
+    const size_t nnz = (size_t)rp[n];
+    std::vector<long long> fill(rp.begin(), rp.end() - 1);
+    std::vector<int> col(nnz);
+    std::vector<double> val(nnz), thr((size_t)n);
+    for (size_t e = 0; e < pv.size(); ++e) {
+        col[fill[pl[e]]] = ph[e];
+        val[fill[pl[e]]++] = pv[e];
+        col[fill[ph[e]]] = pl[e];
+        val[fill[ph[e]]++] = pv[e];
+    }
+    for (int i = 0; i < n; ++i) {
+        double a = 0.0;
+        for (long long p = rp[i]; p < rp[i + 1]; ++p) a += std::fabs(val[p]);
+        thr[i] = tol * a;
+    }
+    d.rp = (long long *)ws.alloc(rp.size() * sizeof(long long));
+    d.col = (int *)ws.alloc(nnz * sizeof(int));
+    d.val = (double *)ws.alloc(nnz * sizeof(double));
+    d.thr = (double *)ws.alloc((size_t)n * sizeof(double));
+    if (!d.rp || !d.col || !d.val || !d.thr) return -1;
+    cudaStream_t st = ws.ctx->stream;
+    CUDA_TRY(cudaMemcpyAsync(d.rp, rp.data(), rp.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+    if (nnz) {
+        CUDA_TRY(cudaMemcpyAsync(d.col, col.data(), nnz * sizeof(int), cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(d.val, val.data(), nnz * sizeof(double), cudaMemcpyHostToDevice, st));
+    }
+    CUDA_TRY(cudaMemcpyAsync(d.thr, thr.data(), (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
+    return 0;
+}
+
+// checks shared by both entry points of the search
+static int ls_check(const char *fn, int n, int64_t max_flips, double tol) {
+    if (n > LS_MAX_N) {
+        smcp_set_error("%s: n = %d exceeds %d, the largest the search's shared-memory layout holds", fn, n, LS_MAX_N);
+        return -2;
+    }
+    if (max_flips < 0 || !(tol >= 0.0) || !std::isfinite(tol)) {
+        smcp_set_error("%s: need max_flips >= 0 and a finite tol >= 0 (got %lld, %g)", fn, (long long)max_flips, tol);
+        return -2;
+    }
+    return 0;
+}
+
+static int launch_ls(smcp_ctx *ctx, int n, int T, const unsigned long long *bits, const LsRows &d, int64_t max_flips, double *V,
+                     long long *flips) {
+    const size_t smem = ls_smem_bytes(n);
+    CUDA_TRY(cudaFuncSetAttribute(round_ls_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0;
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, round_ls_kernel, LS_THREADS, smem));
+    const int grid = std::max(1, std::min(T, std::max(1, per_sm) * ctx->num_sms));
+    {
+        LaunchScope ls(ctx, "round_ls");
+        round_ls_kernel<<<grid, LS_THREADS, smem, ctx->stream>>>(n, T, bits, d.rp, d.col, d.val, d.thr, (long long)max_flips, V,
+                                                                 flips);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+// values[t0 + t] of the T trials whose signs are sign(V[:, t]) (packed into bits first); with `best`, the best trial so
+// far and its signs x are updated
+static int eval_pass(smcp_ctx *ctx, const double *V, int n, int T, unsigned long long *bits, const RoundObj &o, double *part,
+                     int64_t t0, double *values, RoundBest *best, signed char *x) {
+    const int nw = (T + 63) / 64;
+    {
+        LaunchScope ls(ctx, "round_eval", best ? 4 : 3);
+        round_pack_kernel<<<dim3((unsigned)((n + 255) / 256), (unsigned)nw), 256, 0, ctx->stream>>>(V, n, n, T, bits);
+        round_eval_kernel<<<dim3((unsigned)o.S, (unsigned)nw), 32 * EV_WARPS, 0, ctx->stream>>>(o.er, o.ec, o.ev, o.nc, o.per, bits,
+                                                                                             n, part);
+        round_sum_kernel<<<(unsigned)((T + 255) / 256), 256, 0, ctx->stream>>>(part, o.S, T, t0, values);
+        if (best) round_best_kernel<<<1, BEST_THREADS, 0, ctx->stream>>>(values, t0, T, bits, n, best, x);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+// ls == nullptr: smcp_round_pm1; otherwise the search runs on every trial between its evaluation into
+// ls->values0_host and the evaluation that values_host, x_host and best_out report
+struct LsArgs {
+    int64_t max_flips;
+    double tol;
+    double *values0_host;
+    int64_t *flips_host;
+};
+
+static int round_pm1_impl(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc,
+                          const int64_t *crow, const int64_t *ccol, const double *cval, const LsArgs *ls, double *values_host,
+                          int8_t *x_host, int64_t *best_out) {
+    smcp_ctx *ctx = s->ctx;
+    const int n = s->d.n;
+    const char *fn = ls ? "smcp_round_pm1_ls" : "smcp_round_pm1";
+    if (trials < 1 || chunk < 0 || nc < 0) {
+        smcp_set_error("%s: need trials >= 1, chunk >= 0, nc >= 0 (got %lld, %lld, %lld)", fn, (long long)trials,
+                       (long long)chunk, (long long)nc);
+        return -2;
+    }
+    if (!L || !values_host || !x_host || !best_out || (nc > 0 && (!crow || !ccol || !cval)) ||
+        (ls && (!ls->values0_host || !ls->flips_host))) {
+        smcp_set_error("%s: null argument", fn);
+        return -2;
+    }
+    if (ls && ls_check(fn, n, ls->max_flips, ls->tol)) return -2;
     // solve blocks: as few as hold ROUND_BLOCK columns each, all of the same width tb (within 1 GiB)
     const int64_t fit = std::max<int64_t>(1, (int64_t(1) << 30) / (8 * (int64_t)n));
     const int64_t bmax = std::min<int64_t>(ROUND_BLOCK, fit);
@@ -236,45 +562,23 @@ int k_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int
     bp = std::min(bp, nblocks);
     const int64_t pw = bp * tb;                    // trials per pass
     const int64_t nwmax = (pw + 63) / 64;
-    // entry slices: a fixed partition of the entry list, independent of the trials
-    const int S = (int)std::min<int64_t>(256, std::max<int64_t>(1, (nc + 511) / 512));
-    const long long per = std::max<long long>(1, (nc + S - 1) / S);
 
-    struct Ws {
-        smcp_ctx *ctx;
-        std::vector<void *> p;
-        ~Ws() {
-            cudaStreamSynchronize(ctx->stream);
-            for (void *q : p) cudaFree(q);
-        }
-    } ws{ctx, {}};
-    auto alloc = [&](size_t bytes) -> void * {
-        void *q = nullptr;
-        if (cudaMalloc(&q, std::max<size_t>(bytes, 16)) != cudaSuccess) {
-            cudaGetLastError();
-            smcp_set_error("smcp_round_pm1: cudaMalloc(%zu bytes) failed", bytes);
-            return nullptr;
-        }
-        ws.p.push_back(q);
-        return q;
-    };
-    double *V = (double *)alloc((size_t)n * pw * sizeof(double));
-    unsigned long long *bits = (unsigned long long *)alloc((size_t)n * nwmax * sizeof(unsigned long long));
-    double *part = (double *)alloc((size_t)nwmax * S * 64 * sizeof(double));
-    double *values = (double *)alloc((size_t)trials * sizeof(double));
-    RoundBest *best = (RoundBest *)alloc(sizeof(RoundBest));
-    signed char *x = (signed char *)alloc((size_t)n);
-    int *er = (int *)alloc((size_t)nc * sizeof(int));
-    int *ec = (int *)alloc((size_t)nc * sizeof(int));
-    double *ev = (double *)alloc((size_t)nc * sizeof(double));
-    if (!V || !bits || !part || !values || !best || !x || !er || !ec || !ev) return -1;
+    RoundWs ws{ctx, fn, {}};
+    RoundObj o;
+    if (int rc = round_obj_upload(ws, fn, n, nc, crow, ccol, cval, o)) return rc;
+    LsRows d;
+    if (ls && ls_rows_upload(ws, n, nc, crow, ccol, cval, ls->tol, d)) return -1;
+    double *V = (double *)ws.alloc((size_t)n * pw * sizeof(double));
+    unsigned long long *bits = (unsigned long long *)ws.alloc((size_t)n * nwmax * sizeof(unsigned long long));
+    double *part = (double *)ws.alloc((size_t)nwmax * o.S * 64 * sizeof(double));
+    double *values = (double *)ws.alloc((size_t)trials * sizeof(double));
+    RoundBest *best = (RoundBest *)ws.alloc(sizeof(RoundBest));
+    signed char *x = (signed char *)ws.alloc((size_t)n);
+    double *values0 = ls ? (double *)ws.alloc((size_t)trials * sizeof(double)) : nullptr;
+    long long *flips = ls ? (long long *)ws.alloc((size_t)trials * sizeof(long long)) : nullptr;
+    if (!V || !bits || !part || !values || !best || !x || (ls && (!values0 || !flips))) return -1;
     const RoundBest none{0.0, -1};
     CUDA_TRY(cudaMemcpyAsync(best, &none, sizeof(none), cudaMemcpyHostToDevice, ctx->stream));
-    if (nc) {
-        CUDA_TRY(cudaMemcpyAsync(er, hr.data(), (size_t)nc * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-        CUDA_TRY(cudaMemcpyAsync(ec, hc.data(), (size_t)nc * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-        CUDA_TRY(cudaMemcpyAsync(ev, hv.data(), (size_t)nc * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    }
     for (int64_t b0 = 0; b0 < nblocks; b0 += bp) {
         const int64_t b1 = std::min(nblocks, b0 + bp);
         const int64_t t0 = b0 * tb;
@@ -284,25 +588,98 @@ int k_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int
             if (k_trsm(s, L, Vb, n, tb, 1)) return -1;
         }
         const int T = (int)std::min<int64_t>(trials - t0, (b1 - b0) * tb);
-        const int nw = (T + 63) / 64;
-        {
-            LaunchScope ls(ctx, "round_eval", 4);
-            round_pack_kernel<<<dim3((unsigned)((n + 255) / 256), (unsigned)nw), 256, 0, ctx->stream>>>(V, n, n, T, bits);
-            round_eval_kernel<<<dim3((unsigned)S, (unsigned)nw), 32 * EV_WARPS, 0, ctx->stream>>>(er, ec, ev, nc, per, bits, n, part);
-            round_sum_kernel<<<(unsigned)((T + 255) / 256), 256, 0, ctx->stream>>>(part, S, T, t0, values);
-            round_best_kernel<<<1, BEST_THREADS, 0, ctx->stream>>>(values, t0, T, bits, n, best, x);
+        if (!ls) {
+            if (eval_pass(ctx, V, n, T, bits, o, part, t0, values, best, x)) return -1;
+            continue;
         }
-        CUDA_TRY(cudaGetLastError());
+        if (eval_pass(ctx, V, n, T, bits, o, part, t0, values0, nullptr, nullptr)) return -1;
+        if (launch_ls(ctx, n, T, bits, d, ls->max_flips, V, flips + t0)) return -1;
+        if (eval_pass(ctx, V, n, T, bits, o, part, t0, values, best, x)) return -1;
     }
     RoundBest hb;
     CUDA_TRY(cudaMemcpyAsync(values_host, values, (size_t)trials * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaMemcpyAsync(x_host, x, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaMemcpyAsync(&hb, best, sizeof(hb), cudaMemcpyDeviceToHost, ctx->stream));
+    if (ls) {
+        static_assert(sizeof(long long) == sizeof(int64_t), "flip counts are copied as int64");
+        CUDA_TRY(cudaMemcpyAsync(ls->values0_host, values0, (size_t)trials * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(cudaMemcpyAsync(ls->flips_host, flips, (size_t)trials * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+    }
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (hb.t < 0) {
-        smcp_set_error("smcp_round_pm1: no trial has a finite value");
+        smcp_set_error("%s: no trial has a finite value", fn);
         return -1;
     }
     *best_out = hb.t;
+    return 0;
+}
+
+int k_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc, const int64_t *crow,
+                const int64_t *ccol, const double *cval, double *values_host, int8_t *x_host, int64_t *best_out) {
+    return round_pm1_impl(s, L, seed, trials, chunk, nc, crow, ccol, cval, nullptr, values_host, x_host, best_out);
+}
+
+int k_round_pm1_ls(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc, const int64_t *crow,
+                   const int64_t *ccol, const double *cval, int64_t max_flips, double tol, double *values0_host,
+                   double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host) {
+    const LsArgs ls{max_flips, tol, values0_host, flips_host};
+    return round_pm1_impl(s, L, seed, trials, chunk, nc, crow, ccol, cval, &ls, values_host, x_host, best_out);
+}
+
+int k_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow, const int64_t *ccol,
+                       const double *cval, int64_t max_flips, double tol, double *values_host, int64_t *flips_host) {
+    const char *fn = "smcp_pm1_local_search";
+    if (n < 1 || k < 1 || nc < 0) {
+        smcp_set_error("%s: need n >= 1, k >= 1, nc >= 0 (got %lld, %lld, %lld)", fn, (long long)n, (long long)k, (long long)nc);
+        return -2;
+    }
+    if (!x_host || !values_host || !flips_host || (nc > 0 && (!crow || !ccol || !cval))) {
+        smcp_set_error("%s: null argument", fn);
+        return -2;
+    }
+    if (ls_check(fn, (int)std::min<int64_t>(n, INT32_MAX), max_flips, tol)) return -2;
+    for (int64_t e = 0; e < n * k; ++e)
+        if (x_host[e] != 1 && x_host[e] != -1) {
+            smcp_set_error("%s: x[%lld][%lld] = %d is not +-1", fn, (long long)(e / n), (long long)(e % n), (int)x_host[e]);
+            return -2;
+        }
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    // trials per pass: the s workspace (n x pw doubles) within 1 GiB, as in smcp_round_pm1
+    const int64_t fit = std::max<int64_t>(1, (int64_t(1) << 30) / (8 * n));
+    const int64_t pw = std::min<int64_t>(k, std::min<int64_t>(fit, ROUND_MAX_PASS));
+    const int64_t nwmax = (pw + 63) / 64;
+    RoundWs ws{ctx, fn, {}};
+    RoundObj o;
+    if (int rc = round_obj_upload(ws, fn, (int)n, nc, crow, ccol, cval, o)) return rc;
+    LsRows d;
+    if (ls_rows_upload(ws, (int)n, nc, crow, ccol, cval, tol, d)) return -1;
+    double *V = (double *)ws.alloc((size_t)n * pw * sizeof(double));
+    unsigned long long *bits = (unsigned long long *)ws.alloc((size_t)n * nwmax * sizeof(unsigned long long));
+    double *part = (double *)ws.alloc((size_t)nwmax * o.S * 64 * sizeof(double));
+    double *values = (double *)ws.alloc((size_t)k * sizeof(double));
+    long long *flips = (long long *)ws.alloc((size_t)k * sizeof(long long));
+    if (!V || !bits || !part || !values || !flips) return -1;
+    std::vector<double> hx((size_t)n * pw);
+    for (int64_t t0 = 0; t0 < k; t0 += pw) {
+        const int T = (int)std::min<int64_t>(pw, k - t0);
+        const size_t len = (size_t)n * T;
+        for (size_t e = 0; e < len; ++e) hx[e] = (double)x_host[(size_t)t0 * n + e];
+        CUDA_TRY(cudaMemcpyAsync(V, hx.data(), len * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        {
+            LaunchScope ls(ctx, "round_eval");
+            round_pack_kernel<<<dim3((unsigned)((n + 255) / 256), (unsigned)((T + 63) / 64)), 256, 0, ctx->stream>>>(V, n, (int)n, T,
+                                                                                                                  bits);
+        }
+        CUDA_TRY(cudaGetLastError());
+        if (launch_ls(ctx, (int)n, T, bits, d, max_flips, V, flips + t0)) return -1;
+        if (eval_pass(ctx, V, (int)n, T, bits, o, part, t0, values, nullptr, nullptr)) return -1;
+        CUDA_TRY(cudaMemcpyAsync(hx.data(), V, len * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+        for (size_t e = 0; e < len; ++e) x_host[(size_t)t0 * n + e] = hx[e] < 0.0 ? -1 : 1;
+    }
+    static_assert(sizeof(long long) == sizeof(int64_t), "flip counts are copied as int64");
+    CUDA_TRY(cudaMemcpyAsync(values_host, values, (size_t)k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(flips_host, flips, (size_t)k * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return 0;
 }

@@ -18,6 +18,7 @@ _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "libsmcp_b2
 _i64p = np.ctypeslib.ndpointer(dtype=np.int64, flags="C_CONTIGUOUS")
 _f64p = np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS")
 _i32p = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
+_i8p = np.ctypeslib.ndpointer(dtype=np.int8, flags="C_CONTIGUOUS")
 
 
 class SymDesc(C.Structure):
@@ -71,6 +72,9 @@ API = {
     "smcp_csp_sample": (_int, [_vp, _dp, C.c_uint64, _i64, _dp, _i64, _i64]),
     "smcp_round_pm1": (_int, [_vp, _dp, C.c_uint64, _i64, _i64, _i64, _i64p, _i64p, _f64p, _f64p,
                               np.ctypeslib.ndpointer(dtype=np.int8, flags="C_CONTIGUOUS"), C.POINTER(_i64)]),
+    "smcp_round_pm1_ls": (_int, [_vp, _dp, C.c_uint64, _i64, _i64, _i64, _i64p, _i64p, _f64p, _i64, _dbl, _f64p, _f64p,
+                                 _i8p, C.POINTER(_i64), _i64p]),
+    "smcp_pm1_local_search": (_int, [_vp, _i64, _i64, _i8p, _i64, _i64p, _i64p, _f64p, _i64, _dbl, _f64p, _i64p]),
     "smcp_hess_create": (_int, [_vp, _dp, _dp, C.POINTER(_vp)]),
     "smcp_hess_destroy": (_int, [_vp]),
     "smcp_hess_apply": (_int, [_vp, _dp, _i64, _int]),
@@ -506,6 +510,46 @@ class DeviceBackend:
         TRAFFIC["h2d"] += 24 * len(cval)
         TRAFFIC["d2h"] += 8 * len(values) + len(x)
         return values, x, best.value
+
+    def round_pm1_ls(self, Lbuf, crow, ccol, cval, trials, seed, chunk=0, max_flips=None, tol=1e-12):
+        """``round_pm1`` with the one-flip local search run on every trial on the device (``smcp_round_pm1_ls``;
+        ``max_flips`` None: n).  Returns ``(values0, values, flips, x, best)``: the value of every trial before and
+        after the search, its number of flips, and the int8 sign vector (internal order) and index of the best
+        searched trial."""
+        crow, ccol = _i64(crow), _i64(ccol)
+        cval = np.ascontiguousarray(cval, dtype=np.float64)
+        if not len(crow) == len(ccol) == len(cval):
+            raise ValueError("crow, ccol and cval must have the same length")
+        n = self.symb.n
+        max_flips = n if max_flips is None else int(max_flips)
+        nt = max(0, int(trials))
+        values0, values, flips = np.empty(nt), np.empty(nt), np.empty(nt, dtype=np.int64)
+        x = np.empty(n, dtype=np.int8)
+        best = C.c_int64()
+        _ck(self.lib, self.lib.smcp_round_pm1_ls(self.sym, Lbuf, int(seed), int(trials), int(chunk), len(cval), crow, ccol, cval,
+                                                 max_flips, float(tol), values0, values, x, C.byref(best), flips))
+        TRAFFIC["h2d"] += 24 * len(cval)
+        TRAFFIC["d2h"] += 24 * nt + n
+        return values0, values, flips, x, best.value
+
+    def pm1_local_search(self, x, crow, ccol, cval, max_flips=None, tol=1e-12):
+        """One-flip local search of the rows of the k x n +-1 array ``x`` against the objective given by its entries
+        (``crow``, ``ccol``, ``cval``, in the coordinates of x) on the device (``smcp_pm1_local_search``;
+        ``max_flips`` None: n).  Returns ``(x, values, flips)``: the searched int8 vectors (a new array), their
+        values and their numbers of flips."""
+        crow, ccol = _i64(crow), _i64(ccol)
+        cval = np.ascontiguousarray(cval, dtype=np.float64)
+        if not len(crow) == len(ccol) == len(cval):
+            raise ValueError("crow, ccol and cval must have the same length")
+        x = np.array(x, dtype=np.int8, order="C", ndmin=2)
+        k, n = x.shape
+        max_flips = n if max_flips is None else int(max_flips)
+        values, flips = np.empty(k), np.empty(k, dtype=np.int64)
+        _ck(self.lib, self.lib.smcp_pm1_local_search(self.ctx.h, n, k, x, len(cval), crow, ccol, cval, max_flips, float(tol),
+                                                     values, flips))
+        TRAFFIC["h2d"] += 24 * len(cval) + 8 * x.size
+        TRAFFIC["d2h"] += 8 * x.size + 16 * k
+        return x, values, flips
 
     def cholesky_batch(self, buf, count):
         info = np.zeros(count, dtype=np.int32)
