@@ -167,6 +167,31 @@ int smcp_round_pm1_ls(smcp_sym *sym, const double *L, uint64_t seed, int64_t tri
 int smcp_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host,
                           int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
                           int64_t max_flips, double tol, double *values_host, int64_t *flips_host);
+/* Tabu search of ±1 vectors against the same f, rows, s_i and g_i.  D_0 = 0; move u flips the admissible vertex i of
+ * largest g_i (lowest index on ties) and sets D_{u+1} = D_u - 4 g_i (in double, in that form); D_best is the smallest D
+ * so far, updated on a strict decrease only.  A vertex flipped by move u is tabu during moves u+1 .. u+tenure; every
+ * vertex that is not tabu is admissible whatever its gain, a tabu vertex only when D_u - 4 g_i < D_best (aspiration).
+ * Then s is updated along row i as in the one-flip search.  The search stops after tabu_iters moves, or when no vertex
+ * is admissible (possible only for tenure >= n), and returns the vector of the earliest move count at which D reached
+ * D_best (the start if D never drops below 0).  Values are evaluated as smcp_round_pm1 evaluates its trials.  Needs
+ * n <= 2^19, 0 <= tenure <= 8192 and tabu_iters >= 0 (-2 otherwise).
+ * smcp_round_pm1_tabu: smcp_round_pm1_ls, with the tabu search run on every trial after the one-flip search (which runs
+ * only when max_flips > 0; flips_host is 0 otherwise); values0_host[t] is the value of the rounded trial t,
+ * values1_host[t] its value before the tabu search, moves_host[t] its number of moves and best_iter_host[t] the move
+ * count of the returned vector; values_host, x_host and *best_out refer to the trials after the tabu search.
+ * smcp_pm1_tabu_search: the tabu search (tabu_iters = iters) on k caller-given vectors x_host (k x n int8, every entry
+ * ±1), replaced by the searched ones; values_host, moves_host and best_iter_host as above.  Its workspace follows the
+ * pass rule of smcp_round_pm1 (n x pass doubles within 1 GiB). */
+int smcp_round_pm1_tabu(smcp_sym *sym, const double *L, uint64_t seed, int64_t trials, int64_t chunk,
+                        int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
+                        int64_t max_flips, double tol, double *values0_host,
+                        double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host,
+                        int64_t tabu_iters, int64_t tenure, double *values1_host, int64_t *moves_host,
+                        int64_t *best_iter_host);
+int smcp_pm1_tabu_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host,
+                         int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
+                         int64_t iters, int64_t tenure, double *values_host, int64_t *moves_host,
+                         int64_t *best_iter_host);
 
 /* ---- barrier Hessian: chompack.hessian(L, Y, U, adj=None, inv=...) ---------------------- */
 int smcp_hess_create(smcp_sym *sym, const double *L, const double *Y, smcp_hess **out);

@@ -295,7 +295,8 @@ class SDP(object):
         return X0, sol
 
     # -- rounding (an extension: the reference has none) ---------------------------------
-    def round_pm1(self, sol, trials=256, seed=0, chunk=0, local_search=False, max_flips=None, tol=1e-12):
+    def round_pm1(self, sol, trials=256, seed=0, chunk=0, local_search=False, max_flips=None, tol=1e-12, tabu_iters=0,
+                  tenure=None):
         """Goemans-Williamson rounding of a solution with diag(X) = 1: ``trials`` sign vectors
         s_t = sign(v_t), v_t drawn with covariance the max-det completion of ``sol['x']``
         (``completion_sample``), evaluated against the objective C on the device; ``chunk`` trials per pass
@@ -307,7 +308,12 @@ class SDP(object):
         ``local_search=True`` runs the one-flip local search of ``local_search_pm1`` (``max_flips``, ``tol``) on
         every trial on the device, in the internal order of the completion (which decides ties); ``x``, ``value``,
         ``values`` and ``trial`` then refer to the searched trials, ``values_rounded`` holds the values before the
-        search and ``flips`` the number of flips of every trial."""
+        search and ``flips`` the number of flips of every trial.
+
+        ``tabu_iters > 0`` runs the tabu search of ``tabu_search_pm1`` (``tabu_iters`` moves, ``tenure``) on every
+        trial on the device, after the one-flip search when that is on; ``x``, ``value``, ``values`` and ``trial``
+        then refer to the trials after the tabu search, ``values_before_tabu`` holds the values before it, ``moves``
+        the number of moves and ``best_iter`` the move count of every returned vector."""
         trials = _check_count(trials, "trials", 1)
         seed = _check_seed(seed)
         chunk = _check_count(chunk, "chunk", 0)
@@ -316,6 +322,8 @@ class SDP(object):
         if max_flips is not None:
             max_flips = _check_count(max_flips, "max_flips", 0)
         tol = _check_tol(tol)
+        tabu_iters = _check_count(tabu_iters, "tabu_iters", 0)
+        tenure = _tabu_tenure(self.n) if tenure is None else _check_count(tenure, "tenure", 0)
         if not isinstance(sol, dict) or "x" not in sol:
             raise ValueError("sol must be a solution dict holding 'x'")
         L, order = _completion_factor(sol["x"])
@@ -326,7 +334,14 @@ class SDP(object):
         pos = np.empty(n, dtype=np.int64)
         pos[order] = np.arange(n, dtype=np.int64)
         out = {}
-        if local_search:
+        if tabu_iters > 0:
+            mf = (n if max_flips is None else max_flips) if local_search else 0
+            values0, values1, values, flips, moves, best_iter, xi, best = L.ops.round_pm1_tabu(
+                L.buf, pos[I], pos[J], v, trials, seed, tabu_iters, tenure, chunk, mf, tol)
+            out = {"values_before_tabu": values1, "moves": moves, "best_iter": best_iter}
+            if local_search:
+                out.update({"values_rounded": values0, "flips": flips})
+        elif local_search:
             values0, values, flips, xi, best = L.ops.round_pm1_ls(L.buf, pos[I], pos[J], v, trials, seed, chunk,
                                                                   max_flips, tol)
             out = {"values_rounded": values0, "flips": flips}
@@ -353,6 +368,29 @@ class SDP(object):
         xs, values, flips = ops.pm1_local_search(xa.reshape(-1, n), I, J, v, max_flips, tol)
         shape = np.shape(x)
         return {"x": xs.reshape(shape), "values": values.reshape(shape[:-1]), "flips": flips.reshape(shape[:-1])}
+
+    def tabu_search_pm1(self, x, iters, tenure=None):
+        """Tabu search of +-1 vectors against f(x) = C . x x^T (minimized), on the device (an extension).
+        ``x``: integers +-1 of shape (n,) or (k, n), original order.  With s_i and the gain g_i = x_i s_i of
+        ``local_search_pm1``, D_0 = 0 and move u flips the admissible vertex i with the largest g_i (lowest index on
+        ties), setting D_{u+1} = D_u - 4 g_i, the change of f.  A vertex flipped by move u is tabu during moves
+        u+1 .. u+``tenure`` (None: min(n - 1, 10 + n // 100)); a tabu vertex is admissible only when the move would
+        bring D below its smallest value so far (aspiration), every other vertex always is, even when its flip
+        raises f.  A vector's search stops after ``iters`` moves, or when no vertex is admissible, and returns the
+        earliest vector with the smallest D.  Returns a dict: ``x`` (int8, the shape of the input), ``values`` = f
+        of the returned vectors, ``moves``, the numbers of moves made, and ``best_iter``, the move count of each
+        returned vector (0: the input); the last three of shape x.shape[:-1].  Needs n <= 2**19 and
+        tenure <= 8192."""
+        n = self.n
+        xa = _check_pm1(x, n)
+        iters = _check_count(iters, "iters", 0)
+        tenure = _tabu_tenure(n) if tenure is None else _check_count(tenure, "tenure", 0)
+        I, J, v = self._objective_entries()
+        ops = solvers._make_backend(Symbolic(n, np.arange(n + 1), np.arange(n)))
+        xs, values, moves, best_iter = ops.pm1_tabu_search(xa, I, J, v, iters, tenure)
+        shape = np.shape(x)
+        return {"x": xs.reshape(shape), "values": values.reshape(shape[:-1]), "moves": moves.reshape(shape[:-1]),
+                "best_iter": best_iter.reshape(shape[:-1])}
 
     def _objective_entries(self):
         """Lower-triangular entries (row, col, value) of C in the original order."""
@@ -579,13 +617,15 @@ class maxcut_SDP(SDP):
         self._b = np.ones(n)
         self._pname = "maxcut_n%i" % n
 
-    def cut(self, sol, trials=256, seed=0, local_search=False):
+    def cut(self, sol, trials=256, seed=0, local_search=False, tabu_iters=0):
         """A cut from a solution of the relaxation by Goemans-Williamson rounding (``SDP.round_pm1``):
         returns ``(x, weight, bound)`` with the +-1 vector x of the heaviest of ``trials`` random hyperplane
         cuts, its weight (= -C . x x^T) and the certified upper bound -``sol['dual objective']`` on every
         cut's weight.  ``local_search=True`` improves every cut by single-vertex moves first (one-flip local
-        search, see ``SDP.local_search_pm1``) and returns the heaviest improved cut."""
-        r = self.round_pm1(sol, trials=trials, seed=seed, local_search=local_search)
+        search, see ``SDP.local_search_pm1``) and returns the heaviest improved cut.  ``tabu_iters > 0`` then
+        runs that many moves of tabu search on every cut (``SDP.tabu_search_pm1``, default tenure) and returns
+        the heaviest cut it visited."""
+        r = self.round_pm1(sol, trials=trials, seed=seed, local_search=local_search, tabu_iters=tabu_iters)
         return r["x"], -r["value"], -float(sol["dual objective"])
 
 
@@ -639,6 +679,11 @@ def _check_count(k, name, lo):
     if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or int(k) < lo:
         raise ValueError("%s must be an integer >= %d" % (name, lo))
     return int(k)
+
+
+def _tabu_tenure(n):
+    """The default tabu tenure of an n-vertex search."""
+    return min(n - 1, 10 + n // 100)
 
 
 def _check_tol(tol):

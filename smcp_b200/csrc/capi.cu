@@ -533,6 +533,19 @@ extern "C" int smcp_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t
                                      int64_t *flips_host) {
     return k_pm1_local_search(ctx, n, k, x_host, nc, crow, ccol, cval, max_flips, tol, values_host, flips_host);
 }
+extern "C" int smcp_round_pm1_tabu(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc,
+                                   const int64_t *crow, const int64_t *ccol, const double *cval, int64_t max_flips, double tol,
+                                   double *values0_host, double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host,
+                                   int64_t tabu_iters, int64_t tenure, double *values1_host, int64_t *moves_host,
+                                   int64_t *best_iter_host) {
+    return k_round_pm1_tabu(s, L, seed, trials, chunk, nc, crow, ccol, cval, max_flips, tol, values0_host, values_host, x_host,
+                            best_out, flips_host, tabu_iters, tenure, values1_host, moves_host, best_iter_host);
+}
+extern "C" int smcp_pm1_tabu_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow,
+                                    const int64_t *ccol, const double *cval, int64_t iters, int64_t tenure, double *values_host,
+                                    int64_t *moves_host, int64_t *best_iter_host) {
+    return k_pm1_tabu_search(ctx, n, k, x_host, nc, crow, ccol, cval, iters, tenure, values_host, moves_host, best_iter_host);
+}
 
 // ---------------------------------------------------------------------------------------
 // Hessian factor

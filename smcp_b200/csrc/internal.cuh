@@ -293,6 +293,15 @@ int k_round_pm1_ls(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, 
                    double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host);
 int k_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow, const int64_t *ccol,
                        const double *cval, int64_t max_flips, double tol, double *values_host, int64_t *flips_host);
+// tabu search of the +-1 trials (rounding.cu): after the one-flip search inside smcp_round_pm1's passes, and on
+// caller-given vectors
+int k_round_pm1_tabu(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc,
+                     const int64_t *crow, const int64_t *ccol, const double *cval, int64_t max_flips, double tol,
+                     double *values0_host, double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host,
+                     int64_t tabu_iters, int64_t tenure, double *values1_host, int64_t *moves_host, int64_t *best_iter_host);
+int k_pm1_tabu_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow, const int64_t *ccol,
+                      const double *cval, int64_t iters, int64_t tenure, double *values_host, int64_t *moves_host,
+                      int64_t *best_iter_host);
 
 // dense path for the top set of large supernodes (bigfront.cu)
 int big_setup(smcp_sym *s, const smcp_sym_desc *D);

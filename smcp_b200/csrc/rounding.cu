@@ -16,6 +16,7 @@
 //    the device and only its sign vector returns to the host.
 //  * round_ls: one-flip local search of the +-1 trials (see the section before ROUND_MAX_PASS), between the packing
 //    of the samples and their evaluation; the searched signs are evaluated by the same round_pack / eval / sum.
+//  * round_tabu: tabu search of the +-1 trials (see the section after round_ls_kernel), after the one-flip search.
 #include "internal.cuh"
 #include <algorithm>
 #include <cmath>
@@ -234,11 +235,12 @@ __device__ __forceinline__ void ls_warp_first(double &v, int &i) {
     }
 }
 
-// largest qualifying gain of chunk c (one warp); INIT: s of the chunk's vertices is summed from their rows first
-template <bool INIT>
+// largest qualifying gain of chunk c (one warp); INIT: s of the chunk's vertices is summed from their rows first.
+// TABU (round_tabu_kernel): a vertex qualifies when its bit in tw is clear, whatever its gain, and thr is not read.
+template <bool INIT, bool TABU = false>
 __device__ __forceinline__ void ls_chunk(int c, int n, int lane, const long long *__restrict__ rp, const int *__restrict__ col,
                                          const double *__restrict__ val, const double *__restrict__ thr, const unsigned *xw,
-                                         double *s, double *cv, int *ci) {
+                                         double *s, double *cv, int *ci, const unsigned *tw = nullptr) {
     double bv = 0.0;
     int bi = -1;
     const int i1 = min(n, (c + 1) * LS_CHUNK);
@@ -255,7 +257,8 @@ __device__ __forceinline__ void ls_chunk(int c, int n, int lane, const long long
             si = s[i];
         }
         const double g = ((xw[i >> 5] >> (i & 31)) & 1u) ? -si : si;
-        if (g > thr[i] && (bi < 0 || g > bv)) { bv = g; bi = i; }
+        const bool ok = TABU ? !((tw[i >> 5] >> (i & 31)) & 1u) : g > thr[i];
+        if (ok && (bi < 0 || g > bv)) { bv = g; bi = i; }
     }
     ls_warp_first(bv, bi);
     if (lane == 0) {
@@ -344,6 +347,180 @@ __global__ void __launch_bounds__(LS_THREADS, 6) round_ls_kernel(int n, int T, c
         }
         for (int i = threadIdx.x; i < n; i += LS_THREADS) s[i] = ((xw[i >> 5] >> (i & 31)) & 1u) ? -1.0 : 1.0;
         if (threadIdx.x == 0) flips[t] = nf;
+        __syncthreads();
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Tabu search of +-1 trials: the rows, s and g of the one-flip search.  D_0 = 0; move u flips the admissible vertex i of
+// largest g_i (lowest i on ties) and sets D_{u+1} = D_u - 4 g_i; D_best, the smallest D so far, changes only on a strict
+// decrease.  A vertex flipped at move u is tabu during moves u+1 .. u+tenure; a tabu vertex is admissible only when
+// D_u - 4 g_i < D_best (aspiration), every other vertex always is.  The search stops after iters moves or when no vertex
+// is admissible (tenure >= n only) and returns the vector of the earliest move count at which D reached D_best.
+// round_tabu_kernel: round_ls_kernel's layout and chunk maxima, taken over the non-tabu vertices without threshold.  The
+// tabu set is a bit array tw plus a ring of the last `tenure` flips in shared memory; the flip leaving the ring clears
+// its bit only if the vertex has no later entry, and only then is its chunk recomputed.  Aspiration scans the ring.  The
+// best vector is a bit copy in global memory (this CTA's nxw words of bestw), taken just before the first move that
+// leaves a best state, so a descent copies nothing.
+#define TABU_MAX_N (1 << 19)
+#define TABU_MAX_TENURE 8192
+
+// n / 4 bytes of signs and tabu bits, 12 bytes per chunk and the ring: 184 KiB at n = 2^19, tenure = 8192
+static size_t tabu_smem_bytes(int n, int tenure) {
+    return ls_smem_bytes(n) + (size_t)(n + 31) / 32 * sizeof(unsigned) + (size_t)tenure * sizeof(int);
+}
+
+// the sorted columns col[0 .. d) have one in chunk c
+__device__ __forceinline__ bool tabu_row_has_chunk(const int *__restrict__ col, int d, int c) {
+    int lo = 0, hi = d;
+    while (lo < hi) {
+        const int m = (lo + hi) >> 1;
+        if (col[m] < c * LS_CHUNK) lo = m + 1;
+        else hi = m;
+    }
+    return lo < d && col[lo] < (c + 1) * LS_CHUNK;
+}
+
+// trial t of the pass: signs from bit t & 63 of the word group t >> 6 of bits, s in V[t n ..], the best vector back into
+// V[t n + i] as +-1.0 (for round_pack_kernel), the number of moves in moves[t] and the move count of the best vector in
+// best_iter[t]
+__global__ void __launch_bounds__(LS_THREADS, 4) round_tabu_kernel(int n, int T, const unsigned long long *__restrict__ bits,
+                                                                const long long *__restrict__ rp, const int *__restrict__ col,
+                                                                const double *__restrict__ val, long long iters, int tenure,
+                                                                double *V, unsigned *__restrict__ bestw,
+                                                                long long *__restrict__ moves, long long *__restrict__ best_iter) {
+    extern __shared__ __align__(16) unsigned char tabu_smem[];
+    const int nch = (n + LS_CHUNK - 1) / LS_CHUNK, nxw = (n + 31) / 32;
+    double *cv = (double *)tabu_smem;               // largest gain of the non-tabu vertices of each chunk
+    int *ci = (int *)(cv + nch);                    // its vertex, -1: none
+    unsigned *xw = (unsigned *)(ci + nch);          // bit i: x_i = -1
+    unsigned *tw = xw + nxw;                        // bit i: i is tabu
+    int *ring = (int *)(tw + nxw);                  // ring[u % tenure]: the vertex flipped by move u
+    __shared__ double wv[LS_WARPS];
+    __shared__ int wi[LS_WARPS];
+    __shared__ unsigned wdup[LS_WARPS];
+    __shared__ double D, Db;                        // D_u and D_best
+    __shared__ long long ub;                        // the move count of D_best
+    __shared__ int pick, pneg, pexp, pcopy, pend;   // pend: the current vector is the best and has no copy in bestw
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    unsigned *gb = bestw + (long long)blockIdx.x * nxw;
+    for (int t = blockIdx.x; t < T; t += gridDim.x) {
+        const unsigned long long *wg = bits + (long long)(t >> 6) * n;
+        const int b = t & 63;
+        double *s = V + (long long)t * n;
+        for (int w = warp; w < nxw; w += LS_WARPS) {
+            const int i = 32 * w + lane;
+            const unsigned m = __ballot_sync(0xffffffffu, i < n && ((wg[i] >> b) & 1ULL));
+            if (lane == 0) {
+                xw[w] = m;
+                tw[w] = 0u;
+            }
+        }
+        if (threadIdx.x == 0) {
+            D = 0.0;
+            Db = 0.0;
+            ub = 0;
+            pend = 1;
+        }
+        __syncthreads();
+        for (int c = warp; c < nch; c += LS_WARPS) ls_chunk<true, true>(c, n, lane, rp, col, val, nullptr, xw, s, cv, ci, tw);
+        __syncthreads();
+        long long u = 0;
+        for (; u < iters; ++u) {
+            const int nr = (int)min((long long)tenure, u);              // ring entries in use, all of them tabu
+            const int slot = tenure > 0 ? (int)(u % tenure) : 0;
+            const int ex = u >= tenure && tenure > 0 ? ring[slot] : -1;  // its flip leaves the ring with this move
+            double bv = 0.0;
+            int bi = -1;
+            for (int c = threadIdx.x; c < nch; c += LS_THREADS)
+                if (ls_before(cv[c], ci[c], bv, bi)) { bv = cv[c]; bi = ci[c]; }
+            bool dup = false;
+            const double d0 = D, db = Db;
+            for (int r = threadIdx.x; r < nr; r += LS_THREADS) {
+                const int v = ring[r];
+                dup |= r != slot && v == ex;
+                const double g = ((xw[v >> 5] >> (v & 31)) & 1u) ? -s[v] : s[v];
+                if (d0 - 4.0 * g < db && ls_before(g, v, bv, bi)) { bv = g; bi = v; }
+            }
+            ls_warp_first(bv, bi);
+            const unsigned wd = __ballot_sync(0xffffffffu, dup);
+            if (lane == 0) {
+                wv[warp] = bv;
+                wi[warp] = bi;
+                wdup[warp] = wd;
+            }
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                bool later = false;
+                for (int w = 0; w < LS_WARPS; ++w) later |= wdup[w] != 0u;
+                for (int w = 1; w < LS_WARPS; ++w)
+                    if (ls_before(wv[w], wi[w], bv, bi)) { bv = wv[w]; bi = wi[w]; }
+                int e = -1;
+                if (bi >= 0) {
+                    const double dn = d0 - 4.0 * bv;
+                    const bool better = dn < db;
+                    pcopy = pend && !better;
+                    pend = better;
+                    if (better) {
+                        Db = dn;
+                        ub = u + 1;
+                    }
+                    D = dn;
+                    const unsigned m = 1u << (bi & 31);
+                    pneg = (xw[bi >> 5] & m) == 0u;
+                    xw[bi >> 5] ^= m;
+                    if (tenure > 0) {
+                        tw[bi >> 5] |= m;
+                        ring[slot] = bi;
+                    }
+                    if (ex >= 0 && ex != bi && !later) {
+                        tw[ex >> 5] &= ~(1u << (ex & 31));
+                        e = ex;
+                    }
+                }
+                pick = bi;
+                pexp = e;
+            }
+            __syncthreads();
+            const int i = pick;
+            if (i < 0) break;
+            if (pcopy) {                                                 // the vector before this move, bit i restored
+                const int wi0 = i >> 5;
+                const unsigned m = 1u << (i & 31);
+                for (int w = threadIdx.x; w < nxw; w += LS_THREADS) gb[w] = w == wi0 ? xw[w] ^ m : xw[w];
+            }
+            const long long p0 = rp[i], p1 = rp[i + 1];
+            const double two = pneg ? -2.0 : 2.0;
+            for (long long p = p0 + threadIdx.x; p < p1; p += LS_THREADS) {
+                const int j = col[p];
+                s[j] = s[j] + two * val[p];
+            }
+            __syncthreads();
+            // entries as in round_ls_kernel, plus entry d + 1: the chunk of the vertex that left the tabu set
+            const int d = (int)(p1 - p0), c0 = i / LS_CHUNK, ce = pexp >= 0 ? pexp / LS_CHUNK : -1;
+            if (d + 2 >= nch) {
+                for (int c = warp; c < nch; c += LS_WARPS) ls_chunk<false, true>(c, n, lane, rp, col, val, nullptr, xw, s, cv, ci, tw);
+            } else {
+                for (int e = warp; e <= d + 1; e += LS_WARPS) {
+                    int c = c0;
+                    if (e < d) {
+                        c = col[p0 + e] / LS_CHUNK;
+                        if (c == c0 || (e > 0 && col[p0 + e - 1] / LS_CHUNK == c)) continue;
+                    } else if (e == d + 1) {
+                        if (ce < 0 || ce == c0 || tabu_row_has_chunk(col + p0, d, ce)) continue;
+                        c = ce;
+                    }
+                    ls_chunk<false, true>(c, n, lane, rp, col, val, nullptr, xw, s, cv, ci, tw);
+                }
+            }
+            __syncthreads();
+        }
+        const unsigned *res = pend ? xw : gb;
+        for (int i = threadIdx.x; i < n; i += LS_THREADS) s[i] = ((res[i >> 5] >> (i & 31)) & 1u) ? -1.0 : 1.0;
+        if (threadIdx.x == 0) {
+            moves[t] = u;
+            best_iter[t] = ub;
+        }
         __syncthreads();
     }
 }
@@ -479,14 +656,36 @@ static int ls_rows_upload(RoundWs &ws, int n, int64_t nc, const int64_t *crow, c
     return 0;
 }
 
-// checks shared by both entry points of the search
-static int ls_check(const char *fn, int n, int64_t max_flips, double tol) {
-    if (n > LS_MAX_N) {
-        smcp_set_error("%s: n = %d exceeds %d, the largest the search's shared-memory layout holds", fn, n, LS_MAX_N);
+// what runs on every trial between its packing and the evaluation that values_host reports: the one-flip search
+// (max_flips, tol; flips_host) and, with tabu, the tabu search after it (tabu_iters, tenure; moves_host, best_iter_host).
+// With tabu the one-flip search runs only when max_flips > 0.  In smcp_round_pm1_ls / _tabu, values0_host receives the
+// values of the rounded trials, and with tabu values1_host those before the tabu search.
+struct LsArgs {
+    int64_t max_flips;
+    double tol;
+    double *values0_host;
+    int64_t *flips_host;
+    bool tabu;
+    int64_t tabu_iters, tenure;
+    double *values1_host;
+    int64_t *moves_host, *best_iter_host;
+    bool one_flip() const { return !tabu || max_flips > 0; }
+};
+
+// checks shared by the entry points of the searches
+static int ls_check(const char *fn, int n, const LsArgs &a) {
+    const int nmax = a.tabu ? TABU_MAX_N : LS_MAX_N;
+    if (n > nmax) {
+        smcp_set_error("%s: n = %d exceeds %d, the largest the search's shared-memory layout holds", fn, n, nmax);
         return -2;
     }
-    if (max_flips < 0 || !(tol >= 0.0) || !std::isfinite(tol)) {
-        smcp_set_error("%s: need max_flips >= 0 and a finite tol >= 0 (got %lld, %g)", fn, (long long)max_flips, tol);
+    if (a.max_flips < 0 || !(a.tol >= 0.0) || !std::isfinite(a.tol)) {
+        smcp_set_error("%s: need max_flips >= 0 and a finite tol >= 0 (got %lld, %g)", fn, (long long)a.max_flips, a.tol);
+        return -2;
+    }
+    if (a.tabu && (a.tabu_iters < 0 || a.tenure < 0 || a.tenure > TABU_MAX_TENURE)) {
+        smcp_set_error("%s: need tabu_iters >= 0 and 0 <= tenure <= %d (got %lld, %lld)", fn, TABU_MAX_TENURE,
+                       (long long)a.tabu_iters, (long long)a.tenure);
         return -2;
     }
     return 0;
@@ -503,6 +702,26 @@ static int launch_ls(smcp_ctx *ctx, int n, int T, const unsigned long long *bits
         LaunchScope ls(ctx, "round_ls");
         round_ls_kernel<<<grid, LS_THREADS, smem, ctx->stream>>>(n, T, bits, d.rp, d.col, d.val, d.thr, (long long)max_flips, V,
                                                                  flips);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+// the tabu search of the T trials of a pass; bestw (one nxw-word copy per CTA) is allocated at the first pass, which has
+// the most trials and so the largest grid
+static int launch_tabu(RoundWs &ws, int n, int T, const unsigned long long *bits, const LsRows &d, const LsArgs &a, double *V,
+                       unsigned *&bestw, long long *moves, long long *best_iter) {
+    smcp_ctx *ctx = ws.ctx;
+    const size_t smem = tabu_smem_bytes(n, (int)a.tenure);
+    CUDA_TRY(cudaFuncSetAttribute(round_tabu_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0;
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, round_tabu_kernel, LS_THREADS, smem));
+    const int grid = std::max(1, std::min(T, std::max(1, per_sm) * ctx->num_sms));
+    if (!bestw && !(bestw = (unsigned *)ws.alloc((size_t)grid * ((n + 31) / 32) * sizeof(unsigned)))) return -1;
+    {
+        LaunchScope ls(ctx, "round_tabu");
+        round_tabu_kernel<<<grid, LS_THREADS, smem, ctx->stream>>>(n, T, bits, d.rp, d.col, d.val, (long long)a.tabu_iters,
+                                                                   (int)a.tenure, V, bestw, moves, best_iter);
     }
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -525,32 +744,45 @@ static int eval_pass(smcp_ctx *ctx, const double *V, int n, int T, unsigned long
     return 0;
 }
 
-// ls == nullptr: smcp_round_pm1; otherwise the search runs on every trial between its evaluation into
-// ls->values0_host and the evaluation that values_host, x_host and best_out report
-struct LsArgs {
-    int64_t max_flips;
-    double tol;
-    double *values0_host;
-    int64_t *flips_host;
+// device outputs of the searches over all trials; bestw is allocated by launch_tabu
+struct LsOut {
+    double *values1 = nullptr;
+    long long *flips = nullptr, *moves = nullptr, *best_iter = nullptr;
+    unsigned *bestw = nullptr;
 };
 
+// the searches of `a` on the T trials t0 .. t0 + T - 1 of a pass whose signs are packed in bits; V[:, t] then holds the
+// searched signs as +-1.0.  With tabu after the one-flip search, out.values1 receives the values in between.
+static int search_pass(RoundWs &ws, int n, int T, int64_t t0, unsigned long long *bits, const RoundObj &o, double *part,
+                       const LsRows &d, const LsArgs &a, double *V, LsOut &out) {
+    if (a.one_flip()) {
+        if (launch_ls(ws.ctx, n, T, bits, d, a.max_flips, V, out.flips + t0)) return -1;
+        if (a.tabu && eval_pass(ws.ctx, V, n, T, bits, o, part, t0, out.values1, nullptr, nullptr)) return -1;
+    }
+    if (a.tabu && launch_tabu(ws, n, T, bits, d, a, V, out.bestw, out.moves + t0, out.best_iter + t0)) return -1;
+    return 0;
+}
+
+// ls == nullptr: smcp_round_pm1; otherwise the searches run on every trial between its evaluation into
+// ls->values0_host and the evaluation that values_host, x_host and best_out report
 static int round_pm1_impl(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc,
                           const int64_t *crow, const int64_t *ccol, const double *cval, const LsArgs *ls, double *values_host,
                           int8_t *x_host, int64_t *best_out) {
     smcp_ctx *ctx = s->ctx;
     const int n = s->d.n;
-    const char *fn = ls ? "smcp_round_pm1_ls" : "smcp_round_pm1";
+    const char *fn = ls ? (ls->tabu ? "smcp_round_pm1_tabu" : "smcp_round_pm1_ls") : "smcp_round_pm1";
     if (trials < 1 || chunk < 0 || nc < 0) {
         smcp_set_error("%s: need trials >= 1, chunk >= 0, nc >= 0 (got %lld, %lld, %lld)", fn, (long long)trials,
                        (long long)chunk, (long long)nc);
         return -2;
     }
     if (!L || !values_host || !x_host || !best_out || (nc > 0 && (!crow || !ccol || !cval)) ||
-        (ls && (!ls->values0_host || !ls->flips_host))) {
+        (ls && (!ls->values0_host || !ls->flips_host)) ||
+        (ls && ls->tabu && (!ls->values1_host || !ls->moves_host || !ls->best_iter_host))) {
         smcp_set_error("%s: null argument", fn);
         return -2;
     }
-    if (ls && ls_check(fn, n, ls->max_flips, ls->tol)) return -2;
+    if (ls && ls_check(fn, n, *ls)) return -2;
     // solve blocks: as few as hold ROUND_BLOCK columns each, all of the same width tb (within 1 GiB)
     const int64_t fit = std::max<int64_t>(1, (int64_t(1) << 30) / (8 * (int64_t)n));
     const int64_t bmax = std::min<int64_t>(ROUND_BLOCK, fit);
@@ -575,10 +807,20 @@ static int round_pm1_impl(smcp_sym *s, const double *L, uint64_t seed, int64_t t
     RoundBest *best = (RoundBest *)ws.alloc(sizeof(RoundBest));
     signed char *x = (signed char *)ws.alloc((size_t)n);
     double *values0 = ls ? (double *)ws.alloc((size_t)trials * sizeof(double)) : nullptr;
-    long long *flips = ls ? (long long *)ws.alloc((size_t)trials * sizeof(long long)) : nullptr;
-    if (!V || !bits || !part || !values || !best || !x || (ls && (!values0 || !flips))) return -1;
+    LsOut out;
+    const bool tabu = ls && ls->tabu, one_flip = ls && ls->one_flip();
+    if (ls) out.flips = (long long *)ws.alloc((size_t)trials * sizeof(long long));
+    if (tabu && one_flip) out.values1 = (double *)ws.alloc((size_t)trials * sizeof(double));
+    if (tabu) {
+        out.moves = (long long *)ws.alloc((size_t)trials * sizeof(long long));
+        out.best_iter = (long long *)ws.alloc((size_t)trials * sizeof(long long));
+    }
+    if (!V || !bits || !part || !values || !best || !x || (ls && (!values0 || !out.flips)) ||
+        (tabu && ((one_flip && !out.values1) || !out.moves || !out.best_iter)))
+        return -1;
     const RoundBest none{0.0, -1};
     CUDA_TRY(cudaMemcpyAsync(best, &none, sizeof(none), cudaMemcpyHostToDevice, ctx->stream));
+    if (ls && !one_flip) CUDA_TRY(cudaMemsetAsync(out.flips, 0, (size_t)trials * sizeof(long long), ctx->stream));
     for (int64_t b0 = 0; b0 < nblocks; b0 += bp) {
         const int64_t b1 = std::min(nblocks, b0 + bp);
         const int64_t t0 = b0 * tb;
@@ -593,7 +835,7 @@ static int round_pm1_impl(smcp_sym *s, const double *L, uint64_t seed, int64_t t
             continue;
         }
         if (eval_pass(ctx, V, n, T, bits, o, part, t0, values0, nullptr, nullptr)) return -1;
-        if (launch_ls(ctx, n, T, bits, d, ls->max_flips, V, flips + t0)) return -1;
+        if (search_pass(ws, n, T, t0, bits, o, part, d, *ls, V, out)) return -1;
         if (eval_pass(ctx, V, n, T, bits, o, part, t0, values, best, x)) return -1;
     }
     RoundBest hb;
@@ -603,7 +845,15 @@ static int round_pm1_impl(smcp_sym *s, const double *L, uint64_t seed, int64_t t
     if (ls) {
         static_assert(sizeof(long long) == sizeof(int64_t), "flip counts are copied as int64");
         CUDA_TRY(cudaMemcpyAsync(ls->values0_host, values0, (size_t)trials * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaMemcpyAsync(ls->flips_host, flips, (size_t)trials * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(cudaMemcpyAsync(ls->flips_host, out.flips, (size_t)trials * sizeof(long long), cudaMemcpyDeviceToHost,
+                                 ctx->stream));
+    }
+    if (tabu) {
+        CUDA_TRY(cudaMemcpyAsync(ls->values1_host, one_flip ? out.values1 : values0, (size_t)trials * sizeof(double),
+                                 cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(cudaMemcpyAsync(ls->moves_host, out.moves, (size_t)trials * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(cudaMemcpyAsync(ls->best_iter_host, out.best_iter, (size_t)trials * sizeof(long long), cudaMemcpyDeviceToHost,
+                                 ctx->stream));
     }
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     if (hb.t < 0) {
@@ -622,22 +872,31 @@ int k_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int
 int k_round_pm1_ls(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc, const int64_t *crow,
                    const int64_t *ccol, const double *cval, int64_t max_flips, double tol, double *values0_host,
                    double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host) {
-    const LsArgs ls{max_flips, tol, values0_host, flips_host};
+    const LsArgs ls{max_flips, tol, values0_host, flips_host, false, 0, 0, nullptr, nullptr, nullptr};
     return round_pm1_impl(s, L, seed, trials, chunk, nc, crow, ccol, cval, &ls, values_host, x_host, best_out);
 }
 
-int k_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow, const int64_t *ccol,
-                       const double *cval, int64_t max_flips, double tol, double *values_host, int64_t *flips_host) {
-    const char *fn = "smcp_pm1_local_search";
+int k_round_pm1_tabu(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc,
+                     const int64_t *crow, const int64_t *ccol, const double *cval, int64_t max_flips, double tol,
+                     double *values0_host, double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host,
+                     int64_t tabu_iters, int64_t tenure, double *values1_host, int64_t *moves_host, int64_t *best_iter_host) {
+    const LsArgs ls{max_flips, tol, values0_host, flips_host, true, tabu_iters, tenure, values1_host, moves_host, best_iter_host};
+    return round_pm1_impl(s, L, seed, trials, chunk, nc, crow, ccol, cval, &ls, values_host, x_host, best_out);
+}
+
+// the searches of `a` on k caller-given vectors x_host, replaced by the searched ones
+static int pm1_search_impl(smcp_ctx *ctx, const char *fn, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow,
+                           const int64_t *ccol, const double *cval, const LsArgs &a, double *values_host) {
     if (n < 1 || k < 1 || nc < 0) {
         smcp_set_error("%s: need n >= 1, k >= 1, nc >= 0 (got %lld, %lld, %lld)", fn, (long long)n, (long long)k, (long long)nc);
         return -2;
     }
-    if (!x_host || !values_host || !flips_host || (nc > 0 && (!crow || !ccol || !cval))) {
+    if (!x_host || !values_host || (nc > 0 && (!crow || !ccol || !cval)) || (a.one_flip() && !a.flips_host) ||
+        (a.tabu && (!a.moves_host || !a.best_iter_host))) {
         smcp_set_error("%s: null argument", fn);
         return -2;
     }
-    if (ls_check(fn, (int)std::min<int64_t>(n, INT32_MAX), max_flips, tol)) return -2;
+    if (ls_check(fn, (int)std::min<int64_t>(n, INT32_MAX), a)) return -2;
     for (int64_t e = 0; e < n * k; ++e)
         if (x_host[e] != 1 && x_host[e] != -1) {
             smcp_set_error("%s: x[%lld][%lld] = %d is not +-1", fn, (long long)(e / n), (long long)(e % n), (int)x_host[e]);
@@ -652,13 +911,18 @@ int k_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int6
     RoundObj o;
     if (int rc = round_obj_upload(ws, fn, (int)n, nc, crow, ccol, cval, o)) return rc;
     LsRows d;
-    if (ls_rows_upload(ws, (int)n, nc, crow, ccol, cval, tol, d)) return -1;
+    if (ls_rows_upload(ws, (int)n, nc, crow, ccol, cval, a.tol, d)) return -1;
     double *V = (double *)ws.alloc((size_t)n * pw * sizeof(double));
     unsigned long long *bits = (unsigned long long *)ws.alloc((size_t)n * nwmax * sizeof(unsigned long long));
     double *part = (double *)ws.alloc((size_t)nwmax * o.S * 64 * sizeof(double));
     double *values = (double *)ws.alloc((size_t)k * sizeof(double));
-    long long *flips = (long long *)ws.alloc((size_t)k * sizeof(long long));
-    if (!V || !bits || !part || !values || !flips) return -1;
+    LsOut out;
+    if (a.one_flip()) out.flips = (long long *)ws.alloc((size_t)k * sizeof(long long));
+    if (a.tabu) {
+        out.moves = (long long *)ws.alloc((size_t)k * sizeof(long long));
+        out.best_iter = (long long *)ws.alloc((size_t)k * sizeof(long long));
+    }
+    if (!V || !bits || !part || !values || (a.one_flip() && !out.flips) || (a.tabu && (!out.moves || !out.best_iter))) return -1;
     std::vector<double> hx((size_t)n * pw);
     for (int64_t t0 = 0; t0 < k; t0 += pw) {
         const int T = (int)std::min<int64_t>(pw, k - t0);
@@ -671,15 +935,33 @@ int k_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int6
                                                                                                                   bits);
         }
         CUDA_TRY(cudaGetLastError());
-        if (launch_ls(ctx, (int)n, T, bits, d, max_flips, V, flips + t0)) return -1;
+        if (search_pass(ws, (int)n, T, t0, bits, o, part, d, a, V, out)) return -1;
         if (eval_pass(ctx, V, (int)n, T, bits, o, part, t0, values, nullptr, nullptr)) return -1;
         CUDA_TRY(cudaMemcpyAsync(hx.data(), V, len * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
         CUDA_TRY(cudaStreamSynchronize(ctx->stream));
         for (size_t e = 0; e < len; ++e) x_host[(size_t)t0 * n + e] = hx[e] < 0.0 ? -1 : 1;
     }
-    static_assert(sizeof(long long) == sizeof(int64_t), "flip counts are copied as int64");
+    static_assert(sizeof(long long) == sizeof(int64_t), "counts are copied as int64");
     CUDA_TRY(cudaMemcpyAsync(values_host, values, (size_t)k * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(flips_host, flips, (size_t)k * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+    if (a.one_flip())
+        CUDA_TRY(cudaMemcpyAsync(a.flips_host, out.flips, (size_t)k * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+    if (a.tabu) {
+        CUDA_TRY(cudaMemcpyAsync(a.moves_host, out.moves, (size_t)k * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(cudaMemcpyAsync(a.best_iter_host, out.best_iter, (size_t)k * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+    }
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return 0;
+}
+
+int k_pm1_local_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow, const int64_t *ccol,
+                       const double *cval, int64_t max_flips, double tol, double *values_host, int64_t *flips_host) {
+    const LsArgs a{max_flips, tol, nullptr, flips_host, false, 0, 0, nullptr, nullptr, nullptr};
+    return pm1_search_impl(ctx, "smcp_pm1_local_search", n, k, x_host, nc, crow, ccol, cval, a, values_host);
+}
+
+int k_pm1_tabu_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow, const int64_t *ccol,
+                      const double *cval, int64_t iters, int64_t tenure, double *values_host, int64_t *moves_host,
+                      int64_t *best_iter_host) {
+    const LsArgs a{0, 0.0, nullptr, nullptr, true, iters, tenure, nullptr, moves_host, best_iter_host};
+    return pm1_search_impl(ctx, "smcp_pm1_tabu_search", n, k, x_host, nc, crow, ccol, cval, a, values_host);
 }

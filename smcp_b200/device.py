@@ -75,6 +75,9 @@ API = {
     "smcp_round_pm1_ls": (_int, [_vp, _dp, C.c_uint64, _i64, _i64, _i64, _i64p, _i64p, _f64p, _i64, _dbl, _f64p, _f64p,
                                  _i8p, C.POINTER(_i64), _i64p]),
     "smcp_pm1_local_search": (_int, [_vp, _i64, _i64, _i8p, _i64, _i64p, _i64p, _f64p, _i64, _dbl, _f64p, _i64p]),
+    "smcp_round_pm1_tabu": (_int, [_vp, _dp, C.c_uint64, _i64, _i64, _i64, _i64p, _i64p, _f64p, _i64, _dbl, _f64p, _f64p,
+                                   _i8p, C.POINTER(_i64), _i64p, _i64, _i64, _f64p, _i64p, _i64p]),
+    "smcp_pm1_tabu_search": (_int, [_vp, _i64, _i64, _i8p, _i64, _i64p, _i64p, _f64p, _i64, _i64, _f64p, _i64p, _i64p]),
     "smcp_hess_create": (_int, [_vp, _dp, _dp, C.POINTER(_vp)]),
     "smcp_hess_destroy": (_int, [_vp]),
     "smcp_hess_apply": (_int, [_vp, _dp, _i64, _int]),
@@ -550,6 +553,48 @@ class DeviceBackend:
         TRAFFIC["h2d"] += 24 * len(cval) + 8 * x.size
         TRAFFIC["d2h"] += 8 * x.size + 16 * k
         return x, values, flips
+
+    def round_pm1_tabu(self, Lbuf, crow, ccol, cval, trials, seed, tabu_iters, tenure, chunk=0, max_flips=0, tol=1e-12):
+        """``round_pm1_ls`` followed by ``tabu_iters`` moves of tabu search (tabu tenure ``tenure``) on every trial on
+        the device (``smcp_round_pm1_tabu``; the one-flip search runs only when ``max_flips`` > 0, None: n).  Returns
+        ``(values0, values1, values, flips, moves, best_iter, x, best)``: the value of every trial as rounded, before
+        and after the tabu search, its numbers of flips and moves and the move count of its returned vector, and the
+        int8 sign vector (internal order) and index of the best trial."""
+        crow, ccol = _i64(crow), _i64(ccol)
+        cval = np.ascontiguousarray(cval, dtype=np.float64)
+        if not len(crow) == len(ccol) == len(cval):
+            raise ValueError("crow, ccol and cval must have the same length")
+        n = self.symb.n
+        max_flips = n if max_flips is None else int(max_flips)
+        nt = max(0, int(trials))
+        values0, values1, values = np.empty(nt), np.empty(nt), np.empty(nt)
+        flips, moves, best_iter = (np.empty(nt, dtype=np.int64) for _ in range(3))
+        x = np.empty(n, dtype=np.int8)
+        best = C.c_int64()
+        _ck(self.lib, self.lib.smcp_round_pm1_tabu(self.sym, Lbuf, int(seed), int(trials), int(chunk), len(cval), crow, ccol,
+                                                   cval, max_flips, float(tol), values0, values, x, C.byref(best), flips,
+                                                   int(tabu_iters), int(tenure), values1, moves, best_iter))
+        TRAFFIC["h2d"] += 24 * len(cval)
+        TRAFFIC["d2h"] += 48 * nt + n
+        return values0, values1, values, flips, moves, best_iter, x, best.value
+
+    def pm1_tabu_search(self, x, crow, ccol, cval, iters, tenure):
+        """Tabu search (``iters`` moves, tabu tenure ``tenure``) of the rows of the k x n +-1 array ``x`` against the
+        objective given by its entries (in the coordinates of x) on the device (``smcp_pm1_tabu_search``).  Returns
+        ``(x, values, moves, best_iter)``: the returned int8 vectors (a new array), their values, the numbers of moves
+        made and the move count of each returned vector."""
+        crow, ccol = _i64(crow), _i64(ccol)
+        cval = np.ascontiguousarray(cval, dtype=np.float64)
+        if not len(crow) == len(ccol) == len(cval):
+            raise ValueError("crow, ccol and cval must have the same length")
+        x = np.array(x, dtype=np.int8, order="C", ndmin=2)
+        k, n = x.shape
+        values, moves, best_iter = np.empty(k), np.empty(k, dtype=np.int64), np.empty(k, dtype=np.int64)
+        _ck(self.lib, self.lib.smcp_pm1_tabu_search(self.ctx.h, n, k, x, len(cval), crow, ccol, cval, int(iters), int(tenure),
+                                                    values, moves, best_iter))
+        TRAFFIC["h2d"] += 24 * len(cval) + 8 * x.size
+        TRAFFIC["d2h"] += 8 * x.size + 24 * k
+        return x, values, moves, best_iter
 
     def cholesky_batch(self, buf, count):
         info = np.zeros(count, dtype=np.int32)
