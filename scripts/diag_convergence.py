@@ -11,8 +11,8 @@ solvers.options["show_progress"] = False
 solvers.options["maxiters"] = int(sys.argv[4]) if len(sys.argv) > 4 else 60
 t0 = time.time()
 sol = P.solve_feas(kktsolver="chol", primalstart={"x": P._X0})
-print("n=%d m=%d bw=%d env NO_CHAIN=%s GAMMA_MAX=%s: status %s, %d iterations, %.2f s; pobj %.10e dobj %.10e gap %.2e pres %.1e dres %.1e" % (
-    n, m, bw, os.environ.get("SMCP_B200_NO_CHAIN"), os.environ.get("SMCP_B200_CHAIN_GAMMA_MAX"), sol["status"], sol["iterations"], time.time() - t0, sol["primal objective"],
+print("n=%d m=%d bw=%d env NO_CHAIN=%s: status %s, %d iterations, %.2f s; pobj %.10e dobj %.10e gap %.2e pres %.1e dres %.1e" % (
+    n, m, bw, os.environ.get("SMCP_B200_NO_CHAIN"), sol["status"], sol["iterations"], time.time() - t0, sol["primal objective"],
     sol["dual objective"], sol["gap"], sol["primal infeasibility"] or 0, sol["dual infeasibility"] or 0))
 for r in sol["trace"]:
     if r["iter"] % 4 == 0 or r["iter"] >= sol["iterations"] - 3:

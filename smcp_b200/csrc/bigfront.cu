@@ -23,22 +23,9 @@
 #include <algorithm>
 #include <cstdlib>
 
-// thin supernodes: at most THIN_NN columns (the thin_* kernels below); SMCP_B200_NO_THIN / SMCP_B200_NO_DINV switch the
-// round-2 shortcuts off for A/B measurements
+// thin supernodes: at most THIN_NN columns (the thin_* kernels below)
 #define THIN_NN 8
 #define THIN_TS 32         // tile of the alpha x alpha passes (thin_up / thin_hinv_sweep / thin_chol): 32 x 32 per CTA of 256 threads (64 x 64 was slower: 20.5 -> 30.8 us, latency bound)
-static bool dinv_on() {
-    static const bool off = getenv("SMCP_B200_NO_DINV") && atoi(getenv("SMCP_B200_NO_DINV")) != 0;
-    return !off;
-}
-static bool side_on() {
-    static const bool off = getenv("SMCP_B200_NO_SIDE") && atoi(getenv("SMCP_B200_NO_SIDE")) != 0;
-    return !off;
-}
-static bool thin_on() {
-    static const bool off = getenv("SMCP_B200_NO_THIN") && atoi(getenv("SMCP_B200_NO_THIN")) != 0;
-    return !off;
-}
 
 // ---------------------------------------------------------------------------------------
 // elementwise kernels
@@ -578,7 +565,7 @@ int big_cholesky(smcp_sym *s, const BigNode &q, double *X, int64_t b) {
     double *blk = X + (size_t)b * s->d.nblk + q.boff;
     double *Uk = s->upd + (size_t)b * s->d.nupd + q.uoff;
     double *F = WS(0);
-    if (nn <= THIN_NN && na >= 1 && thin_on()) {
+    if (nn <= THIN_NN && na >= 1) {
         if (!s->thin_counters) {
             CUDA_TRY(cudaMalloc(&s->thin_counters, 64 * sizeof(unsigned)));
             CUDA_TRY(cudaMemset(s->thin_counters, 0, 64 * sizeof(unsigned)));
@@ -1006,7 +993,7 @@ int big_hess_up(smcp_sym *s, const BigNode &q, const double *Lt, const double *Y
     double *Uk = s->upd + (size_t)b * s->d.nupd + q.uoff;
     const double *Lb = Lt + q.boff, *Ltan = Lb + nn, *Yaa = Yaa_all + q.uoff;
     double *F = WS(0), *T1 = WS(1), *T2 = WS(2);
-    if (nn <= THIN_NN && na >= 1 && thin_on()) {
+    if (nn <= THIN_NN && na >= 1) {
         // W of this supernode outlives the launch on its lane (the product below runs on a side stream): own slot
         const size_t tidx = (size_t)(&q - s->big.data());
         if (s->thin_w_off.empty()) {
@@ -1031,7 +1018,7 @@ int big_hess_up(smcp_sym *s, const BigNode &q, const double *Lt, const double *Y
         // Nothing in the rest of the leaves-to-root pass reads M_an (the parents take the update matrix): the product
         // leaves the chain of dependent launches and runs on a side stream; big_thin_join() waits for all of them before
         // the root-to-leaves pass
-        if (ctx->prof || !side_on()) {
+        if (ctx->prof) {
             if (G(s, true, false, Yaa, na, W, nn, blk + nn, nj, na, nn, na, 1.0, 0)) return -1;
         } else {
             if (s->thin_side.empty()) {
@@ -1071,7 +1058,7 @@ int big_hess_up(smcp_sym *s, const BigNode &q, const double *Lt, const double *Y
         ELEM(big_copy_mat_kernel, (long long)na * na, Faa, nj, Uk, na, na, na, 0);
     }
     // M_nn = D^{-1} F_nn D^{-1}
-    if (nn >= 256 && dinv_on()) {
+    if (nn >= 256) {
         // wide supernode (the root of rand_SDP: 1186 columns): D^-1 = L^-T L^-1 is formed ONCE per scaling point
         // (one triangular solve on the identity + one product) and every Hessian is two DMMA products instead of
         // four triangular solves with nn right-hand sides and two transposes (1.4 ms -> 0.4 ms at nn = 1186)
@@ -1129,7 +1116,7 @@ int big_hess_down(smcp_sym *s, const BigNode &q, const double *Lt, double *X, in
     double *blk = Xb + q.boff;
     const double *Ltan = Lt + q.boff + nn;
     double *Zaa = WS(0), *Mold = WS(1), *S = WS(2);
-    if (nn <= THIN_NN && na >= 1 && thin_on()) {
+    if (nn <= THIN_NN && na >= 1) {
         if (!s->thin_counters) {
             CUDA_TRY(cudaMalloc(&s->thin_counters, 64 * sizeof(unsigned)));
             CUDA_TRY(cudaMemset(s->thin_counters, 0, 64 * sizeof(unsigned)));
@@ -1167,7 +1154,7 @@ int big_hess_inv_local(smcp_sym *s, const BigNode &q, const double *Lt, const do
     const double *Lb = Lt + q.boff, *Ltan = Lb + nn, *R = Raa_all + q.uoff;
     double *D = WS(0), *Zaa = WS(1), *Man = WS(2), *T = WS(4);
     double *Mnn = KS + q.boff, *Kan = Mnn + (size_t)nn * nn;
-    if (nn <= THIN_NN && na >= 1 && thin_on()) {
+    if (nn <= THIN_NN && na >= 1) {
         if (!s->thin_counters) {
             CUDA_TRY(cudaMalloc(&s->thin_counters, 64 * sizeof(unsigned)));
             CUDA_TRY(cudaMemset(s->thin_counters, 0, 64 * sizeof(unsigned)));
@@ -1181,7 +1168,7 @@ int big_hess_inv_local(smcp_sym *s, const BigNode &q, const double *Lt, const do
         // K_an = Y_aa^-1 M_an D.  One or two columns against the ~1100-row factor R = chol(Y_aa): ONE cluster launch
         // for both substitutions; R's inverted 64 x 64 diagonal blocks are kept per supernode for the whole life of
         // the scaling point (they were rebuilt by a trtri launch in front of every solve)
-        if (nn <= 2 && na >= 256 && na <= 16384 && potrs_cluster_enabled()) {
+        if (nn <= 2 && na >= 256 && na <= 16384) {
             const size_t idx = (size_t)(&q - s->big.data());
             if (s->thin_dinv_off.empty()) {
                 size_t tot = 0;
@@ -1231,7 +1218,7 @@ int big_hess_inv_sweep(smcp_sym *s, const BigNode &q, const double *Lt, double *
     const double *Ltan = Lt + q.boff + nn;
     const double *Mnn = KS + q.boff, *Kan = Mnn + (size_t)nn * nn;
     double *Zaa = WS(1), *Man = WS(2);
-    if (nn <= THIN_NN && na >= 1 && thin_on()) {
+    if (nn <= THIN_NN && na >= 1) {
         LaunchScope ls_(ctx, "thin_hinv_sweep");
         thin_hinv_sweep_kernel<<<dim3((unsigned)((na + THIN_TS - 1) / THIN_TS), (unsigned)((na + THIN_TS - 1) / THIN_TS)), 256, 0, ctx->stream>>>(big_args(s, q, b), Lt + q.boff, Mnn,
                                                                                                                       Kan, blk, Uk);
@@ -1355,11 +1342,11 @@ int big_completion(smcp_sym *s, const BigNode &q, double *X, const double *Xin, 
     ELEM(big_compl_front_kernel, (long long)nj * nj, s->d.aaidx + q.uoff, Xi, bin, T, nn, na, nj);
     if (na) {
         if (front_potrf(ctx, T, nj, nj, na, BIG_INFO)) return -1;
-        if (!(nn <= THIN_NN && thin_on())) big_flag_kernel<<<1, 1, 0, ctx->stream>>>(BIG_INFO, s->fail + b);   // thin: in the tail kernel
+        if (nn > THIN_NN) big_flag_kernel<<<1, 1, 0, ctx->stream>>>(BIG_INFO, s->fail + b);   // thin: in the tail kernel
         big_transpose(s, T + na, nj, nn, na, Z, na);                                                // Z = R^-1 X_an
         if (d_trsm_left_lower(ctx, true, T, nj, na, Z, na, nn)) return -1;                          // W = X_aa^-1 X_an
     }
-    if (nn <= THIN_NN && na >= 1 && thin_on()) {
+    if (nn <= THIN_NN && na >= 1) {
         LaunchScope ls_(ctx, "thin_compl_tail");
         thin_compl_tail_kernel<<<(unsigned)((na + 127) / 128), 128, 0, ctx->stream>>>(nn, na, nj, T, Z, bout, BIG_INFO, s->fail + b);
         CUDA_TRY(cudaGetLastError());
@@ -1558,12 +1545,6 @@ __global__ void __launch_bounds__(256) thin_trsm_run_kernel(const int4 *__restri
 int big_trsm_all(smcp_sym *s, const double *L, double *B, int64_t ldb, int64_t nrhs, int trans) {
     smcp_ctx *ctx = s->ctx;
     const int nb = (int)s->big.size();
-    static const bool run_off = getenv("SMCP_B200_NO_TRSM_RUN") && atoi(getenv("SMCP_B200_NO_TRSM_RUN")) != 0;
-    if (!thin_on() || run_off) {
-        if (trans) { for (int i = nb - 1; i >= 0; --i) if (big_trsm_node(s, s->big[i], L, B, ldb, nrhs, 1)) return -1; }
-        else { for (int i = 0; i < nb; ++i) if (big_trsm_node(s, s->big[i], L, B, ldb, nrhs, 0)) return -1; }
-        return 0;
-    }
     if (!s->thin_desc) {
         std::vector<int4> d(nb);
         std::vector<longlong2> o(nb);
@@ -1606,7 +1587,7 @@ int big_trsm_node(smcp_sym *s, const BigNode &q, const double *L, double *B, int
     const double *blk = L + q.boff;
     const int r0 = q.r0;                                  // first row of the supernode (its columns are contiguous)
     const int *rows = s->d.rowidx + q.rowoff + nn;        // the separator rows
-    if (nn <= THIN_NN && na >= 1 && thin_on()) {
+    if (nn <= THIN_NN && na >= 1) {
         LaunchScope ls_(ctx, "thin_trsm");
         if (!trans) thin_trsm_fwd_kernel<<<(unsigned)((nrhs + 7) / 8), 256, 0, ctx->stream>>>(nn, na, nj, blk, rows, r0, B, ldb, nrhs);
         else thin_trsm_bwd_kernel<<<(unsigned)((nrhs + 7) / 8), 256, 0, ctx->stream>>>(nn, na, nj, blk, rows, r0, B, ldb, nrhs);

@@ -1239,8 +1239,7 @@ static int assemble_sparse_range(smcp_op *op, smcp_hess *h, int64_t s0, int64_t 
     // (almost) single entries; otherwise the pairwise form of the reference
     const long long cap = 25600;                 // doubles of dynamic shared memory (200 KB)
     const int E = (int)std::min<long long>(64, cap / (2 * n));
-    static const bool allow_pos = !(getenv("SMCP_B200_SCM_PAIRWISE") && atoi(getenv("SMCP_B200_SCM_PAIRWISE")) != 0);
-    if (allow_pos && op->sp_pid && E >= 2 && n < 65536 && op->npos <= 32 * SCM_T && op->npos + 1 <= cap && op->sp_avg_nnz >= 3.0) {
+    if (op->sp_pid && E >= 2 && n < 65536 && op->npos <= 32 * SCM_T && op->npos + 1 <= cap && op->sp_avg_nnz >= 3.0) {
         const int kpos = (op->npos + SCM_T - 1) / SCM_T;
         // materialised kernel matrix when it fits (SMCP_B200_SCM_KMAT_GB, default 4 GB) and pays: building it
         // costs npos^2 entries, the direct form npos * nnz per column

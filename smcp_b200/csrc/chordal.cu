@@ -22,7 +22,6 @@
 //    order (bitwise reproducible; no floating-point atomics anywhere).
 #include "internal.cuh"
 #include <cstdio>
-#include <cstdlib>
 #include <algorithm>
 
 #include "chordal_ops.cuh"
@@ -161,11 +160,10 @@ static bool use_big(const smcp_sym *s, int64_t batch) { return !s->big.empty() &
 
 // Number of ranks that share the per-supernode-independent operations on the top set (completion, the
 // Cholesky factors of Y_aa): all ranks of the communicator when the library runs as N replicas of one
-// solve (bench / drivers under torchrun); 1 otherwise.  SMCP_B200_DIST_OPS=0 keeps every rank on its own.
+// solve (bench / drivers under torchrun); 1 otherwise.
 static int dist_ops(const smcp_sym *s, int64_t batch) {
-    static const bool off = getenv("SMCP_B200_DIST_OPS") && atoi(getenv("SMCP_B200_DIST_OPS")) == 0;
     const smcp_ctx *ctx = s->ctx;
-    if (off || !ctx->nccl_comm || ctx->comm_nranks < 2 || batch != 1 || s->big.size() < 2) return 1;
+    if (!ctx->nccl_comm || ctx->comm_nranks < 2 || batch != 1 || s->big.size() < 2) return 1;
     return ctx->comm_nranks;
 }
 
@@ -187,15 +185,14 @@ static int big_sweep(smcp_sym *s, const std::vector<std::vector<int>> &levels, F
 
 // The tree kernel of an operation whose top-set part does not depend on it (completion, chol(Y_aa), the local phase of
 // the inverse Hessian: all per-supernode independent) runs on a side stream next to the concurrent lanes of the top set;
-// side_join() makes the main stream wait for it.  Off while profiling (per-launch events) and with SMCP_B200_NO_SIDE=1.
+// side_join() makes the main stream wait for it.  Off while profiling (per-launch events).
 struct SideScope {
     smcp_sym *s;
     cudaStream_t saved = nullptr;
     bool on = false;
     SideScope(smcp_sym *sym, bool enable) : s(sym) {
-        static const bool off = getenv("SMCP_B200_NO_SIDE") && atoi(getenv("SMCP_B200_NO_SIDE")) != 0;
         smcp_ctx *ctx = s->ctx;
-        if (!enable || off || ctx->prof || ctx->lanes_active) return;
+        if (!enable || ctx->prof || ctx->lanes_active) return;
         if (!s->tree_side) {
             if (cudaStreamCreateWithFlags(&s->tree_side, cudaStreamNonBlocking) != cudaSuccess) { s->tree_side = nullptr; return; }
             cudaEventCreateWithFlags(&s->tree_ev[0], cudaEventDisableTiming);
@@ -412,8 +409,7 @@ int k_hess_apply(smcp_hess *h, double *U, int64_t batch, int inv) {
     a.Yaa = h->Yaa;
     a.Raa = h->Raa;
     // forward map on a batch (Schur assembly): the top set goes to the batched dense path
-    static const bool allow_bb = !(getenv("SMCP_B200_NO_BIG_BATCH") && atoi(getenv("SMCP_B200_NO_BIG_BATCH")) != 0);
-    const bool bigb = !inv && !s->big.empty() && batch > 4 && allow_bb;
+    const bool bigb = !inv && !s->big.empty() && batch > 4;
     const bool big = use_big(s, batch);
     if (big || bigb) a.skipflag = s->big_flag;
     int threads = pick_threads(s, big || bigb);
@@ -678,9 +674,8 @@ int k_trsm(smcp_sym *s, const double *L, double *B, int64_t ldb, int64_t nrhs, i
     // sweep it comes after everything else and in the backward sweep before
     const bool big = !s->big.empty() && nrhs >= 32;
     if (big && trans && big_trsm_all(s, L, B, ldb, nrhs, 1)) return -1;
-    static const bool warp_off = getenv("SMCP_B200_NO_TRSM_WARP") && atoi(getenv("SMCP_B200_NO_TRSM_WARP")) != 0;
     const size_t tw_smem = (size_t)TW_WARPS * s->d.n * sizeof(double);
-    if (!warp_off && nrhs >= 64 && tw_smem <= 96 * 1024) {
+    if (nrhs >= 64 && tw_smem <= 96 * 1024) {
         static size_t tw_attr = 0;
         if (tw_smem > tw_attr) {
             CUDA_TRY(cudaFuncSetAttribute(trsm_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));

@@ -48,14 +48,13 @@ enum { CH_PROBE = 0, CH_FINAL = 1, CH_BASIS = 2 };
 
 #define TRI(p, q) ((p) * ((p) + 1) / 2 + (q))
 
-__device__ __forceinline__ void prefetch_l1(const void *p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 __device__ __forceinline__ void chain_cp_async8(void *smem, const void *gmem) {
     unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(sa), "l"(gmem));
 }
 
-// PF = how many nodes ahead the block / factor entries are fetched: 1 for large batches (occupancy
-// hides the latency, registers matter), 4 for a single matrix (nothing else hides it).
+// PF = how many nodes ahead the block / factor entries are fetched: 4 for the propagators (one thread per
+// (segment, basis vector) straight from global memory), 1 for the staged kernels (entries in shared memory).
 // One segment of the up sweep for matrix / basis vector b.  x, l and yaa are indexed by the ABSOLUTE
 // node number: global arrays, or shared-memory copies of the segment shifted by its first node.
 template <int W, int MODE, int PF>
@@ -95,13 +94,6 @@ __device__ __forceinline__ void chain_up_body(const ChainArgs &a, const int s, c
                     for (int i = 0; i < NJ; ++i) xb[t][i] = (MODE != CH_BASIS) ? x[(long long)(k + PF) * NJ + i] : 0.0;
 #pragma unroll
                     for (int i = 0; i < W; ++i) lb[t][i] = l[(long long)(k + PF) * NJ + 1 + i];
-                    if (MODE == CH_FINAL && PF > 1 && yaa) {      // single matrix: nothing else hides the Y_aa loads
-                        const double *yn = yaa + (long long)(k + PF) * W * W;
-                        prefetch_l1(yn);
-                        if (W * W > 16) prefetch_l1(yn + 16);
-                        if (W * W > 32) prefetch_l1(yn + 32);
-                        if (W * W > 48) prefetch_l1(yn + W * W - 1);
-                    }
                 }
                 const double f0 = xv[0] + u[0][0];
                 double fa[W], ka[W];
@@ -165,14 +157,14 @@ __device__ __forceinline__ void chain_up_body(const ChainArgs &a, const int s, c
     }
 }
 
-template <int W, int MODE, int PF>
+// propagators Phi_s of the up sweep: one thread per (segment, basis vector)
+template <int W>
 __global__ void __launch_bounds__(128) chain_up_kernel(ChainArgs a) {
     constexpr int D = W * (W + 1) / 2;
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const int nb = (MODE == CH_BASIS) ? D : a.B;
-    const int s = (int)(idx / nb), b = (int)(idx - (long long)s * nb);
+    const int s = (int)(idx / D), b = (int)(idx - (long long)s * D);
     if (s >= a.P) return;
-    chain_up_body<W, MODE, PF>(a, s, b, a.X + (long long)b * a.nblk, a.Lt, a.Yaa);
+    chain_up_body<W, CH_BASIS, 4>(a, s, b, a.X + (long long)b * a.nblk, a.Lt, a.Yaa);
 }
 
 // Few matrices (Newton solves, line-search steps): one WARP per (segment, matrix) copies the
@@ -270,14 +262,14 @@ __device__ __forceinline__ void chain_down_body(const ChainArgs &a, const int s,
     }
 }
 
-template <int W, int MODE, int PF>
+// propagators Phi_s of the down sweep
+template <int W>
 __global__ void __launch_bounds__(128) chain_down_kernel(ChainArgs a) {
     constexpr int D = W * (W + 1) / 2;
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const int nb = (MODE == CH_BASIS) ? D : a.B;
-    const int s = (int)(idx / nb), b = (int)(idx - (long long)s * nb);
+    const int s = (int)(idx / D), b = (int)(idx - (long long)s * D);
     if (s >= a.P) return;
-    chain_down_body<W, MODE, PF>(a, s, b, a.X + (long long)b * a.nblk, a.Lt);
+    chain_down_body<W, CH_BASIS, 4>(a, s, b, a.X + (long long)b * a.nblk, a.Lt);
 }
 
 template <int W, int MODE, bool UP>
@@ -657,12 +649,18 @@ __device__ __forceinline__ bool chain_chol_node(double *xn, double (&u)[W][W]) {
     return bad;
 }
 
-// Staged variant: a warp owns up to 32 matrices (one per lane).  The chain is cut into chunks of C
-// nodes; the warp copies the chunk of every one of its matrices into shared memory with coalesced
-// cp.async (each matrix's chunk is contiguous), double-buffered so that the next chunk is in
-// flight while the lanes run the recurrence on the current one, and writes the factor back
-// coalesced.  The kernel above issues one uncoalesced 8-byte load per lane and per entry, i.e. a
-// DRAM round trip per node (0.3 - 0.6 us): 1.7 ms for one matrix, 2.9 ms for 255 candidates.
+// Cholesky on a chain (chompack.cholesky, solvers.py:640, 884, 1218): the recurrence is NOT linear
+// (the pivot depends on the incoming update), so it stays sequential — but one THREAD per matrix
+// with the W x W update matrix in registers has a critical path of one rsqrt + three FP64 ops per
+// node (~60 cycles) instead of the ~400 cycles of a warp that exchanges the front through shared
+// memory, and a batch of line-search candidates costs the same latency as one matrix.  Same
+// operation order as the warp sweep (chordal_small.cu, SW_CHOL): bitwise identical factors.
+// A warp owns up to 32 matrices (one per lane).  The chain is cut into chunks of C nodes; the warp
+// copies the chunk of every one of its matrices into shared memory with coalesced cp.async (each
+// matrix's chunk is contiguous), double-buffered so that the next chunk is in flight while the
+// lanes run the recurrence on the current one, and writes the factor back coalesced.  Straight
+// from global memory, every lane would issue one uncoalesced 8-byte load per entry, i.e. a DRAM
+// round trip per node (0.3 - 0.6 us): 1.7 ms for one matrix, 2.9 ms for 255 candidates.
 template <int W>
 __global__ void __launch_bounds__(32) chain_chol_staged_kernel(ChainArgs a, int *fail, int C, int R) {
     constexpr int NJ = W + 1;
@@ -712,357 +710,6 @@ __global__ void __launch_bounds__(32) chain_chol_staged_kernel(ChainArgs a, int 
     if (lane < nmat) {
         anybad |= chain_chol_root<W>(a, a.X + (long long)(b0 + lane) * a.nblk, u);
         if (anybad) fail[b0 + lane] = 1;
-    }
-}
-
-// Cholesky on a chain (chompack.cholesky, solvers.py:640, 884, 1218): the recurrence is NOT linear
-// (the pivot depends on the incoming update), so it stays sequential — but one THREAD per matrix
-// with the W x W update matrix in registers has a critical path of one rsqrt + three FP64 ops per
-// node (~60 cycles) instead of the ~400 cycles of a warp that exchanges the front through shared
-// memory, and a batch of line-search candidates costs the same latency as one matrix.  Same
-// operation order as the warp sweep (chordal_small.cu, SW_CHOL): bitwise identical factors.
-// Block entries are fetched PF nodes ahead of the recurrence.
-template <int W>
-__global__ void __launch_bounds__(64) chain_chol_kernel(ChainArgs a, int *fail) {
-    constexpr int NJ = W + 1, PF = 4;
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= a.B) return;
-    double *x = a.X + (long long)b * a.nblk;
-    double u[W][W];
-#pragma unroll
-    for (int p = 0; p < W; ++p)
-#pragma unroll
-        for (int q = 0; q <= p; ++q) u[p][q] = 0.0;
-    double xb[PF][NJ];
-#pragma unroll
-    for (int t = 0; t < PF; ++t)
-#pragma unroll
-        for (int i = 0; i < NJ; ++i) xb[t][i] = (t < a.N) ? x[t * NJ + i] : 0.0;
-    bool anybad = false;
-    for (int k = 0; k < a.N; k += PF) {
-#pragma unroll
-        for (int t = 0; t < PF; ++t) {
-            if (k + t < a.N) {
-                double xv[NJ];
-#pragma unroll
-                for (int i = 0; i < NJ; ++i) xv[i] = xb[t][i];
-                if (k + t + PF < a.N) {
-#pragma unroll
-                    for (int i = 0; i < NJ; ++i) xb[t][i] = x[(long long)(k + t + PF) * NJ + i];
-                }
-                const double f0 = xv[0] + u[0][0];
-                const bool bad = !(f0 > 0.0);
-                anybad |= bad;
-                const double rs = bad ? 1.0 : rsqrt(f0);
-                double li[W];
-#pragma unroll
-                for (int i = 0; i < W; ++i) {
-                    const double fa = (i + 1 < W) ? xv[1 + i] + u[i + 1][0] : xv[1 + i];
-                    li[i] = fa * rs;
-                }
-                double un[W][W];
-#pragma unroll
-                for (int i = 0; i < W; ++i)
-#pragma unroll
-                    for (int j = 0; j <= i; ++j) {
-                        const double faa = (i + 1 < W) ? u[i + 1][j + 1] : 0.0;
-                        un[i][j] = fma(-li[i], li[j], faa);
-                    }
-#pragma unroll
-                for (int i = 0; i < W; ++i)
-#pragma unroll
-                    for (int j = 0; j <= i; ++j) u[i][j] = un[i][j];
-                double dg = f0 * rs;
-                dg = fma(fma(-dg, dg, f0), 0.5 * rs, dg);
-                double *o = x + (long long)(k + t) * NJ;
-                o[0] = bad ? 1.0 : dg;
-#pragma unroll
-                for (int i = 0; i < W; ++i) o[1 + i] = li[i];
-            }
-        }
-    }
-    anybad |= chain_chol_root<W>(a, x, u);
-    if (anybad) fail[b] = 1;
-}
-
-// ---------------------------------------------------------------------------------------
-// Single-matrix forward Hessian on a chain, ALL phases in one CTA (no launch gaps, boundary
-// states in shared memory): thread s < P owns segment s.
-//   1 up-probe | 2 up-scan (warp 0) + carry into the root | 3 up-final fused with the scaling
-//   (M_nn = K_nn / l^4, M_an = Y_aa K_an / l^2) and the root scaling (last warp) followed, with
-//   no barrier, by 4 down-probe of the same segment | 5 down-scan (warp 0) | 6 down-final.
-// The Newton solves of an iteration apply the Hessian ~20 times to ONE matrix each (solvers.py:
-// 506-539 plus iterative refinement), so this latency is what an IPM iteration waits for.
-// ---------------------------------------------------------------------------------------
-#define CH1_THREADS 256
-#define CH1_MAXP (CH1_THREADS - 32)
-
-template <int W, bool UP>
-__device__ __forceinline__ void chain_scan_smem(const ChainArgs &a, const double *phi, double *stateS, double *root, int lane) {
-    constexpr int D = W * (W + 1) / 2, PD = 3;
-    int p = 0, q = 0;
-    if (lane < D) {
-        while (TRI(p + 1, 0) <= lane) ++p;
-        q = lane - TRI(p, 0);
-    }
-    const int r = lane < D ? lane : 0;
-    double bv = 0.0;
-    if (!UP && lane < D) bv = root[p + q * a.root_nj];
-    double ph[PD][D];
-#pragma unroll
-    for (int t = 0; t < PD; ++t) {
-        const int s = UP ? t : a.P - 1 - t;
-        const bool in = t < a.P;
-        const double *src = phi + (long long)(in ? s : 0) * D * (D + 1) + r;
-#pragma unroll
-        for (int c = 0; c < D; ++c) ph[t][c] = in ? src[c * (D + 1)] : 0.0;
-    }
-    for (int it0 = 0; it0 < a.P; it0 += PD) {
-#pragma unroll
-        for (int t = 0; t < PD; ++t) {
-            const int it = it0 + t;
-            if (it < a.P) {
-                const int s = UP ? it : a.P - 1 - it;
-                double pc[D];
-#pragma unroll
-                for (int c = 0; c < D; ++c) pc[c] = ph[t][c];
-                if (it + PD < a.P) {
-                    const int sn = UP ? it + PD : a.P - 1 - (it + PD);
-                    const double *src = phi + (long long)sn * D * (D + 1) + r;
-#pragma unroll
-                    for (int c = 0; c < D; ++c) ph[t][c] = src[c * (D + 1)];
-                }
-                double acc0 = stateS[s * D + r], acc1 = 0.0, acc2 = 0.0;
-                __syncwarp();
-                if (lane < D) stateS[s * D + lane] = bv;
-#pragma unroll
-                for (int c = 0; c < D; ++c) {
-                    const double bc = __shfl_sync(0xffffffffu, bv, c);
-                    if (c % 3 == 0) acc0 = fma(pc[c], bc, acc0);
-                    else if (c % 3 == 1) acc1 = fma(pc[c], bc, acc1);
-                    else acc2 = fma(pc[c], bc, acc2);
-                }
-                bv = acc0 + (acc1 + acc2);
-            }
-        }
-    }
-    if (UP && lane < D) root[p + q * a.root_nj] += bv;
-}
-
-template <int W>
-__global__ void __launch_bounds__(CH1_THREADS) chain_hessian1_kernel(ChainArgs a, TreeArgs t, const double *phi_up, const double *phi_dn) {
-    constexpr int D = W * (W + 1) / 2, NJ = W + 1, PF = 4;
-    extern __shared__ double ch1_sm[];
-    double *stateS = ch1_sm;                       // P x D
-    double *ws = ch1_sm + (size_t)a.P * D;         // FLAT_WS doubles for the root scaling
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int s = tid;
-    const bool seg = s < a.P;
-    const int k0 = s * a.SEG, k1 = seg ? min(a.N, k0 + a.SEG) : 0;
-    double *x = a.X;
-    const double *l = a.Lt;
-    double *root = a.X + a.root_off;
-    // ---- 1: up-probe
-    if (seg) {
-        double u[W][W];
-#pragma unroll
-        for (int p = 0; p < W; ++p)
-#pragma unroll
-            for (int q = 0; q <= p; ++q) u[p][q] = 0.0;
-        double xb[PF][NJ], lb[PF][W];
-#pragma unroll
-        for (int tt = 0; tt < PF; ++tt) {
-            const bool in = k0 + tt < k1;
-#pragma unroll
-            for (int i = 0; i < NJ; ++i) xb[tt][i] = in ? x[(long long)(k0 + tt) * NJ + i] : 0.0;
-#pragma unroll
-            for (int i = 0; i < W; ++i) lb[tt][i] = in ? l[(long long)(k0 + tt) * NJ + 1 + i] : 0.0;
-        }
-        for (int kk = k0; kk < k1; kk += PF) {
-#pragma unroll
-            for (int tt = 0; tt < PF; ++tt) {
-                const int k = kk + tt;
-                if (k < k1) {
-                    double xv[NJ], lt[W];
-#pragma unroll
-                    for (int i = 0; i < NJ; ++i) xv[i] = xb[tt][i];
-#pragma unroll
-                    for (int i = 0; i < W; ++i) lt[i] = lb[tt][i];
-                    if (k + PF < k1) {
-#pragma unroll
-                        for (int i = 0; i < NJ; ++i) xb[tt][i] = x[(long long)(k + PF) * NJ + i];
-#pragma unroll
-                        for (int i = 0; i < W; ++i) lb[tt][i] = l[(long long)(k + PF) * NJ + 1 + i];
-                    }
-                    const double f0 = xv[0] + u[0][0];
-                    double fa[W], ka[W];
-#pragma unroll
-                    for (int i = 0; i < W; ++i) {
-                        fa[i] = (i + 1 < W) ? xv[1 + i] + u[i + 1][0] : xv[1 + i];
-                        ka[i] = fma(-lt[i], f0, fa[i]);
-                    }
-                    double un[W][W];
-#pragma unroll
-                    for (int i = 0; i < W; ++i)
-#pragma unroll
-                        for (int j = 0; j <= i; ++j) {
-                            const double faa = (i + 1 < W) ? u[i + 1][j + 1] : 0.0;
-                            un[i][j] = fma(-ka[i], lt[j], fma(-lt[i], fa[j], faa));
-                        }
-#pragma unroll
-                    for (int i = 0; i < W; ++i)
-#pragma unroll
-                        for (int j = 0; j <= i; ++j) u[i][j] = un[i][j];
-                }
-            }
-        }
-#pragma unroll
-        for (int p = 0; p < W; ++p)
-#pragma unroll
-            for (int q = 0; q <= p; ++q) stateS[s * D + TRI(p, q)] = u[p][q];
-    }
-    __syncthreads();
-    // ---- 2: up-scan
-    if (warp == 0) chain_scan_smem<W, true>(a, phi_up, stateS, root, lane);
-    __syncthreads();
-    // ---- 3 + 4: up-final with scaling, then down-probe of the same segment; root scaling on the last warp
-    if (warp == CH1_THREADS / 32 - 1) {
-        Node q = node_of(t.S, a.N);
-        fl_hscale(t, q, 0, ws);
-    }
-    double zst[W][W];
-    if (seg) {
-        double u[W][W];
-#pragma unroll
-        for (int p = 0; p < W; ++p)
-#pragma unroll
-            for (int q = 0; q <= p; ++q) u[p][q] = stateS[s * D + TRI(p, q)];
-        for (int k = k0; k < k1; ++k) {
-            double xv[NJ], lt[W], yy[W][W];
-            const double *xp = x + (long long)k * NJ, *lp = l + (long long)k * NJ;
-            const double *yp = t.Yaa + (long long)k * W * W;
-            if (k + 6 < k1) {       // single warp per segment group: pull the lines of node k+6 into L1 now
-                prefetch_l1(xp + 6 * NJ);
-                prefetch_l1(xp + 6 * NJ + W);
-                prefetch_l1(lp + 6 * NJ);
-                prefetch_l1(lp + 6 * NJ + W);
-                prefetch_l1(yp + 6 * W * W);
-                prefetch_l1(yp + 6 * W * W + 16);
-                if (W * W > 32) prefetch_l1(yp + 6 * W * W + 32);
-                if (W * W > 48) prefetch_l1(yp + 7 * W * W - 1);
-            }
-#pragma unroll
-            for (int i = 0; i < NJ; ++i) xv[i] = xp[i];
-            const double l0 = lp[0];
-#pragma unroll
-            for (int i = 0; i < W; ++i) lt[i] = lp[1 + i];
-#pragma unroll
-            for (int i = 0; i < W; ++i)
-#pragma unroll
-                for (int j = 0; j < W; ++j) yy[i][j] = yp[i + j * W];
-            const double f0 = xv[0] + u[0][0];
-            double fa[W], ka[W];
-#pragma unroll
-            for (int i = 0; i < W; ++i) {
-                fa[i] = (i + 1 < W) ? xv[1 + i] + u[i + 1][0] : xv[1 + i];
-                ka[i] = fma(-lt[i], f0, fa[i]);
-            }
-            double un[W][W];
-#pragma unroll
-            for (int i = 0; i < W; ++i)
-#pragma unroll
-                for (int j = 0; j <= i; ++j) {
-                    const double faa = (i + 1 < W) ? u[i + 1][j + 1] : 0.0;
-                    un[i][j] = fma(-ka[i], lt[j], fma(-lt[i], fa[j], faa));
-                }
-#pragma unroll
-            for (int i = 0; i < W; ++i)
-#pragma unroll
-                for (int j = 0; j <= i; ++j) u[i][j] = un[i][j];
-            // scaling (App. A.4 step 2, single-column supernode)
-            const double inv = 1.0 / (l0 * l0);
-            double kv[W];
-#pragma unroll
-            for (int i = 0; i < W; ++i) kv[i] = ka[i] * inv;
-            double *o = x + (long long)k * NJ;
-            o[0] = f0 * inv * inv;
-#pragma unroll
-            for (int r = 0; r < W; ++r) {
-                double acc = 0.0;
-#pragma unroll
-                for (int c = 0; c < W; ++c) acc = fma(yy[r][c], kv[c], acc);
-                o[1 + r] = acc;
-            }
-        }
-        // down-probe (zero incoming state) over the segment just written
-#pragma unroll
-        for (int p = 0; p < W; ++p)
-#pragma unroll
-            for (int q = 0; q <= p; ++q) zst[p][q] = 0.0;
-    }
-    auto down_pass = [&](bool write) {
-        for (int k = k1 - 1; k >= k0; --k) {
-            double m[NJ], lt[W];
-            double *xp = x + (long long)k * NJ;
-            const double *lp = l + (long long)k * NJ;
-            if (k - 6 >= k0) {
-                prefetch_l1(xp - 6 * NJ);
-                prefetch_l1(xp - 6 * NJ + W);
-                prefetch_l1(lp - 6 * NJ);
-                prefetch_l1(lp - 6 * NJ + W);
-            }
-#pragma unroll
-            for (int i = 0; i < NJ; ++i) m[i] = xp[i];
-#pragma unroll
-            for (int i = 0; i < W; ++i) lt[i] = lp[1 + i];
-            double za[W], tt[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) tt[i] = 0.0;
-#pragma unroll
-            for (int i = 0; i < W; ++i) {
-                double a0 = m[1 + i], a1 = 0.0;
-#pragma unroll
-                for (int r = 0; r < W; ++r) {
-                    const double zir = (i >= r) ? zst[i][r] : zst[r][i];
-                    if (r & 1) a1 = fma(-zir, lt[r], a1);
-                    else a0 = fma(-zir, lt[r], a0);
-                }
-                za[i] = a0 + a1;
-                tt[1 + i] = lt[i] * (m[1 + i] + za[i]);
-            }
-            const double z0 = m[0] - (((tt[0] + tt[1]) + (tt[2] + tt[3])) + ((tt[4] + tt[5]) + (tt[6] + tt[7])));
-            if (write) {
-                xp[0] = z0;
-#pragma unroll
-                for (int i = 0; i < W; ++i) xp[1 + i] = za[i];
-            }
-#pragma unroll
-            for (int p = W - 1; p >= 1; --p)
-#pragma unroll
-                for (int q = p; q >= 1; --q) zst[p][q] = zst[p - 1][q - 1];
-#pragma unroll
-            for (int p = 1; p < W; ++p) zst[p][0] = za[p - 1];
-            zst[0][0] = z0;
-        }
-    };
-    if (seg) {
-        down_pass(false);
-#pragma unroll
-        for (int p = 0; p < W; ++p)
-#pragma unroll
-            for (int q = 0; q <= p; ++q) stateS[s * D + TRI(p, q)] = zst[p][q];
-    }
-    __syncthreads();
-    // ---- 5: down-scan
-    if (warp == 0) chain_scan_smem<W, false>(a, phi_dn, stateS, root, lane);
-    __syncthreads();
-    // ---- 6: down-final
-    if (seg) {
-#pragma unroll
-        for (int p = 0; p < W; ++p)
-#pragma unroll
-            for (int q = 0; q <= p; ++q) zst[p][q] = stateS[s * D + TRI(p, q)];
-        down_pass(true);
     }
 }
 
@@ -1179,18 +826,16 @@ static int chain_fill(smcp_sym *s, ChainArgs &a, double *X, const double *Lt, in
 
 template <int W, int MODE>
 static void chain_launch_dir(bool up, const ChainArgs &a, cudaStream_t st) {
-    const long long threads = (long long)a.P * (MODE == CH_BASIS ? a.D : a.B);
-    const unsigned grid = (unsigned)((threads + 127) / 128);
-    static const bool staged = !(getenv("SMCP_B200_CHAIN_STAGED") && atoi(getenv("SMCP_B200_CHAIN_STAGED")) == 0);
-    if (MODE != CH_BASIS && a.B < 32 && a.SEG == CHAIN_SEG && staged) {
+    if (MODE == CH_BASIS) {
+        const unsigned grid = (unsigned)(((long long)a.P * a.D + 127) / 128);
+        if (up) chain_up_kernel<W><<<grid, 128, 0, st>>>(a);
+        else chain_down_kernel<W><<<grid, 128, 0, st>>>(a);
+    } else if (a.B < 32) {
         constexpr int WPC = (W <= 5) ? 4 : 2;
         const unsigned g2 = (unsigned)(((long long)a.P * a.B + WPC - 1) / WPC);
         if (up) chain_staged_kernel<W, MODE, true><<<g2, 32 * WPC, 0, st>>>(a);
         else chain_staged_kernel<W, MODE, false><<<g2, 32 * WPC, 0, st>>>(a);
-    } else if (MODE == CH_BASIS || a.B < 32) {
-        if (up) chain_up_kernel<W, MODE, 4><<<grid, 128, 0, st>>>(a);
-        else chain_down_kernel<W, MODE, 4><<<grid, 128, 0, st>>>(a);
-    } else if (staged && a.SEG == CHAIN_SEG && !getenv("SMCP_B200_NO_BATCH_STAGED")) {
+    } else {
         constexpr int RS = (CHAIN_SEG * (W + 1)) | 1;
         const int smem = (32 * RS + CHAIN_SEG * (W + 1) + CHAIN_SEG * W * W) * (int)sizeof(double);
         const unsigned g3 = (unsigned)((long long)a.P * ((a.B + 31) / 32));
@@ -1201,9 +846,6 @@ static void chain_launch_dir(bool up, const ChainArgs &a, cudaStream_t st) {
             cudaFuncSetAttribute(chain_staged_batch_kernel<W, MODE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
             chain_staged_batch_kernel<W, MODE, false><<<g3, 32, smem, st>>>(a);
         }
-    } else {
-        if (up) chain_up_kernel<W, MODE, 1><<<grid, 128, 0, st>>>(a);
-        else chain_down_kernel<W, MODE, 1><<<grid, 128, 0, st>>>(a);
     }
 }
 
@@ -1277,6 +919,9 @@ __global__ void chain_gamma_kernel(const double *__restrict__ phi, long long nco
     if ((threadIdx.x & 31) == 0) atomicMax(out, (unsigned long long)__double_as_longlong(mx));    // non-negative doubles order like integers
 }
 
+// largest |entry| of the segment propagators for which the segment-parallel sweeps are used
+static const double CHAIN_GAMMA_MAX = 1e3;
+
 // propagators of both sweeps for the scaling point of `h` (once per smcp_hess)
 static int chain_prepare(smcp_hess *h) {
     smcp_sym *s = h->sym;
@@ -1308,10 +953,9 @@ static int chain_prepare(smcp_hess *h) {
     // when the entries of Phi_s (products of L_an L_nn^{-1} over a segment) grow, g_s and Phi_s b_s cancel
     // and the boundary states lose digits: on the benchmark problem the Schur complement assembled through
     // the segment-parallel sweeps was only ~1e-2 accurate in the last iterations (cond(S) > 1e12) and the
-    // solver stalled at a primal residual of 3e-5.  Scaling points whose propagators exceed the threshold use
+    // solver stalled at a primal residual of 3e-5.  Scaling points whose propagators exceed CHAIN_GAMMA_MAX use
     // the sequential warp-per-chain sweeps instead (exact recurrences, ~2x slower per iteration).
     {
-        static const double gmax = getenv("SMCP_B200_CHAIN_GAMMA_MAX") ? atof(getenv("SMCP_B200_CHAIN_GAMMA_MAX")) : 1e3;
         unsigned long long *dv = (unsigned long long *)s->counter + 2;       // scratch next to the work-queue head (64 bytes)
         CUDA_TRY(cudaMemsetAsync(dv, 0, sizeof(unsigned long long), ctx->stream));
         {
@@ -1325,7 +969,7 @@ static int chain_prepare(smcp_hess *h) {
         double g;
         memcpy(&g, &hv, sizeof(g));
         h->chain_gamma = g;
-        h->chain_ok = g <= gmax;
+        h->chain_ok = g <= CHAIN_GAMMA_MAX;
         if (getenv("SMCP_B200_CHAIN_DEBUG")) fprintf(stderr, "[smcp_b200] chain propagators: max |Phi| = %.3e -> %s\n", g, h->chain_ok ? "segment-parallel sweeps" : "sequential sweeps");
     }
     return 0;
@@ -1377,17 +1021,15 @@ static int chain_cholesky(smcp_sym *s, double *X, int64_t batch, const char *nam
     smcp_ctx *ctx = s->ctx;
     ChainArgs a = {};
     if (chain_fill(s, a, X, nullptr, batch)) return -1;
-    const unsigned grid = (unsigned)((batch + 63) / 64);
-    static const bool staged = !(getenv("SMCP_B200_CHAIN_STAGED") && atoi(getenv("SMCP_B200_CHAIN_STAGED")) == 0);
-    if (staged) {
-        // chunk length: 2 buffers x 32 rows of C*NJ doubles within ~96 KB; fewer matrices -> longer chunks
-        // the recurrence costs ~300 cycles per node whatever the number of active lanes, so a batch is
-        // spread over many warps: 8 matrices per warp (255 line-search candidates -> 32 SMs)
-        const int NJ = s->chW + 1, nmat = (int)std::min<int64_t>(batch >= 64 ? 8 : 32, batch);
-        int C = 6000 / (nmat * NJ);
-        C = std::max(8, std::min(C, 512));
-        const size_t smem = (size_t)2 * nmat * ((C * NJ) | 1) * sizeof(double);
-        const unsigned g2 = (unsigned)((batch + nmat - 1) / nmat);
+    // chunk length: 2 buffers x 32 rows of C*NJ doubles within ~96 KB; fewer matrices -> longer chunks
+    // the recurrence costs ~300 cycles per node whatever the number of active lanes, so a batch is
+    // spread over many warps: 8 matrices per warp (255 line-search candidates -> 32 SMs)
+    const int NJ = s->chW + 1, nmat = (int)std::min<int64_t>(batch >= 64 ? 8 : 32, batch);
+    int C = 6000 / (nmat * NJ);
+    C = std::max(8, std::min(C, 512));
+    const size_t smem = (size_t)2 * nmat * ((C * NJ) | 1) * sizeof(double);
+    const unsigned g2 = (unsigned)((batch + nmat - 1) / nmat);
+    {
         LaunchScope ls(ctx, name, 1, (double)batch);
 #define CHOL_ST(W_)                                                                                                         \
     do {                                                                                                                    \
@@ -1404,63 +1046,7 @@ static int chain_cholesky(smcp_sym *s, double *X, int64_t batch, const char *nam
             default: CHOL_ST(7); break;
         }
 #undef CHOL_ST
-    } else {
-        LaunchScope ls(ctx, name, 1, (double)batch);
-        switch (s->chW) {
-            case 1: chain_chol_kernel<1><<<grid, 64, 0, ctx->stream>>>(a, s->fail); break;
-            case 2: chain_chol_kernel<2><<<grid, 64, 0, ctx->stream>>>(a, s->fail); break;
-            case 3: chain_chol_kernel<3><<<grid, 64, 0, ctx->stream>>>(a, s->fail); break;
-            case 4: chain_chol_kernel<4><<<grid, 64, 0, ctx->stream>>>(a, s->fail); break;
-            case 5: chain_chol_kernel<5><<<grid, 64, 0, ctx->stream>>>(a, s->fail); break;
-            case 6: chain_chol_kernel<6><<<grid, 64, 0, ctx->stream>>>(a, s->fail); break;
-            default: chain_chol_kernel<7><<<grid, 64, 0, ctx->stream>>>(a, s->fail); break;
-        }
     }
-    CUDA_TRY(cudaGetLastError());
-    return 0;
-}
-
-// single-matrix forward Hessian in one launch (falls back to the three-launch sweeps for long chains)
-static bool chain_hessian1_ok(const smcp_sym *s) { return s->chP <= CH1_MAXP; }
-
-template <int W>
-static int chain_hessian1_launch(smcp_sym *s, const ChainArgs &a, const TreeArgs &t, const double *pu, const double *pd) {
-    const size_t smem = ((size_t)a.P * a.D + FLAT_WS + 8) * sizeof(double);
-    static size_t attr = 0;
-    if (smem > attr) {
-        CUDA_TRY(cudaFuncSetAttribute(chain_hessian1_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr = smem;
-    }
-    chain_hessian1_kernel<W><<<1, CH1_THREADS, smem, s->ctx->stream>>>(a, t, pu, pd);
-    return 0;
-}
-
-static int chain_hessian1(smcp_hess *h, double *U) {
-    smcp_sym *s = h->sym;
-    smcp_ctx *ctx = s->ctx;
-    if (chain_prepare(h)) return -1;
-    ChainArgs a = {};
-    if (chain_fill(s, a, U, h->Lt, 1)) return -1;
-    TreeArgs t = {};
-    t.S = s->d;
-    t.X = U;
-    t.Lt = h->Lt;
-    t.Yaa = h->Yaa;
-    t.B = 1;
-    int rc = 0;
-    {
-        LaunchScope ls(ctx, "hessian_chain_single", 1, 1.0);
-        switch (s->chW) {
-            case 1: rc = chain_hessian1_launch<1>(s, a, t, h->phi_up, h->phi_dn); break;
-            case 2: rc = chain_hessian1_launch<2>(s, a, t, h->phi_up, h->phi_dn); break;
-            case 3: rc = chain_hessian1_launch<3>(s, a, t, h->phi_up, h->phi_dn); break;
-            case 4: rc = chain_hessian1_launch<4>(s, a, t, h->phi_up, h->phi_dn); break;
-            case 5: rc = chain_hessian1_launch<5>(s, a, t, h->phi_up, h->phi_dn); break;
-            case 6: rc = chain_hessian1_launch<6>(s, a, t, h->phi_up, h->phi_dn); break;
-            default: rc = chain_hessian1_launch<7>(s, a, t, h->phi_up, h->phi_dn); break;
-        }
-    }
-    if (rc) return rc;
     CUDA_TRY(cudaGetLastError());
     return 0;
 }

@@ -1210,7 +1210,6 @@ int ks_hess_apply(smcp_hess *h, double *U, int64_t batch, int inv) {
     if (sym_ensure(s, batch, false)) return -1;
     const bool big = batch >= 32;
     if (!inv) {
-        if (s->chain && batch == 1 && chain_hessian1_ok(s) && getenv("SMCP_B200_FUSED")) return chain_hessian1(h, U);   // experimental: slower than the 8-launch path (r01 v9)
         SmallArgs a = {};
         a.t.X = U;
         a.t.Lt = h->Lt;

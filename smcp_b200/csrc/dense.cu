@@ -8,7 +8,6 @@
 // are bank-conflict free, and keeps a 32x32 accumulator tile per warp in registers (16 warps per CTA).
 #include "internal.cuh"
 #include <algorithm>
-#include <cstdlib>
 
 // ---------------------------------------------------------------------------------------
 // DMMA GEMM:  C(i, j) = [C(i, j) +] alpha * sum_k A'(i, k) B'(j, k)
@@ -463,178 +462,10 @@ int d_gemm_tn(smcp_ctx *ctx, const double *A, int64_t lda, const double *B, int6
 
 // ---------------------------------------------------------------------------------------
 // blocked right-looking Cholesky (lower), column-major, in place (lapack.potrf, solvers.py:501)
-//
-// Two-level blocking: column blocks of OB = 128 (= one DMMA tile column, and the unit of the
-// block-cyclic distribution over GPUs), factored by two 64-column panels.
-//   panel kernel : every CTA factors the 64 x 64 diagonal block itself (one warp, rows in
-//                  registers, pivots and multipliers exchanged by shuffles: no barriers, ~10 us)
-//                  and solves X L^T = B for its 128 panel rows;
-//   DMMA kernel  : trailing updates, K = 64 inside a block, K = 128 for the rest of the matrix.
-// Look-ahead: block q+1 is updated, factored (and, with several GPUs, broadcast) on a second
-// stream while the main stream applies panel q to the blocks >= q+2.
-// Several GPUs (north star (3), SURVEY 8e): 1-D block-cyclic columns, owner(q) = q mod nranks;
-// the owner factors block q and broadcasts its columns (NCCL); every rank updates only the
-// column tiles it owns.  Every rank ends with the full factor (all panels arrive by broadcast),
-// and the arithmetic per entry is the same as on one GPU, so the result is bitwise independent
-// of the number of ranks.
 // `ncols` < m gives the partial factorisation of a frontal matrix: the leading ncols columns
 // hold L, the trailing (m - ncols)^2 block its Schur complement (the update matrix).
 // ---------------------------------------------------------------------------------------
 #define NB 64
-#define OB 128
-#define LDT 66          // column stride of the factor in shared memory
-
-#define PP_THREADS 128
-#define PP_ROWS 128       // panel rows per CTA
-
-// Cholesky of a 32 x 32 block held one row per lane (a[c] = A(lane, c), c <= lane significant).
-// Rows/columns >= nv are treated as identity.  On return a[] is the row of L (zeros above the
-// diagonal); the return value is 0 or the 1-based index of the first non-positive pivot
-// (dpotrf's info), after which the result is meaningless but finite work continues.
-// The multipliers of a step are exchanged through a 32-entry column in shared memory (double
-// buffered): one STS + 16 broadcast LDS.128 per step instead of 2 x 31 shuffles, whose
-// scoreboard-limited issue made the first version run at 0.14 instructions per cycle.
-__device__ __forceinline__ int warp_chol32(double (&a)[32], const int lane, const int nv, double *colbuf /* 2 x 32, 16-byte aligned */) {
-    int bad = 0;
-#pragma unroll
-    for (int j = 0; j < 32; ++j) {
-        double d = __shfl_sync(0xffffffffu, a[j], j);
-        if (j >= nv) d = 1.0;
-        if (!(d > 0.0)) {
-            if (!bad) bad = j + 1;
-            d = 1.0;
-        }
-        const double sq = sqrt(d);
-        const double l = (lane == j) ? sq : ((lane > j && lane < nv && j < nv) ? a[j] / sq : 0.0);
-        a[j] = l;
-        double *cb = colbuf + (j & 1) * 32;
-        cb[lane] = l;
-        __syncwarp();
-        const double2 *cb2 = reinterpret_cast<const double2 *>(cb);
-#pragma unroll
-        for (int c2 = (j + 1) / 2; c2 < 16; ++c2) {
-            const double2 lc = cb2[c2];
-            if (2 * c2 > j) a[2 * c2] = fma(-l, lc.x, a[2 * c2]);
-            a[2 * c2 + 1] = fma(-l, lc.y, a[2 * c2 + 1]);
-        }
-    }
-    return bad;
-}
-
-// Diagonal block D = H[k0:k0+kb, k0:k0+kb] (kb <= 64) factored in place by ONE warp:
-// [L11 0; L21 L22] with 32 x 32 register blocks.  A separate launch (not fused into the panel
-// kernel) because the panel CTAs must all read the FACTORED block: an in-place write-back by one
-// CTA of a fused kernel races with CTAs that are scheduled late.
-__global__ void __launch_bounds__(32) potrf_diag_kernel(double *H, long long ld, int kb, long long k0, int *info) {
-    __shared__ __align__(16) double LT[32 * LDT];      // LT[c*LDT + r] = L(r, c) for c < 32 (first block column)
-    __shared__ __align__(16) double colbuf[64];
-    const int lane = threadIdx.x;
-    double *D = H + k0 + k0 * ld;
-    double a[32], b[32];
-#pragma unroll 1
-    for (int h = 0; h < 2; ++h) {
-        const int nv = min(32, kb - 32 * h);
-        if (nv <= 0) break;
-        const int r = 32 * h + lane;
-        const bool live = lane < nv;
-        if (h == 1) {
-            // L21 = D21 L11^{-T}: right-looking substitution on this lane's row
-#pragma unroll
-            for (int c = 0; c < 32; ++c) b[c] = live ? D[r + (long long)c * ld] : 0.0;
-#pragma unroll
-            for (int c = 0; c < 32; ++c) {
-                const double x = b[c] / LT[c * LDT + c];
-                b[c] = x;
-#pragma unroll
-                for (int c2 = c + 1; c2 < 32; ++c2) b[c2] = fma(-x, LT[c * LDT + c2], b[c2]);
-            }
-#pragma unroll
-            for (int c = 0; c < 32; ++c) {
-                LT[c * LDT + r] = b[c];
-                if (live) D[r + (long long)c * ld] = b[c];
-            }
-            __syncwarp();
-        }
-#pragma unroll
-        for (int c = 0; c < 32; ++c) a[c] = (live && c <= lane) ? D[r + (long long)(32 * h + c) * ld] : 0.0;
-        if (h == 1) {
-            // D22 -= L21 L21^T
-#pragma unroll 4
-            for (int p = 0; p < 32; ++p) {
-                const double bp = LT[p * LDT + r];
-                const double2 *lp = reinterpret_cast<const double2 *>(LT + p * LDT + 32);
-#pragma unroll
-                for (int c = 0; c < 16; ++c) {
-                    const double2 lv = lp[c];
-                    a[2 * c] = fma(-bp, lv.x, a[2 * c]);
-                    a[2 * c + 1] = fma(-bp, lv.y, a[2 * c + 1]);
-                }
-            }
-        }
-        const int bad = warp_chol32(a, lane, nv, colbuf);
-        if (bad && lane == 0 && *info == 0) *info = (int)(k0 + 32 * h + bad);   // dpotrf's info
-#pragma unroll
-        for (int c = 0; c < 32; ++c)
-            if (c <= lane) {
-                if (h == 0) LT[c * LDT + r] = a[c];
-                if (live && c < nv) D[r + (long long)(32 * h + c) * ld] = a[c];
-            }
-        __syncwarp();
-    }
-}
-
-// Panel rows below a FACTORED diagonal block: X L^T = B, one row per thread, the row lives in
-// shared memory (column-major over threads, conflict free), left-looking over 8-column register
-// blocks; L is read as broadcast double2.  H has leading dimension ld and mrows rows.
-__global__ void __launch_bounds__(PP_THREADS) potrf_panel_kernel(double *H, long long ld, int kb, long long k0, long long mrows) {
-    extern __shared__ __align__(16) double ppsm[];
-    double *LT = ppsm;                       // NB x LDT: LT[c*LDT + r] = L(r, c)
-    double *xs = LT + NB * LDT;              // NB x PP_ROWS
-    const int tid = threadIdx.x;
-    const double *D = H + k0 + k0 * ld;
-    for (int idx = tid; idx < NB * LDT; idx += PP_THREADS) LT[idx] = 0.0;
-    __syncthreads();
-    for (int idx = tid; idx < kb * kb; idx += PP_THREADS) {
-        const int r = idx % kb, c = idx / kb;
-        if (r >= c) LT[c * LDT + r] = D[r + (long long)c * ld];
-    }
-    __syncthreads();
-    const long long row = k0 + kb + (long long)blockIdx.x * PP_ROWS + tid;
-    if (row >= mrows) return;
-    double *P = H + row + k0 * ld;
-    for (int c = 0; c < kb; ++c) xs[c * PP_ROWS + tid] = P[(long long)c * ld];
-    for (int cb8 = 0; cb8 < kb; cb8 += 8) {
-        double x8[8];
-#pragma unroll
-        for (int k = 0; k < 8; ++k) x8[k] = (cb8 + k < kb) ? xs[(cb8 + k) * PP_ROWS + tid] : 0.0;
-        for (int p = 0; p < cb8; ++p) {
-            const double xp = xs[p * PP_ROWS + tid];
-            const double2 *lp = reinterpret_cast<const double2 *>(LT + p * LDT + cb8);
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                const double2 lv = lp[k];
-                x8[2 * k] = fma(-xp, lv.x, x8[2 * k]);
-                x8[2 * k + 1] = fma(-xp, lv.y, x8[2 * k + 1]);
-            }
-        }
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-            if (cb8 + k < kb) {
-                const double xk = x8[k] / LT[(cb8 + k) * LDT + cb8 + k];
-                x8[k] = xk;
-#pragma unroll
-                for (int k2 = k + 1; k2 < 8; ++k2) x8[k2] = fma(-xk, LT[(cb8 + k) * LDT + cb8 + k2], x8[k2]);
-            }
-        }
-#pragma unroll
-        for (int k = 0; k < 8; ++k)
-            if (cb8 + k < kb) {
-                xs[(cb8 + k) * PP_ROWS + tid] = x8[k];
-                P[(long long)(cb8 + k) * ld] = x8[k];
-            }
-    }
-}
-
 namespace {
 struct StreamSwap {      // run the launch helpers (which use ctx->stream) on another stream
     smcp_ctx *ctx;
@@ -663,109 +494,8 @@ __global__ void panel_transpose_kernel(const double *__restrict__ P, long long l
     }
 }
 
-// factor the column block [c0, c0+w) of H (rows c0..mrows): two 64-column panels
-static int potrf_block(smcp_ctx *ctx, double *H, int64_t ld, int64_t mrows, int64_t c0, int64_t w, int32_t *info_dev, size_t pp_smem) {
-    for (int64_t k0 = c0; k0 < c0 + w; k0 += NB) {
-        const int kb = (int)std::min<int64_t>(NB, c0 + w - k0);
-        const int64_t below = mrows - k0 - kb;
-        {
-            LaunchScope ls(ctx, "potrf_panel", below > 0 ? 2 : 1, 16.0 * (double)(mrows - k0) * kb);
-            potrf_diag_kernel<<<1, 32, 0, ctx->stream>>>(H, ld, kb, k0, info_dev);
-            if (below > 0)
-                potrf_panel_kernel<<<(unsigned)((below + PP_ROWS - 1) / PP_ROWS), PP_THREADS, pp_smem, ctx->stream>>>(H, ld, kb, k0, mrows);
-        }
-        const int64_t ncr = c0 + w - (k0 + kb);      // columns of the block still to be updated
-        if (ncr > 0 && below > 0) {
-            const double *P = H + (k0 + kb) + k0 * ld;
-            double *Ct = H + (k0 + kb) + (k0 + kb) * ld;
-            if (launch_gemm(ctx, false, false, P, ld, P, ld, Ct, ld, below, ncr, kb, -1.0, 1, 1, 0, "potrf_syrk_dmma")) return -1;
-        }
-    }
-    return 0;
-}
-
-// Round-1 factorisation (launch chain: diagonal kernel + panel kernel + DMMA update per 64-column
-// panel, 128-column distribution blocks); kept behind SMCP_B200_POTRF_CHAIN=1 for A/B measurements.
-static int d_potrf_chain(smcp_ctx *ctx, double *H, int64_t ld, int64_t m, int64_t ncols, int32_t *info_dev, int rank, int nranks) {
-    if (ncols > m) ncols = m;
-    if (nranks < 1) nranks = 1;
-    const size_t pp_smem = (size_t)(NB * LDT + NB * PP_ROWS) * sizeof(double);
-    static bool pp_attr = false;
-    if (!pp_attr) {
-        CUDA_TRY(cudaFuncSetAttribute(potrf_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pp_smem));
-        pp_attr = true;
-    }
-    const int64_t nblocks = (ncols + OB - 1) / OB;
-    if (nranks > 1 && (ld != m || ncols != m)) { smcp_set_error("d_potrf: the distributed factorisation needs a full square matrix"); return -2; }
-    // one profiling scope for the whole factorisation (the two streams overlap)
-    LaunchScope outer(ctx, ctx->potrf_family ? ctx->potrf_family : "potrf_dmma", 0, (double)ncols * ncols * ncols / 3.0 + (double)(m - ncols) * ncols * (double)m);
-    ctx->prof_mute++;
-    struct Unmute { smcp_ctx *c; ~Unmute() { c->prof_mute--; } } unmute{ctx};
-    cudaStream_t sB = ctx->stream, sA = ctx->stream2;
-    static const bool lookahead = !(getenv("SMCP_B200_LOOKAHEAD") && atoi(getenv("SMCP_B200_LOOKAHEAD")) == 0);
-    // (measured at m = 1000: 1.49 -> 1.29 ms; below ~512 there is nothing to overlap)
-    const bool two = lookahead && (sA != nullptr) && (nblocks > 1) && (m >= 512);
-    if (!two) sA = sB;
-    while ((int64_t)ctx->potrf_ev.size() < 2 * nblocks + 2) {
-        cudaEvent_t e;
-        CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        ctx->potrf_ev.push_back(e);
-    }
-    cudaEvent_t *E = ctx->potrf_ev.data(), *F = ctx->potrf_ev.data() + nblocks;
-    cudaEvent_t fork = ctx->potrf_ev[2 * nblocks], join = ctx->potrf_ev[2 * nblocks + 1];
-    CUDA_TRY(cudaMemsetAsync(info_dev, 0, sizeof(int), sB));
-    if (two) {
-        CUDA_TRY(cudaEventRecord(fork, sB));
-        CUDA_TRY(cudaStreamWaitEvent(sA, fork, 0));
-    }
-    auto blk_c0 = [&](int64_t q) { return q * OB; };
-    auto blk_w = [&](int64_t q) { return std::min<int64_t>(OB, ncols - q * OB); };
-    // block 0
-    {
-        StreamSwap sw(ctx, sA);
-        if (rank == 0 % nranks && potrf_block(ctx, H, ld, m, 0, blk_w(0), info_dev, pp_smem)) return -1;
-        if (nranks > 1 && comm_bcast(ctx, H, (size_t)blk_w(0) * ld, 0, sA)) return -1;
-        if (two) CUDA_TRY(cudaEventRecord(E[0], sA));
-    }
-    for (int64_t q = 0; q < nblocks; ++q) {
-        const int64_t c0 = blk_c0(q), w = blk_w(q), c1 = c0 + w;
-        if (c1 >= m) break;
-        const double *P1 = H + c1 + c0 * ld;          // panel q, rows c1..
-        if (two) CUDA_TRY(cudaStreamWaitEvent(sB, E[q], 0));
-        int64_t c2 = c1;
-        if (q + 1 < nblocks) {
-            // look-ahead: block q+1 gets panel q, is factored and published on stream A
-            const int64_t w1 = blk_w(q + 1);
-            c2 = c1 + w1;
-            StreamSwap sw(ctx, sA);
-            if (two && q >= 1) CUDA_TRY(cudaStreamWaitEvent(sA, F[q - 1], 0));
-            if ((q + 1) % nranks == rank) {
-                if (launch_gemm(ctx, false, false, P1, ld, P1, ld, H + c1 + c1 * ld, ld, m - c1, w1, w, -1.0, 1, 1, 0, "potrf_syrk_dmma")) return -1;
-                if (potrf_block(ctx, H, ld, m, c1, w1, info_dev, pp_smem)) return -1;
-            }
-            if (nranks > 1 && comm_bcast(ctx, H + c1 * ld, (size_t)w1 * ld, (int)((q + 1) % nranks), sA)) return -1;
-            if (two) CUDA_TRY(cudaEventRecord(E[q + 1], sA));
-        }
-        // panel q applied to everything right of block q+1 (own column tiles only)
-        if (c2 < m) {
-            const double *P2 = H + c2 + c0 * ld;
-            const int64_t qb = c2 / OB;                              // block index of the first tile column
-            const int jt0 = (int)(((rank - qb) % nranks + nranks) % nranks);
-            if (launch_gemm_cyc(ctx, false, false, P2, ld, P2, ld, H + c2 + c2 * ld, ld, m - c2, m - c2, w, -1.0, 1, 1, 0,
-                                "potrf_syrk_dmma", jt0, nranks)) return -1;
-        }
-        if (two) CUDA_TRY(cudaEventRecord(F[q], sB));
-    }
-    if (two) {
-        CUDA_TRY(cudaEventRecord(join, sA));
-        CUDA_TRY(cudaStreamWaitEvent(sB, join, 0));
-    }
-    CUDA_TRY(cudaGetLastError());
-    return 0;
-}
-
 // lapack.potrf (solvers.py:501, 1931) / partial factorisation of a frontal matrix.
-//  * L2-resident matrices (m <= SMCP_B200_POTRF_TILE_MAX = 2560) on one GPU: ONE cooperative launch
+//  * L2-resident matrices (m <= POTRF_TILE_MAX) on one GPU: ONE cooperative launch
 //    (potrf_tile_kernel, dense_tile.cu).
 //  * larger m: right-looking over column blocks of `block` columns (512 on one GPU, the distribution
 //    block on several).  A block is factored by potrf_tile_kernel in panel mode (all rows of the
@@ -775,19 +505,18 @@ static int d_potrf_chain(smcp_ctx *ctx, double *H, int64_t ld, int64_t m, int64_
 //    The owner of block q+1 applies panel q to it, factors it and broadcasts it (NCCL) on the
 //    look-ahead stream while every rank applies panel q to the other blocks it owns.  Every rank ends
 //    with the full factor, and the arithmetic per entry does not depend on the number of ranks.
+static const int64_t POTRF_TILE_MAX = 2560;
+static const int POTRF_LA_CTAS = 48;
 int d_potrf(smcp_ctx *ctx, double *H, int64_t ld, int64_t m, int64_t ncols, int32_t *info_dev, int rank, int nranks, int64_t block) {
-    static const bool chain = getenv("SMCP_B200_POTRF_CHAIN") && atoi(getenv("SMCP_B200_POTRF_CHAIN")) != 0;
-    if (chain && (block == 0 || block == OB)) return d_potrf_chain(ctx, H, ld, m, ncols, info_dev, rank, nranks);
     if (ncols > m) ncols = m;
     if (nranks < 1) nranks = 1;
     if (m <= 0 || ncols <= 0) return 0;
-    static const int64_t tile_max = getenv("SMCP_B200_POTRF_TILE_MAX") ? atoll(getenv("SMCP_B200_POTRF_TILE_MAX")) : 2560;
     if (nranks > 1 && (ld != m || ncols != m)) { smcp_set_error("d_potrf: the distributed factorisation needs a full square matrix"); return -2; }
     LaunchScope outer(ctx, ctx->potrf_family ? ctx->potrf_family : "potrf_dmma", 0, (double)ncols * ncols * ncols / 3.0 + (double)(m - ncols) * ncols * (double)m);
     ctx->prof_mute++;
     struct Unmute { smcp_ctx *c; ~Unmute() { c->prof_mute--; } } unmute{ctx};
     CUDA_TRY(cudaMemsetAsync(info_dev, 0, sizeof(int), ctx->stream));
-    if (nranks == 1 && m <= tile_max && potrf_tile_fits(ctx, m, ncols, false))
+    if (nranks == 1 && m <= POTRF_TILE_MAX && potrf_tile_fits(ctx, m, ncols, false))
         return potrf_tile(ctx, H, ld, m, ncols, false, info_dev, 0);
     if (block <= 0) block = nranks > 1 ? 256 : 512;
     if (block % BN) { smcp_set_error("d_potrf: the column block must be a multiple of %d", BN); return -2; }
@@ -806,10 +535,10 @@ int d_potrf(smcp_ctx *ctx, double *H, int64_t ld, int64_t m, int64_t ncols, int3
         return potrf_tile(ctx, H + c0 + c0 * ld, ld, m - c0, w, !full_mode, info_dev, (int)c0);
     };
     // one GPU: the look-ahead schedule of the block-cyclic path -- panel q+1 on the second (high-priority) stream, on at most
-    // SMCP_B200_POTRF_LA SMs (default 48; 0 = plain loop), while the main stream applies panel q to the rest.
-    // m = 10^4: 25.6 -> 23.5 ms (gpurun_out/r02_v31_potrf_la.log)
-    static const int la_ctas = getenv("SMCP_B200_POTRF_LA") ? atoi(getenv("SMCP_B200_POTRF_LA")) : 48;
-    if (nranks == 1 && !(la_ctas > 0 && ld == m && ncols == m && ctx->stream2)) {
+    // POTRF_LA_CTAS SMs, while the main stream applies panel q to the rest.  m = 10^4: 25.6 -> 23.5 ms
+    // (profiles/r02_v31_potrf_la.log).  The plain loop below serves ld != m, partial factorisations and
+    // contexts without a second stream.
+    if (nranks == 1 && !(ld == m && ncols == m && ctx->stream2)) {
         for (int64_t q = 0; q < nblocks; ++q) {
             const int64_t c0 = q * block, w = blk_w(q), c1 = c0 + w;
             if (factor_block(q)) return -1;
@@ -836,8 +565,7 @@ int d_potrf(smcp_ctx *ctx, double *H, int64_t ld, int64_t m, int64_t ncols, int3
         CUDA_TRY(cudaStreamWaitEvent(sA, fork, 0));
     }
     // one GPU: K-major copies of the panels (two buffers: panel q+1 is transposed while panel q is still being applied)
-    static const bool pt_off = getenv("SMCP_B200_POTRF_NO_PT") && atoi(getenv("SMCP_B200_POTRF_NO_PT")) != 0;
-    const bool use_pt = nranks == 1 && !pt_off && (block % 2) == 0;
+    const bool use_pt = nranks == 1 && (block % 2) == 0;
     double *PT[2] = {nullptr, nullptr};
     if (use_pt) {
         if (grow((void **)&ctx->potrf_pt, &ctx->potrf_pt_cap, (size_t)2 * block * m * sizeof(double))) return -1;
@@ -877,7 +605,7 @@ int d_potrf(smcp_ctx *ctx, double *H, int64_t ld, int64_t m, int64_t ncols, int3
                 } else {
                     if (launch_gemm(ctx, false, false, P1, ld, P1, ld, H + c1 + c1 * ld, ld, m - c1, w1, w, -1.0, 1, 1, 0, "potrf_syrk_dmma")) return -1;
                 }
-                if (nranks == 1) ctx->potrf_grid_cap = la_ctas;
+                if (nranks == 1) ctx->potrf_grid_cap = POTRF_LA_CTAS;
                 const int rcf = factor_block(q + 1);
                 ctx->potrf_grid_cap = 0;
                 if (rcf) return -1;

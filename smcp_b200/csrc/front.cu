@@ -8,7 +8,6 @@
 // 904 (llt), 483/524/531 (hessian), 405 (inverse hessian).
 #include "internal.cuh"
 #include <algorithm>
-#include <cstdlib>
 
 #define FNB 64
 #define FLDT 66
@@ -157,20 +156,18 @@ int d_trsm_left_lower(smcp_ctx *ctx, bool trans, const double *L, int64_t ldl, i
         CUDA_TRY(cudaGetLastError());
         return 0;
     }
-    // L2-resident factors: one launch, every CTA keeps 8 right-hand sides in shared memory for the whole
-    // solve (dense_tile.cu); SMCP_B200_TRSM_BLOCKED=1 keeps the launch chain below (A/B measurements)
-    static const bool blocked_only = getenv("SMCP_B200_TRSM_BLOCKED") && atoi(getenv("SMCP_B200_TRSM_BLOCKED")) != 0;
     // one or two right-hand sides against a large factor (the ~1100-row separators of thin supernodes):
     // a single CTA is bound by what one SM pulls out of L2; a cluster of 8-16 CTAs on the inverted
     // diagonal blocks (potrs_cluster.cu) takes ~0.07 ms instead of 0.25
-    static const bool no_cluster = getenv("SMCP_B200_TRSM_NO_CLUSTER") && atoi(getenv("SMCP_B200_TRSM_NO_CLUSTER")) != 0;
-    if (!blocked_only && !no_cluster && potrs_cluster_enabled() && nrhs <= 2 && n >= 256 && n <= 16384) {
+    if (nrhs <= 2 && n >= 256 && n <= 16384) {
         const size_t need = (size_t)((n + 63) / 64) * 4096 * sizeof(double);
         if (grow((void **)&ctx->trs_dinv, &ctx->trs_dinv_cap, need)) return -1;
         if (d_potrs_prepare(ctx, L, ldl, n, ctx->trs_dinv)) return -1;
         return d_trs_cluster(ctx, L, ldl, n, ctx->trs_dinv, B, ldb, nrhs, trans ? 0 : 1, trans ? 1 : 0, "trsm_cluster");
     }
-    if (!blocked_only && trsm_slab_fits(n)) return trsm_slab(ctx, trans, L, ldl, n, B, ldb, nrhs);
+    // L2-resident factors: one launch, every CTA keeps 8 right-hand sides in shared memory for the whole
+    // solve (dense_tile.cu); larger ones take the launch chain below
+    if (trsm_slab_fits(n)) return trsm_slab(ctx, trans, L, ldl, n, B, ldb, nrhs);
     const size_t smem = (size_t)(FNB * FLDT + FNB * 128) * sizeof(double);
     static bool attr = false;
     if (!attr) {

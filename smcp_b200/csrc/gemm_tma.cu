@@ -22,7 +22,6 @@
 #include "internal.cuh"
 #include <cuda.h>
 #include <algorithm>
-#include <cstdlib>
 
 #define TM_BM 128
 #define TM_BN 128
@@ -207,8 +206,7 @@ static bool tm_make(CUtensorMap *map, const double *G, int64_t ld, int64_t rows,
 
 // true when (A, lda) / (B, ldb) are legal tensor maps and the shape is worth the pipeline
 bool gemm_tma_eligible(const double *A, int64_t lda, const double *B, int64_t ldb, int64_t M, int64_t N, int64_t K) {
-    static const bool off = getenv("SMCP_B200_NO_TMA") && atoi(getenv("SMCP_B200_NO_TMA")) != 0;
-    if (off || K < 256 || M < 1 || N < 1) return false;
+    if (K < 256 || M < 1 || N < 1) return false;
     if (((uintptr_t)A & 15) || ((uintptr_t)B & 15) || (lda & 1) || (ldb & 1)) return false;
     if (K >= (1LL << 31) || M >= (1LL << 31) || N >= (1LL << 31)) return false;
     return tm_encode_fn() != nullptr;

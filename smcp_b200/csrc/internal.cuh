@@ -334,7 +334,6 @@ int d_potrs(smcp_ctx *ctx, const double *H, int64_t m, double *y_dev);
 bool potrs_wave_for(const smcp_ctx *ctx, int64_t m);
 int d_potrs_wave(smcp_ctx *ctx, const double *H, int64_t m, const double *Dinv, double *y_dev);
 // potrs as one thread-block-cluster launch on the inverted 64 x 64 diagonal blocks (potrs_cluster.cu)
-bool potrs_cluster_enabled();
 bool potrs_cluster_for(int64_t m);
 int d_potrs_prepare(smcp_ctx *ctx, const double *H, int64_t ld, int64_t m, double *Dinv);
 int d_potrs_cluster(smcp_ctx *ctx, const double *H, int64_t m, const double *Dinv, double *y_dev);

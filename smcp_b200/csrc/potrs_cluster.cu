@@ -13,11 +13,11 @@
 // The backward sweep with L^T mirrors it.  All sums have a fixed order: bitwise reproducible.
 // Inverting only the 64 x 64 DIAGONAL blocks keeps the solve as accurate as substitution up to the
 // condition of those blocks (the iterative refinement of the Newton systems, solvers.py:907-913, absorbs
-// it); SMCP_B200_POTRS_SUBST=1 selects the substitution kernel of dense.cu instead.
+// it).  Orders whose blocks outnumber what the wavefront kernel can own go to the substitution kernel
+// of dense.cu.
 #include "internal.cuh"
 #include <cooperative_groups.h>
 #include <algorithm>
-#include <cstdlib>
 
 namespace cg = cooperative_groups;
 
@@ -358,13 +358,12 @@ __global__ void __launch_bounds__(PW_T, 1) potrs_wave_kernel(WaveArgs a) {
     }
 }
 
+// from m = 512 on the wavefront beats the 16-CTA cluster kernel as well (m = 1000: 0.22 -> 0.13 ms, m = 4000: 1.75 -> 0.43 ms,
+// profiles/r02_v39_potrs_wave_min.log)
+static const int64_t POTRS_WAVE_MIN = 512;
 bool potrs_wave_for(const smcp_ctx *ctx, int64_t m) {
-    static const bool off = getenv("SMCP_B200_POTRS_NO_WAVE") && atoi(getenv("SMCP_B200_POTRS_NO_WAVE")) != 0;
-    // from m = 512 on the wavefront beats the 16-CTA cluster kernel as well (m = 1000: 0.22 -> 0.13 ms, m = 4000: 1.75 -> 0.43 ms,
-    // gpurun_out/r02_v39_potrs_wave_min.log); SMCP_B200_POTRS_WAVE_MIN moves the switch
-    static const int64_t wave_min = getenv("SMCP_B200_POTRS_WAVE_MIN") ? atoll(getenv("SMCP_B200_POTRS_WAVE_MIN")) : 512;
     const int64_t nb = (m + 63) / 64;
-    return !off && potrs_cluster_enabled() && m >= wave_min && nb <= (int64_t)PW_MAXOWN * ctx->num_sms;
+    return m >= POTRS_WAVE_MIN && nb <= (int64_t)PW_MAXOWN * ctx->num_sms;
 }
 
 int d_potrs_wave(smcp_ctx *ctx, const double *H, int64_t m, const double *Dinv, double *y_dev) {
@@ -411,14 +410,10 @@ int d_potrs_prepare(smcp_ctx *ctx, const double *H, int64_t ld, int64_t m, doubl
     return 0;
 }
 
-bool potrs_cluster_enabled() {
-    static const bool off = getenv("SMCP_B200_POTRS_SUBST") && atoi(getenv("SMCP_B200_POTRS_SUBST")) != 0;
-    return !off;
-}
 // One cluster (16 SMs at most) streams the whole factor: fine while it sits in L2 and the solve is a
 // latency chain (m = 1000: 0.09 ms against 0.24), slower than the many-SM streamed updates of dense.cu
 // once the factor is hundreds of MB (m = 10^4: 5.1 ms against 3.6)
-bool potrs_cluster_for(int64_t m) { return potrs_cluster_enabled() && m <= 4096; }
+bool potrs_cluster_for(int64_t m) { return m <= 4096; }
 
 int d_potrs_cluster(smcp_ctx *ctx, const double *H, int64_t m, const double *Dinv, double *y_dev) {
     return d_trs_cluster(ctx, H, m, m, Dinv, y_dev, m, 1, 1, 1, "potrs");
