@@ -192,6 +192,32 @@ int smcp_pm1_tabu_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host,
                          int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
                          int64_t iters, int64_t tenure, double *values_host, int64_t *moves_host,
                          int64_t *best_iter_host);
+/* Low-rank (Burer-Monteiro) solve of  min C . X  s.t.  X_ii = b_i (b_i > 0 finite), X >= 0  with X = V V^T, V n x r
+ * (1 <= r <= 512), by the mixing method: colours of a greedy colouring of C's off-diagonal pattern (vertex i takes the
+ * smallest colour none of its lower-index neighbours has) are swept in order, and every vertex i of a colour gets
+ * v_i <- -sqrt(b_i) w_i / ||w_i||, w_i = sum_{j != i} C_ij v_j (unchanged when w_i = 0).  C is given by nc objective
+ * entries as in smcp_pm1_local_search.  Row i of the start is the standard normal sample i of smcp_csp_sample's
+ * generator (length r) scaled to norm sqrt(b_i).  f_k = sum_i C_ii b_i + <v_i, w_i> after k sweeps goes to f_host[k];
+ * the run stops after the first sweep k with f_{k-1} - f_k <= tol max(1, |f_k|), or after max_sweeps sweeps
+ * (*sweeps_out; f_host holds max_sweeps + 1 doubles, of which sweeps + 1 are written).  V_host receives V (n x r,
+ * row-major), y_host y_i = (C_ii b_i + <v_i, w_i>) / b_i at the final V, *colors_out the number of colours.  Every
+ * result is bitwise reproducible (lowrank.cu states the summation orders).  -2: r outside 1..512, b_i <= 0 or not
+ * finite, max_sweeps < 0, a negative or non-finite tol, or an entry outside 0..n-1. */
+int smcp_lowrank_solve(smcp_ctx *ctx, int64_t n, int64_t r, int64_t nc, const int64_t *crow, const int64_t *ccol,
+                       const double *cval, const double *b, uint64_t seed, int64_t max_sweeps, double tol,
+                       double *V_host, double *f_host, double *y_host, int64_t *sweeps_out, int64_t *colors_out);
+/* ±1 rounding from a low-rank factor: smcp_round_pm1 with the samples V g_t, V the n x r factor V_host (row-major,
+ * original coordinates, as smcp_lowrank_solve returns it) and g_t the length-r normal sample t under seed, computed in
+ * blocks of one width as one DMMA product each, so every output is independent of chunk.  The objective entries are in
+ * the coordinates of V.  The one-flip search runs on every trial when max_flips > 0 (tol, values0_host, flips_host as
+ * in smcp_round_pm1_ls), the tabu search when tabu_iters > 0 (tenure, values1_host, moves_host, best_iter_host as in
+ * smcp_round_pm1_tabu); values0_host and flips_host are needed when either search runs, the other search outputs
+ * when the tabu search runs, and may be null otherwise.  The limits on n and tenure are those of the searches. */
+int smcp_round_pm1_factor(smcp_ctx *ctx, int64_t n, int64_t r, const double *V_host, uint64_t seed, int64_t trials,
+                          int64_t chunk, int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
+                          int64_t max_flips, double tol, int64_t tabu_iters, int64_t tenure,
+                          double *values0_host, double *values1_host, double *values_host, int8_t *x_host,
+                          int64_t *best_out, int64_t *flips_host, int64_t *moves_host, int64_t *best_iter_host);
 
 /* ---- barrier Hessian: chompack.hessian(L, Y, U, adj=None, inv=...) ---------------------- */
 int smcp_hess_create(smcp_sym *sym, const double *L, const double *Y, smcp_hess **out);

@@ -313,7 +313,11 @@ class SDP(object):
         ``tabu_iters > 0`` runs the tabu search of ``tabu_search_pm1`` (``tabu_iters`` moves, ``tenure``) on every
         trial on the device, after the one-flip search when that is on; ``x``, ``value``, ``values`` and ``trial``
         then refer to the trials after the tabu search, ``values_before_tabu`` holds the values before it, ``moves``
-        the number of moves and ``best_iter`` the move count of every returned vector."""
+        the number of moves and ``best_iter`` the move count of every returned vector.
+
+        When ``sol`` holds ``V`` (a low-rank solution from ``solve_lowrank``), trial t is sign(V g_t) instead, g_t the
+        length-r normal sample t under ``seed``: the samples are one DMMA product per block of trials on the device, in
+        the original order, and need no completion; everything else is as above."""
         trials = _check_count(trials, "trials", 1)
         seed = _check_seed(seed)
         chunk = _check_count(chunk, "chunk", 0)
@@ -324,8 +328,10 @@ class SDP(object):
         tol = _check_tol(tol)
         tabu_iters = _check_count(tabu_iters, "tabu_iters", 0)
         tenure = _tabu_tenure(self.n) if tenure is None else _check_count(tenure, "tenure", 0)
-        if not isinstance(sol, dict) or "x" not in sol:
-            raise ValueError("sol must be a solution dict holding 'x'")
+        if not isinstance(sol, dict) or ("x" not in sol and "V" not in sol):
+            raise ValueError("sol must be a solution dict holding 'x' or 'V'")
+        if "V" in sol:
+            return self._round_pm1_factor(sol["V"], trials, seed, chunk, local_search, max_flips, tol, tabu_iters, tenure)
         L, order = _completion_factor(sol["x"])
         n = self.n
         if len(order) != n:
@@ -351,6 +357,114 @@ class SDP(object):
         x[order] = xi
         out.update({"x": x, "value": float(values[best]), "values": values, "trial": int(best)})
         return out
+
+    def _round_pm1_factor(self, V, trials, seed, chunk, local_search, max_flips, tol, tabu_iters, tenure):
+        """``round_pm1`` from the factor V (checked arguments)."""
+        n = self.n
+        V = np.asarray(V, dtype=np.float64)
+        if V.ndim != 2 or V.shape[0] != n or not 1 <= V.shape[1] <= _LOWRANK_MAX_RANK:
+            raise ValueError("sol['V'] must be n x r with n = %d and 1 <= r <= %d" % (n, _LOWRANK_MAX_RANK))
+        I, J, v = self._objective_entries()
+        ops = solvers._make_backend(Symbolic(n, np.arange(n + 1), np.arange(n)))
+        mf = (n if max_flips is None else max_flips) if local_search else 0
+        values0, values1, values, flips, moves, best_iter, x, best = ops.round_pm1_factor(
+            V, I, J, v, trials, seed, chunk, mf, tol, tabu_iters, tenure)
+        out = {}
+        if tabu_iters > 0:
+            out.update({"values_before_tabu": values1, "moves": moves, "best_iter": best_iter})
+        if local_search:
+            if values0 is None:                     # max_flips = 0 and no tabu search: nothing ran
+                values0, flips = values.copy(), np.zeros(len(values), dtype=np.int64)
+            out.update({"values_rounded": values0, "flips": flips})
+        out.update({"x": x, "value": float(values[best]), "values": values, "trial": int(best)})
+        return out
+
+    # -- low-rank solve (an extension: the reference has none) ----------------------------
+    def solve_lowrank(self, rank=None, seed=0, tol=1e-6, max_sweeps=1000, bound=True):
+        """Low-rank (Burer-Monteiro) solve of  min C . X  s.t.  X_ii = b_i, X >= 0  on the device, for an SDP whose m = n
+        constraints each hold one entry, coefficient 1 at a diagonal position (d_k, d_k), d a permutation of 0..n-1, and
+        b > 0 (``maxcut_SDP`` has this form; any other problem raises ``ValueError``).
+
+        X = V V^T with V n x ``rank`` (None: the smallest r with r(r+1)/2 > n, at most 512), solved by the mixing method:
+        with the rows of C's off-diagonal entries (both triangles, duplicates summed in input order) and a greedy
+        colouring in increasing vertex index (vertex i takes the smallest colour none of its lower-index neighbours
+        has), each sweep takes the colours in order and sets v_i <- -sqrt(b_i) w_i / ||w_i|| for every vertex i of the
+        colour, w_i = sum_{j != i} C_ij v_j (v_i stays when w_i = 0).  Row i of the start is the standard normal sample
+        i (length r) under ``seed`` of ``completion_sample``'s generator, scaled to norm sqrt(b_i).  The objective
+        f = sum_i C_ii b_i + <v_i, w_i> is evaluated at the start and after every sweep; the run stops after the first
+        sweep k with f_{k-1} - f_k <= ``tol`` max(1, |f_k|), or after ``max_sweeps`` sweeps.  csrc/lowrank.cu states the
+        summation orders: every result is bitwise reproducible.
+
+        ``bound=True`` certifies a lower bound on the optimum (``_lowrank_certificate``): with y_i = (C_ii b_i +
+        <v_i, w_i>) / b_i, the smallest shift t >= 0 found by bisection with C - Diag(y) + tI >= 0 proven by chordal
+        Cholesky factorizations on the backend, so y - t is dual feasible and b^T y - t sum(b) a lower bound.
+
+        Returns a dict: ``V`` (n x r, original order), ``x`` = P_V(V V^T) on the chordal embedding of C's pattern (the
+        form ``solve_feas`` returns), ``y`` (constraint order, shifted by t), ``primal objective`` f, ``dual objective``
+        (the certified bound, None when bound=False), ``gap`` (their difference, None without a bound), ``converged``,
+        ``sweeps``, ``objective history`` (f_0 .. f_sweeps), ``colors`` (the number of colours), ``rank``, ``shift`` (t)
+        and ``probes`` (Cholesky factorizations of the certificate)."""
+        n = self.n
+        d, bk = self._lowrank_form()
+        if rank is None:
+            rank = min(_LOWRANK_MAX_RANK, next(r for r in range(1, n + 2) if r * (r + 1) // 2 > n))
+        rank = _check_count(rank, "rank", 1)
+        if rank > _LOWRANK_MAX_RANK:
+            raise ValueError("rank must be at most %d" % _LOWRANK_MAX_RANK)
+        seed = _check_seed(seed)
+        tol = _check_tol(tol)
+        max_sweeps = _check_count(max_sweeps, "max_sweeps", 0)
+        bv = np.empty(n)
+        bv[d] = bk                                  # b per vertex
+        I, J, v = self._objective_entries()
+        ops = solvers._make_backend(Symbolic(n, np.arange(n + 1), np.arange(n)))
+        V, f, yv, sweeps, colors = ops.lowrank_solve(I, J, v, bv, rank, seed, max_sweeps, tol)
+        fk = float(f[-1])
+        converged = sweeps > 0 and float(f[-2]) - fk <= tol * max(1.0, abs(fk))
+        symb, p, _ = _chordal_embedding(sp.coo_matrix((np.concatenate([v, np.ones(n)]),
+                                                       (np.concatenate([I, np.arange(n)]),
+                                                        np.concatenate([J, np.arange(n)]))), shape=(n, n)))
+        ri, ci = p[symb.Ip], p[symb.Jp]
+        xv = np.empty(len(ri))
+        step = max(1, (1 << 24) // rank)
+        for a in range(0, len(ri), step):
+            xv[a:a + step] = np.einsum("ij,ij->i", V[ri[a:a + step]], V[ci[a:a + step]])
+        off = ri != ci
+        x = sp.csc_matrix((np.concatenate([xv, xv[off]]), (np.concatenate([ri, ci[off]]), np.concatenate([ci, ri[off]]))),
+                          shape=(n, n))
+        t, probes, dual = 0.0, 0, None
+        if bound:
+            t, probes = _lowrank_certificate(n, I, J, v, yv, bv, fk)
+            bsum = float(bv.sum())
+            dual = float(np.dot(bv, yv)) - t * bsum
+            # rounding of the two sums above (gamma_{n+2} of their absolute terms): the bound stays a bound
+            dual -= _gamma(n + 2) * (float(np.abs(bv * yv).sum()) + t * bsum)
+        return {"V": V, "x": x, "y": yv[d] - t, "primal objective": fk, "dual objective": dual,
+                "gap": None if dual is None else fk - dual, "converged": bool(converged), "sweeps": int(sweeps),
+                "objective history": f, "colors": int(colors), "rank": rank, "shift": t, "probes": probes}
+
+    def _lowrank_form(self):
+        """(d, b) of an SDP whose constraint k holds the single entry 1 at (d_k, d_k), d a permutation, b > 0; raises
+        ``ValueError`` for any other problem."""
+        A, n, m = self._need(), self.n, self.m
+        if m != n:
+            raise ValueError("solve_lowrank needs m = n constraints X_ii = b_i (got m = %d, n = %d)" % (m, n))
+        cnt = np.diff(A.indptr)[1:]
+        if (cnt != 1).any():
+            raise ValueError("solve_lowrank needs constraints with one entry each (constraint %d has %d)" % (
+                int(np.flatnonzero(cnt != 1)[0]), int(cnt[cnt != 1][0])))
+        pos = A.indices[A.indptr[1]:A.indptr[m + 1]]
+        val = A.data[A.indptr[1]:A.indptr[m + 1]]
+        r, c = misc.ind2sub(n, pos)
+        if (np.asarray(r) != np.asarray(c)).any() or (val != 1.0).any():
+            raise ValueError("solve_lowrank needs constraints X_ii = b_i: coefficient 1 at a diagonal position")
+        d = np.asarray(r, dtype=np.int64)
+        if len(np.unique(d)) != n:
+            raise ValueError("solve_lowrank needs one constraint per diagonal entry")
+        b = self.b
+        if not (np.isfinite(b).all() and (b > 0).all()):
+            raise ValueError("solve_lowrank needs b > 0")
+        return d, b
 
     def local_search_pm1(self, x, max_flips=None, tol=1e-12):
         """One-flip local search of +-1 vectors against f(x) = C . x x^T (minimized), on the device (an
@@ -629,13 +743,10 @@ class maxcut_SDP(SDP):
         return r["x"], -r["value"], -float(sol["dual objective"])
 
 
-def _completion_factor(X):
-    """``symbolic`` of the pattern of ``X`` (lower triangle used) under a fill-reducing ordering and
-    ``chompack.completion`` on the backend: returns the factor L (a cspmatrix, P_V((L L^T)^-1) = X) and
-    ``order``, the original vertex at each internal position.  Raises ``ArithmeticError`` if X has no
-    positive definite completion."""
-    from .chordal import cspmatrix
-    from . import chordal
+def _chordal_embedding(X):
+    """``symbolic`` of the pattern of the sparse symmetric ``X`` (lower triangle used) under a fill-reducing ordering
+    (maximum cardinality search when it adds no fill, else minimum degree).  Returns ``(symb, p, full)``: the symbolic,
+    the ordering (vertex p[k] is the k-th of the embedding) and X with both triangles as CSR."""
     X = sp.tril(sp.csc_matrix(X), format="coo")
     n = X.shape[0]
     cp, ri = lower_pattern(n, X.row, X.col)
@@ -644,13 +755,99 @@ def _completion_factor(X):
     if fc[-1] != cp[-1]:
         p = min_degree(n, cp, ri)
         fc, fr, _ = embed(n, cp, ri, p)
-    symb = Symbolic(n, fc, fr)
-    ops = solvers._make_backend(symb)
     lo = sp.tril(X, format="csc")
-    full = (lo + sp.tril(lo, -1).T).tocsr()
+    return Symbolic(n, fc, fr), p, (lo + sp.tril(lo, -1).T).tocsr()
+
+
+def _completion_factor(X):
+    """``symbolic`` of the pattern of ``X`` (``_chordal_embedding``) and ``chompack.completion`` on the backend: returns
+    the factor L (a cspmatrix, P_V((L L^T)^-1) = X) and ``order``, the original vertex at each internal position.  Raises
+    ``ArithmeticError`` if X has no positive definite completion."""
+    from .chordal import cspmatrix
+    from . import chordal
+    symb, p, full = _chordal_embedding(X)
+    ops = solvers._make_backend(symb)
     L = cspmatrix.from_vec(ops, np.asarray(full[p[symb.Ip], p[symb.Jp]]).ravel())
     chordal.completion(L)                       # ArithmeticError if X has no PD completion
     return L, p[symb.perm]                      # internal order: vertex p[perm[i]] at position i
+
+
+_LOWRANK_MAX_RANK = 512
+_U = 2.0 ** -53                                 # unit roundoff of IEEE double
+
+
+def _gamma(k):
+    """gamma_k = k u / (1 - k u) (Higham, Accuracy and Stability of Numerical Algorithms, 3.1)."""
+    return k * _U / (1.0 - k * _U)
+
+
+def _lowrank_delta(n, sdiag_abs, t):
+    """Backward-error margin delta(t) of a probe of ``_lowrank_certificate`` that factors M = fl(S + (t - delta) I).
+
+    If floating-point Cholesky runs to completion on a symmetric M of order n, the computed factor satisfies
+    L L^T = M + dM with |dM| <= gamma_{n+1} |L| |L^T| (Higham, Thm 10.3; any order of the inner sums, blocked and
+    supernodal included, FMA or not), and ||l_i||^2 <= M_ii / (1 - gamma_{n+1}) from the diagonal equation.  Hence
+    ||dM||_2 <= gamma_{n+1} sum_i ||l_i||^2 <= alpha tr(M) with alpha = gamma_{n+1} / (1 - gamma_{n+1}), and
+    lambda_min(M) >= -alpha tr(M) (Rump, "Verification of positive definiteness", BIT 46 (2006), Lemma 2.1 and
+    Theorem 2.3; no underflow term is needed at these magnitudes).  M differs from the exact S + (t - delta) I only on
+    the diagonal, by at most 2u |M_ii| (the rounded t - delta and the rounded sum), and the rounded S_ii = fl(C_ii - y_i)
+    differs from the exact C_ii - y_i by at most u |S_ii|.  With |M_ii| <= (|S_ii| + |t|)(1 + 2u) this gives
+
+        lambda_min(C - Diag(y) + t I) >= delta - alpha sum_i (|S_ii| + |t|)(1 + 2u) - 3u (1 + 2u) max_i (|S_ii| + |t|),
+
+    so delta = (1 + 1e-6) (alpha sum_i (|S_ii| + |t|) + 3u max_i (|S_ii| + |t|)) makes a successful probe prove
+    C - Diag(y) + t I >= 0; the factor 1 + 1e-6 covers 2u and the rounding of this evaluation."""
+    alpha = _gamma(n + 1) / (1.0 - _gamma(n + 1))
+    a = sdiag_abs + abs(t)
+    return (1.0 + 1e-6) * (alpha * float(a.sum()) + 3.0 * _U * float(a.max()))
+
+
+def _lowrank_certificate(n, I, J, v, y, b, f):
+    """The smallest shift t >= 0 (up to the bisection tolerance) with C - Diag(y) + t I >= 0 proven, and the number of
+    Cholesky probes spent.  S = C - Diag(y) lives on the chordal embedding of C's pattern (``_chordal_embedding``); a
+    probe at t factors S + (t - delta(t)) I (``_lowrank_delta``) with the backend's chordal ``cholesky``, and its
+    success proves S + t I >= 0.  t = 0 is probed first; otherwise the bracket [0, t_hi] starts from the Gershgorin
+    shift max_i (sum_{j != i} |S_ij| - S_ii) plus a margin, and is halved until (t_hi - t_lo) sum(b) <= 1e-6 max(1, |f|).
+    Returns t_hi, the upper end: a probe at it succeeded."""
+    from .chordal import cspmatrix, cholesky
+    S = sp.coo_matrix((np.concatenate([v, -y]), (np.concatenate([I, np.arange(n)]), np.concatenate([J, np.arange(n)]))),
+                      shape=(n, n))
+    symb, p, full = _chordal_embedding(S)
+    ops = solvers._make_backend(symb)
+    sv = np.asarray(full[p[symb.Ip], p[symb.Jp]]).ravel()
+    dpos = symb.diag_vec
+    sdiag = sv[dpos]
+    sabs = np.abs(sdiag)
+    probes = 0
+
+    def ok(t):
+        nonlocal probes
+        probes += 1
+        w = sv.copy()
+        w[dpos] = sdiag + (t - _lowrank_delta(n, sabs, t))
+        try:
+            cholesky(cspmatrix.from_vec(ops, w))
+            return True
+        except ArithmeticError:
+            return False
+
+    if ok(0.0):
+        return 0.0, probes
+    Sf = full.tocoo()
+    offd = np.zeros(n)
+    np.add.at(offd, Sf.row[Sf.row != Sf.col], np.abs(Sf.data[Sf.row != Sf.col]))
+    g = max(0.0, float((offd - full.diagonal()).max()))
+    lo, hi = 0.0, g + 4.0 * _lowrank_delta(n, sabs, g) + 1e-12 * max(1.0, g)
+    while not ok(hi):
+        lo, hi = hi, 2.0 * hi
+    tol = 1e-6 * max(1.0, abs(f)) / float(b.sum())
+    while hi - lo > tol:
+        mid = 0.5 * (lo + hi)
+        if ok(mid):
+            hi = mid
+        else:
+            lo = mid
+    return hi, probes
 
 
 def completion(X):

@@ -546,6 +546,20 @@ extern "C" int smcp_pm1_tabu_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t 
                                     int64_t *moves_host, int64_t *best_iter_host) {
     return k_pm1_tabu_search(ctx, n, k, x_host, nc, crow, ccol, cval, iters, tenure, values_host, moves_host, best_iter_host);
 }
+extern "C" int smcp_lowrank_solve(smcp_ctx *ctx, int64_t n, int64_t r, int64_t nc, const int64_t *crow, const int64_t *ccol,
+                                  const double *cval, const double *b, uint64_t seed, int64_t max_sweeps, double tol,
+                                  double *V_host, double *f_host, double *y_host, int64_t *sweeps_out, int64_t *colors_out) {
+    return k_lowrank_solve(ctx, n, r, nc, crow, ccol, cval, b, seed, max_sweeps, tol, V_host, f_host, y_host, sweeps_out,
+                           colors_out);
+}
+extern "C" int smcp_round_pm1_factor(smcp_ctx *ctx, int64_t n, int64_t r, const double *V_host, uint64_t seed, int64_t trials,
+                                     int64_t chunk, int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
+                                     int64_t max_flips, double tol, int64_t tabu_iters, int64_t tenure, double *values0_host,
+                                     double *values1_host, double *values_host, int8_t *x_host, int64_t *best_out,
+                                     int64_t *flips_host, int64_t *moves_host, int64_t *best_iter_host) {
+    return k_round_pm1_factor(ctx, n, r, V_host, seed, trials, chunk, nc, crow, ccol, cval, max_flips, tol, tabu_iters, tenure,
+                              values0_host, values1_host, values_host, x_host, best_out, flips_host, moves_host, best_iter_host);
+}
 
 // ---------------------------------------------------------------------------------------
 // Hessian factor

@@ -302,6 +302,55 @@ int k_round_pm1_tabu(smcp_sym *s, const double *L, uint64_t seed, int64_t trials
 int k_pm1_tabu_search(smcp_ctx *ctx, int64_t n, int64_t k, int8_t *x_host, int64_t nc, const int64_t *crow, const int64_t *ccol,
                       const double *cval, int64_t iters, int64_t tenure, double *values_host, int64_t *moves_host,
                       int64_t *best_iter_host);
+// rounding of the +-1 trials sign(V g_t) from a low-rank factor V (n x r, row-major, host), with the searches of
+// k_round_pm1_tabu (max_flips = 0 and tabu_iters = 0: plain rounding; the search outputs may then be null)
+int k_round_pm1_factor(smcp_ctx *ctx, int64_t n, int64_t r, const double *V_host, uint64_t seed, int64_t trials, int64_t chunk,
+                       int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval, int64_t max_flips, double tol,
+                       int64_t tabu_iters, int64_t tenure, double *values0_host, double *values1_host, double *values_host,
+                       int8_t *x_host, int64_t *best_out, int64_t *flips_host, int64_t *moves_host, int64_t *best_iter_host);
+// B[i + c ldb] = entry i < n of the standard normal sample col0 + c < col0 + k under seed (round_normal_kernel)
+int launch_round_normals(smcp_ctx *ctx, uint64_t seed, int64_t col0, int n, double *B, int64_t ldb, int64_t k);
+
+// device workspace of one call, freed (after the stream drains) when it goes out of scope
+struct RoundWs {
+    smcp_ctx *ctx;
+    const char *fn;
+    std::vector<void *> p;
+    ~RoundWs() {
+        cudaStreamSynchronize(ctx->stream);
+        for (void *q : p) cudaFree(q);
+    }
+    void *alloc(size_t bytes) {
+        void *q = nullptr;
+        if (cudaMalloc(&q, bytes < 16 ? 16 : bytes) != cudaSuccess) {
+            cudaGetLastError();
+            smcp_set_error("%s: cudaMalloc(%zu bytes) failed", fn, bytes);
+            return nullptr;
+        }
+        p.push_back(q);
+        return q;
+    }
+};
+
+// the rows of the one-flip search on the device (see round_ls_kernel in rounding.cu): CSR of the off-diagonal entries of
+// C from both triangles, increasing columns, duplicates summed in input order, and thr_i = tol sum_j |C_ij|
+struct LsRows {
+    long long *rp = nullptr;
+    int *col = nullptr;
+    double *val = nullptr, *thr = nullptr;
+};
+struct LsRowsHost {
+    std::vector<long long> rp;
+    std::vector<int> col;
+};
+// entries must lie in 0..n-1 (checked by the caller); with `host`, the host copy of rp and col is kept there
+int ls_rows_upload(RoundWs &ws, int n, int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval, double tol,
+                   LsRows &d, LsRowsHost *host);
+
+// low-rank (Burer-Monteiro) solve of min C . X s.t. X_ii = b_i, X >= 0 by the mixing method (lowrank.cu)
+int k_lowrank_solve(smcp_ctx *ctx, int64_t n, int64_t r, int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
+                    const double *b, uint64_t seed, int64_t max_sweeps, double tol, double *V_host, double *f_host, double *y_host,
+                    int64_t *sweeps_out, int64_t *colors_out);
 
 // dense path for the top set of large supernodes (bigfront.cu)
 int big_setup(smcp_sym *s, const smcp_sym_desc *D);

@@ -175,13 +175,12 @@ __global__ void __launch_bounds__(BEST_THREADS) round_best_kernel(const double *
     for (int i = tid; i < n; i += BEST_THREADS) x[i] = ((wg[i] >> b) & 1ULL) ? -1 : 1;
 }
 
-static int launch_normals(smcp_sym *s, uint64_t seed, int64_t col0, double *B, int64_t ldb, int64_t k) {
-    smcp_ctx *ctx = s->ctx;
-    const long long total = (long long)((s->d.n + 3) / 4) * k;
+int launch_round_normals(smcp_ctx *ctx, uint64_t seed, int64_t col0, int n, double *B, int64_t ldb, int64_t k) {
+    const long long total = (long long)((n + 3) / 4) * k;
     const long long grid = std::max(1LL, std::min((total + 255) / 256, (long long)ctx->num_sms * 16));
     {
         LaunchScope ls(ctx, "round_normal");
-        round_normal_kernel<<<(unsigned)grid, 256, 0, ctx->stream>>>(seed, col0, s->d.n, k, B, ldb);
+        round_normal_kernel<<<(unsigned)grid, 256, 0, ctx->stream>>>(seed, col0, n, k, B, ldb);
     }
     CUDA_TRY(cudaGetLastError());
     return 0;
@@ -193,7 +192,7 @@ int k_sample(smcp_sym *s, const double *L, uint64_t seed, int64_t col0, double *
         return -2;
     }
     if (k == 0) return 0;
-    if (launch_normals(s, seed, col0, B, ldb, k)) return -1;
+    if (launch_round_normals(s->ctx, seed, col0, s->d.n, B, ldb, k)) return -1;
     return k_trsm(s, L, B, ldb, k, 1);
 }
 
@@ -531,27 +530,6 @@ __global__ void __launch_bounds__(LS_THREADS, 4) round_tabu_kernel(int n, int T,
 // same bits whatever the pass size (k_trsm picks its kernels from the number of right-hand sides)
 #define ROUND_BLOCK 256
 
-// device workspace of one call, freed (after the stream drains) when it goes out of scope
-struct RoundWs {
-    smcp_ctx *ctx;
-    const char *fn;
-    std::vector<void *> p;
-    ~RoundWs() {
-        cudaStreamSynchronize(ctx->stream);
-        for (void *q : p) cudaFree(q);
-    }
-    void *alloc(size_t bytes) {
-        void *q = nullptr;
-        if (cudaMalloc(&q, std::max<size_t>(bytes, 16)) != cudaSuccess) {
-            cudaGetLastError();
-            smcp_set_error("%s: cudaMalloc(%zu bytes) failed", fn, bytes);
-            return nullptr;
-        }
-        p.push_back(q);
-        return q;
-    }
-};
-
 // the objective on the device, as round_eval_kernel reads it: nc entries (r, c, coef), the factor 2 off the diagonal
 // folded into coef, cut into S fixed slices of `per` entries (independent of the trials)
 struct RoundObj {
@@ -590,16 +568,8 @@ static int round_obj_upload(RoundWs &ws, const char *fn, int n, int64_t nc, cons
     return 0;
 }
 
-// the search's rows on the device (see round_ls_kernel): CSR of the off-diagonal entries and thr_i = tol a_i
-struct LsRows {
-    long long *rp = nullptr;
-    int *col = nullptr;
-    double *val = nullptr, *thr = nullptr;
-};
-
-// entries already checked by round_obj_upload
-static int ls_rows_upload(RoundWs &ws, int n, int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval,
-                          double tol, LsRows &d) {
+int ls_rows_upload(RoundWs &ws, int n, int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval, double tol,
+                   LsRows &d, LsRowsHost *host) {
     std::vector<int64_t> q;
     for (int64_t e = 0; e < nc; ++e)
         if (crow[e] != ccol[e]) q.push_back(e);
@@ -653,6 +623,10 @@ static int ls_rows_upload(RoundWs &ws, int n, int64_t nc, const int64_t *crow, c
         CUDA_TRY(cudaMemcpyAsync(d.val, val.data(), nnz * sizeof(double), cudaMemcpyHostToDevice, st));
     }
     CUDA_TRY(cudaMemcpyAsync(d.thr, thr.data(), (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
+    if (host) {
+        host->rp = std::move(rp);
+        host->col = std::move(col);
+    }
     return 0;
 }
 
@@ -763,20 +737,38 @@ static int search_pass(RoundWs &ws, int n, int T, int64_t t0, unsigned long long
     return 0;
 }
 
-// ls == nullptr: smcp_round_pm1; otherwise the searches run on every trial between its evaluation into
-// ls->values0_host and the evaluation that values_host, x_host and best_out report
-static int round_pm1_impl(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc,
-                          const int64_t *crow, const int64_t *ccol, const double *cval, const LsArgs *ls, double *values_host,
-                          int8_t *x_host, int64_t *best_out) {
-    smcp_ctx *ctx = s->ctx;
-    const int n = s->d.n;
-    const char *fn = ls ? (ls->tabu ? "smcp_round_pm1_tabu" : "smcp_round_pm1_ls") : "smcp_round_pm1";
+// where the samples of a pass come from: L^-T g, the normals through the chordal trsm with the completion factor L of
+// s (smcp_round_pm1*), or V g, normals of length r times the factor V (n x r, row-major on the device) in one DMMA
+// product (smcp_round_pm1_factor; G holds the r x tb normals of a block)
+struct RoundSrc {
+    smcp_sym *s;
+    const double *L;
+    const double *V;
+    int r;
+    double *G;
+};
+
+// the samples col0 .. col0 + tb - 1 into the n x tb block Vb
+static int round_samples(smcp_ctx *ctx, int n, const RoundSrc &src, uint64_t seed, int64_t col0, double *Vb, int64_t tb) {
+    if (src.L) {
+        if (launch_round_normals(ctx, seed, col0, n, Vb, n, tb)) return -1;
+        return k_trsm(src.s, src.L, Vb, n, tb, 1);
+    }
+    if (launch_round_normals(ctx, seed, col0, src.r, src.G, src.r, tb)) return -1;
+    return launch_gemm(ctx, true, true, src.V, src.r, src.G, src.r, Vb, n, n, tb, src.r, 1.0, 0, 0, 0, "round_factor");
+}
+
+// ls == nullptr: plain rounding; otherwise the searches run on every trial between its evaluation into
+// ls->values0_host and the evaluation that values_host, x_host and best_out report.  src.G is allocated here.
+static int round_pm1_impl(smcp_ctx *ctx, const char *fn, int n, RoundSrc src, uint64_t seed, int64_t trials, int64_t chunk,
+                          int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval, const LsArgs *ls,
+                          double *values_host, int8_t *x_host, int64_t *best_out) {
     if (trials < 1 || chunk < 0 || nc < 0) {
         smcp_set_error("%s: need trials >= 1, chunk >= 0, nc >= 0 (got %lld, %lld, %lld)", fn, (long long)trials,
                        (long long)chunk, (long long)nc);
         return -2;
     }
-    if (!L || !values_host || !x_host || !best_out || (nc > 0 && (!crow || !ccol || !cval)) ||
+    if (!(src.L || src.V) || !values_host || !x_host || !best_out || (nc > 0 && (!crow || !ccol || !cval)) ||
         (ls && (!ls->values0_host || !ls->flips_host)) ||
         (ls && ls->tabu && (!ls->values1_host || !ls->moves_host || !ls->best_iter_host))) {
         smcp_set_error("%s: null argument", fn);
@@ -796,10 +788,11 @@ static int round_pm1_impl(smcp_sym *s, const double *L, uint64_t seed, int64_t t
     const int64_t nwmax = (pw + 63) / 64;
 
     RoundWs ws{ctx, fn, {}};
+    if (!src.L && !(src.G = (double *)ws.alloc((size_t)src.r * tb * sizeof(double)))) return -1;
     RoundObj o;
     if (int rc = round_obj_upload(ws, fn, n, nc, crow, ccol, cval, o)) return rc;
     LsRows d;
-    if (ls && ls_rows_upload(ws, n, nc, crow, ccol, cval, ls->tol, d)) return -1;
+    if (ls && ls_rows_upload(ws, n, nc, crow, ccol, cval, ls->tol, d, nullptr)) return -1;
     double *V = (double *)ws.alloc((size_t)n * pw * sizeof(double));
     unsigned long long *bits = (unsigned long long *)ws.alloc((size_t)n * nwmax * sizeof(unsigned long long));
     double *part = (double *)ws.alloc((size_t)nwmax * o.S * 64 * sizeof(double));
@@ -826,8 +819,7 @@ static int round_pm1_impl(smcp_sym *s, const double *L, uint64_t seed, int64_t t
         const int64_t t0 = b0 * tb;
         for (int64_t b = b0; b < b1; ++b) {
             double *Vb = V + (size_t)(b - b0) * tb * n;
-            if (launch_normals(s, seed, b * tb, Vb, n, tb)) return -1;
-            if (k_trsm(s, L, Vb, n, tb, 1)) return -1;
+            if (round_samples(ctx, n, src, seed, b * tb, Vb, tb)) return -1;
         }
         const int T = (int)std::min<int64_t>(trials - t0, (b1 - b0) * tb);
         if (!ls) {
@@ -866,14 +858,16 @@ static int round_pm1_impl(smcp_sym *s, const double *L, uint64_t seed, int64_t t
 
 int k_round_pm1(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc, const int64_t *crow,
                 const int64_t *ccol, const double *cval, double *values_host, int8_t *x_host, int64_t *best_out) {
-    return round_pm1_impl(s, L, seed, trials, chunk, nc, crow, ccol, cval, nullptr, values_host, x_host, best_out);
+    return round_pm1_impl(s->ctx, "smcp_round_pm1", s->d.n, RoundSrc{s, L, nullptr, 0, nullptr}, seed, trials, chunk, nc, crow,
+                          ccol, cval, nullptr, values_host, x_host, best_out);
 }
 
 int k_round_pm1_ls(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc, const int64_t *crow,
                    const int64_t *ccol, const double *cval, int64_t max_flips, double tol, double *values0_host,
                    double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host) {
     const LsArgs ls{max_flips, tol, values0_host, flips_host, false, 0, 0, nullptr, nullptr, nullptr};
-    return round_pm1_impl(s, L, seed, trials, chunk, nc, crow, ccol, cval, &ls, values_host, x_host, best_out);
+    return round_pm1_impl(s->ctx, "smcp_round_pm1_ls", s->d.n, RoundSrc{s, L, nullptr, 0, nullptr}, seed, trials, chunk, nc, crow,
+                          ccol, cval, &ls, values_host, x_host, best_out);
 }
 
 int k_round_pm1_tabu(smcp_sym *s, const double *L, uint64_t seed, int64_t trials, int64_t chunk, int64_t nc,
@@ -881,7 +875,37 @@ int k_round_pm1_tabu(smcp_sym *s, const double *L, uint64_t seed, int64_t trials
                      double *values0_host, double *values_host, int8_t *x_host, int64_t *best_out, int64_t *flips_host,
                      int64_t tabu_iters, int64_t tenure, double *values1_host, int64_t *moves_host, int64_t *best_iter_host) {
     const LsArgs ls{max_flips, tol, values0_host, flips_host, true, tabu_iters, tenure, values1_host, moves_host, best_iter_host};
-    return round_pm1_impl(s, L, seed, trials, chunk, nc, crow, ccol, cval, &ls, values_host, x_host, best_out);
+    return round_pm1_impl(s->ctx, "smcp_round_pm1_tabu", s->d.n, RoundSrc{s, L, nullptr, 0, nullptr}, seed, trials, chunk, nc, crow,
+                          ccol, cval, &ls, values_host, x_host, best_out);
+}
+
+// the factor crosses to the device once; the searches are on when max_flips > 0 (one-flip) or tabu_iters > 0 (tabu, after
+// the one-flip search when that is on too)
+int k_round_pm1_factor(smcp_ctx *ctx, int64_t n, int64_t r, const double *V_host, uint64_t seed, int64_t trials, int64_t chunk,
+                       int64_t nc, const int64_t *crow, const int64_t *ccol, const double *cval, int64_t max_flips, double tol,
+                       int64_t tabu_iters, int64_t tenure, double *values0_host, double *values1_host, double *values_host,
+                       int8_t *x_host, int64_t *best_out, int64_t *flips_host, int64_t *moves_host, int64_t *best_iter_host) {
+    const char *fn = "smcp_round_pm1_factor";
+    if (n < 1 || n > INT32_MAX || r < 1 || !V_host || max_flips < 0 || tabu_iters < 0) {
+        smcp_set_error("%s: need 1 <= n < 2^31, r >= 1, a factor, max_flips >= 0 and tabu_iters >= 0 (got %lld, %lld, %lld, %lld)",
+                       fn, (long long)n, (long long)r, (long long)max_flips, (long long)tabu_iters);
+        return -2;
+    }
+    for (int64_t e = 0; e < n * r; ++e)
+        if (!std::isfinite(V_host[e])) {
+            smcp_set_error("%s: V[%lld][%lld] is not finite", fn, (long long)(e / r), (long long)(e % r));
+            return -2;
+        }
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    RoundWs ws{ctx, fn, {}};
+    double *V = (double *)ws.alloc((size_t)n * r * sizeof(double));
+    if (!V) return -1;
+    CUDA_TRY(cudaMemcpyAsync(V, V_host, (size_t)n * r * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    const RoundSrc src{nullptr, nullptr, V, (int)r, nullptr};
+    const bool tabu = tabu_iters > 0;
+    const LsArgs ls{max_flips, tol, values0_host, flips_host, tabu, tabu_iters, tenure, values1_host, moves_host, best_iter_host};
+    return round_pm1_impl(ctx, fn, (int)n, src, seed, trials, chunk, nc, crow, ccol, cval, max_flips > 0 || tabu ? &ls : nullptr,
+                          values_host, x_host, best_out);
 }
 
 // the searches of `a` on k caller-given vectors x_host, replaced by the searched ones
@@ -911,7 +935,7 @@ static int pm1_search_impl(smcp_ctx *ctx, const char *fn, int64_t n, int64_t k, 
     RoundObj o;
     if (int rc = round_obj_upload(ws, fn, (int)n, nc, crow, ccol, cval, o)) return rc;
     LsRows d;
-    if (ls_rows_upload(ws, (int)n, nc, crow, ccol, cval, a.tol, d)) return -1;
+    if (ls_rows_upload(ws, (int)n, nc, crow, ccol, cval, a.tol, d, nullptr)) return -1;
     double *V = (double *)ws.alloc((size_t)n * pw * sizeof(double));
     unsigned long long *bits = (unsigned long long *)ws.alloc((size_t)n * nwmax * sizeof(unsigned long long));
     double *part = (double *)ws.alloc((size_t)nwmax * o.S * 64 * sizeof(double));

@@ -78,6 +78,10 @@ API = {
     "smcp_round_pm1_tabu": (_int, [_vp, _dp, C.c_uint64, _i64, _i64, _i64, _i64p, _i64p, _f64p, _i64, _dbl, _f64p, _f64p,
                                    _i8p, C.POINTER(_i64), _i64p, _i64, _i64, _f64p, _i64p, _i64p]),
     "smcp_pm1_tabu_search": (_int, [_vp, _i64, _i64, _i8p, _i64, _i64p, _i64p, _f64p, _i64, _i64, _f64p, _i64p, _i64p]),
+    "smcp_lowrank_solve": (_int, [_vp, _i64, _i64, _i64, _i64p, _i64p, _f64p, _f64p, C.c_uint64, _i64, _dbl, _f64p, _f64p,
+                                  _f64p, C.POINTER(_i64), C.POINTER(_i64)]),
+    "smcp_round_pm1_factor": (_int, [_vp, _i64, _i64, _f64p, C.c_uint64, _i64, _i64, _i64, _i64p, _i64p, _f64p, _i64, _dbl,
+                                     _i64, _i64, _vp, _vp, _f64p, _i8p, C.POINTER(_i64), _vp, _vp, _vp]),
     "smcp_hess_create": (_int, [_vp, _dp, _dp, C.POINTER(_vp)]),
     "smcp_hess_destroy": (_int, [_vp]),
     "smcp_hess_apply": (_int, [_vp, _dp, _i64, _int]),
@@ -595,6 +599,58 @@ class DeviceBackend:
         TRAFFIC["h2d"] += 24 * len(cval) + 8 * x.size
         TRAFFIC["d2h"] += 8 * x.size + 24 * k
         return x, values, moves, best_iter
+
+    # -- low-rank solve ----------------------------------------------------------------------
+    def lowrank_solve(self, crow, ccol, cval, b, rank, seed, max_sweeps, tol):
+        """Mixing-method solve of min C . V V^T s.t. ||v_i||^2 = b_i on the device (``smcp_lowrank_solve``; C given by
+        its entries, b per vertex).  Returns ``(V, f, y, sweeps, colors)``: the n x rank factor, the objective after
+        0 .. sweeps sweeps, y_i = (C_ii b_i + <v_i, w_i>) / b_i, the number of sweeps and of colours."""
+        crow, ccol = _i64(crow), _i64(ccol)
+        cval = np.ascontiguousarray(cval, dtype=np.float64)
+        b = np.ascontiguousarray(b, dtype=np.float64)
+        if not len(crow) == len(ccol) == len(cval):
+            raise ValueError("crow, ccol and cval must have the same length")
+        n, r, max_sweeps = len(b), int(rank), int(max_sweeps)
+        V = np.empty((n, max(r, 0)))
+        f = np.empty(max(max_sweeps, 0) + 1)
+        y = np.empty(n)
+        sweeps, colors = C.c_int64(), C.c_int64()
+        _ck(self.lib, self.lib.smcp_lowrank_solve(self.ctx.h, n, r, len(cval), crow, ccol, cval, b, int(seed), max_sweeps,
+                                                  float(tol), V, f, y, C.byref(sweeps), C.byref(colors)))
+        TRAFFIC["h2d"] += 24 * len(cval) + 8 * n
+        TRAFFIC["d2h"] += 8 * V.size + 8 * (sweeps.value + 1) + 8 * n
+        return V, f[:sweeps.value + 1].copy(), y, sweeps.value, colors.value
+
+    def round_pm1_factor(self, V, crow, ccol, cval, trials, seed, chunk=0, max_flips=0, tol=1e-12, tabu_iters=0, tenure=0):
+        """``trials`` +-1 roundings sign(V g_t) of the n x r factor V against the objective given by its entries (in the
+        coordinates of V) on the device (``smcp_round_pm1_factor``), with the one-flip search when ``max_flips`` > 0
+        and the tabu search when ``tabu_iters`` > 0.  Returns ``(values0, values1, values, flips, moves, best_iter, x,
+        best)`` as ``round_pm1_tabu``; the outputs of a search that does not run are None."""
+        crow, ccol = _i64(crow), _i64(ccol)
+        cval = np.ascontiguousarray(cval, dtype=np.float64)
+        if not len(crow) == len(ccol) == len(cval):
+            raise ValueError("crow, ccol and cval must have the same length")
+        V = np.ascontiguousarray(V, dtype=np.float64)
+        n, r = V.shape
+        nt = max(0, int(trials))
+        search, tabu = int(max_flips) > 0 or int(tabu_iters) > 0, int(tabu_iters) > 0
+        values = np.empty(nt)
+        values0, flips = (np.empty(nt), np.empty(nt, dtype=np.int64)) if search else (None, None)
+        values1, moves, best_iter = (np.empty(nt), np.empty(nt, dtype=np.int64), np.empty(nt, dtype=np.int64)) if tabu \
+            else (None, None, None)
+        x = np.empty(n, dtype=np.int8)
+        best = C.c_int64()
+
+        def ptr(a):
+            return None if a is None else a.ctypes.data
+
+        _ck(self.lib, self.lib.smcp_round_pm1_factor(self.ctx.h, n, r, V, int(seed), int(trials), int(chunk), len(cval), crow,
+                                                     ccol, cval, int(max_flips), float(tol), int(tabu_iters), int(tenure),
+                                                     ptr(values0), ptr(values1), values, x, C.byref(best), ptr(flips),
+                                                     ptr(moves), ptr(best_iter)))
+        TRAFFIC["h2d"] += 24 * len(cval) + 8 * V.size
+        TRAFFIC["d2h"] += 8 * nt * (1 + 2 * search + 3 * tabu) + n
+        return values0, values1, values, flips, moves, best_iter, x, best.value
 
     def cholesky_batch(self, buf, count):
         info = np.zeros(count, dtype=np.int32)
